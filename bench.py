@@ -2,6 +2,7 @@
 """bench.py - pseudo-label images/s of the homography-adaptation export (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--precision fp32|f16|bf16]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -192,7 +193,7 @@ def run_reference(args):
     if rank != 0:
         return
     world = int(os.environ.get("WORLD_SIZE", 1))
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, args.warmup
     calib = cpu_reference_sample(2)
     per_h = calib["seconds"] / 2
     h = int(min(max(2, args.ref_budget_s / ((steps + warmup) * per_h)), max(2, args.ref_homographies)))
@@ -212,6 +213,33 @@ def run_reference(args):
             "cpu_baseline": {"value": v, "unit": "img/s", "cores": calib["cores"], "kind": "port", "sample": sample},
             "e2e": {"value": v, "unit": "img/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line), flush=True)
+
+
+DUMP_MAX_IMAGES = 128   # 128 heatmaps (39 MB) + at most 128 x 16384 keypoints (17 MB) stay under 64 MB
+DUMP_MAX_BYTES = 64 * 2**20
+
+
+def dump_outputs(out_dir, step, max_kp):
+    """Write what the timed path returned in its last step, as float32 DIR/<name>.npy:
+    heatmap (n,H,W) aggregated heatmaps, homographies (n,NUM_H-1,3,3) the warps they aggregate, keypoints (N,2) the (row,
+    col) box_nms kept, concatenated in image order, keypoint_counts (n,) keypoints per image.  A step of more than
+    DUMP_MAX_IMAGES images is represented by a fixed seeded sample of DUMP_MAX_IMAGES of them, in image order."""
+    import numpy as np
+
+    n = step["heat"].shape[0]
+    idx = np.arange(n) if n <= DUMP_MAX_IMAGES else np.sort(np.random.RandomState(0).choice(n, DUMP_MAX_IMAGES, replace=False))
+    counts = step["kp_count"].cpu().numpy()[idx]
+    kp = step["kp"].cpu().numpy()[idx]
+    arrays = {"heatmap": step["heat"].cpu().numpy()[idx],
+              "homographies": step["homographies"].cpu().numpy()[idx],
+              "keypoints": np.concatenate([kp[j, :min(int(c), max_kp)] for j, c in enumerate(counts)]),
+              "keypoint_counts": counts}
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"dump of {total} bytes exceeds {DUMP_MAX_BYTES}"
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out_dir / f"{k}.npy", a)
 
 
 def run_native(args):
@@ -251,9 +279,11 @@ def run_native(args):
 
     def device_step(i):
         imgs = dev_pool[i * ips:(i + 1) * ips]
-        heat, _ = eng.heatmaps(imgs, first_index=my_ids[i * ips])
-        return ctx.box_nms(heat, float(dh["nms"]), 0.1, float(dh["det_thresh"]), int(dh["top_k"]),
-                           det_thresh=float(dh["det_thresh"]), want_map=False, max_kp=max_kp)
+        heat, hom = eng.heatmaps(imgs, first_index=my_ids[i * ips])
+        r = ctx.box_nms(heat, float(dh["nms"]), 0.1, float(dh["det_thresh"]), int(dh["top_k"]),
+                        det_thresh=float(dh["det_thresh"]), want_map=False, max_kp=max_kp)
+        r.update(heat=heat, homographies=hom)
+        return r
 
     def barrier():
         if world > 1:
@@ -291,7 +321,7 @@ def run_native(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.warmup, n_steps):
-        r = device_step(i)
+        last = device_step(i)
     e1.record()
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
@@ -416,6 +446,8 @@ def run_native(args):
                                              "steps, each with the in-model NMS that export.py:69 discards"}
         except Exception as e:   # e.g. torchvision built without CUDA ops
             line["gpu_reference"] = {"unavailable": f"{type(e).__name__}: {e}"[:200]}
+    if args.dump_outputs:
+        dump_outputs(Path(args.dump_outputs), last, max_kp)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -439,7 +471,14 @@ def main():
     ap.add_argument("--ref-budget-s", type=float, default=150.0,
                     help="--impl reference: target wall time of warm-up + timed steps; sets the homographies per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's heatmaps, homographies and keypoints as float32 "
+                         "DIR/<name>.npy (rank 0's images; inputs are seeded, so two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the native arm's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

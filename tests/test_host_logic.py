@@ -326,6 +326,18 @@ def test_bench_reference_arm_contract():
     assert other.returncode == 0 and other.stdout.strip() == ""
 
 
+def test_bench_rejects_arguments_it_cannot_honour():
+    """No step count is silently changed: --steps 0 or a negative --warmup is an argument error (exit 2, no JSON line),
+    as is --dump-outputs with the reference arm, which has no native outputs to write."""
+    import subprocess
+    import sys
+    from conftest import ROOT
+    for extra in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--steps", "0"],
+                  ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, str(ROOT / "bench.py"), *extra], capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and not [l for l in out.stdout.splitlines() if l.startswith("{")], (extra, out.stderr[-500:])
+
+
 def test_cabi_rejects_null_context_without_a_gpu(built_lib):
     """Error behaviour at the boundary (include/spn_b200.h: 'return 0 or a negative SPN_E_* code with spn_last_error()'):
     every entry point called with a NULL context and zeroed arguments returns a negative code and sets a message - no

@@ -4,9 +4,25 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import HA_CFG, MP_MODEL, SP_MODEL
+from conftest import HA_CFG, MP_MODEL, SP_MODEL, rel_err
 from oracle import kornia_shim as K
 from oracle import spn_oracle as O
+
+# The oracle's convolutions run on torch's CPU backend (oneDNN), whose float32 accumulation order depends on the host's
+# instruction set and thread count.  On a host like the one that generated the goldens the oracle reproduces them bit
+# for bit; on others every convolution output moves in its last bits (up to 5e-6 of the largest value was seen with one
+# thread and AVX2).  So values computed through a convolution are compared to CONV_RTOL of the golden's largest magnitude
+# with the same zero pattern, and everything discrete (NMS support, point maps, keypoint lists) or computed without a
+# convolution stays bit-exact.
+CONV_RTOL = 3e-5
+
+
+def assert_conv_close(got, want, what):
+    got, want = np.asarray(got), np.asarray(want)
+    assert got.shape == want.shape and got.dtype == want.dtype, what
+    assert np.array_equal(got != 0, want != 0), f"{what}: zero pattern differs"
+    err = rel_err(got, want)
+    assert err <= CONV_RTOL, f"{what}: {err:.2e} relative"
 
 
 def test_nms_python_and_c_match_reference(golden):
@@ -44,13 +60,14 @@ def test_forward_matches_reference(golden, tag, cfg):
     g = golden(f"forward_{tag}.npz")
     sd = O.make_state_dict(cfg["model_name"], seed=int(g["seed"]), logit_gain=float(g["gain"]))
     out = O.model_forward(sd, torch.from_numpy(g["x"]), cfg)
-    for k in ("logits", "prob_heatmap", "prob_heatmap_nms", "pred_pts"):
-        assert np.array_equal(out["detector_output"][k].numpy(), g[k]), k
+    for k in ("logits", "prob_heatmap", "prob_heatmap_nms"):
+        assert_conv_close(out["detector_output"][k].numpy(), g[k], k)
+    assert np.array_equal(out["detector_output"]["pred_pts"].numpy(), g["pred_pts"])
     if tag == "superpoint":
-        assert np.array_equal(out["descriptor_output"]["desc_raw"].numpy(), g["desc_raw"])
+        assert_conv_close(out["descriptor_output"]["desc_raw"].numpy(), g["desc_raw"], "desc_raw")
         d = out["descriptor_output"]["desc"][0].numpy()
         pts = g["desc_pts"]
-        assert np.array_equal(d[:, pts[:, 0], pts[:, 1]].T, g["desc_at_pts"])
+        assert_conv_close(d[:, pts[:, 0], pts[:, 1]].T, g["desc_at_pts"], "desc_at_pts")
         sparse = O.sparse_descriptors(torch.from_numpy(g["desc_raw"][0]), pts).numpy()
         assert np.abs(sparse - g["desc_at_pts"]).max() < 1e-6
 
@@ -111,8 +128,8 @@ def test_ha_export_matches_reference(golden):
     sd = O.make_state_dict("magicpoint", seed=int(g["seed"]), logit_gain=float(g["gain"]))
     cfg = {"homography_adaptation": HA_CFG, "model": MP_MODEL}
     r = O.homography_adaptation(sd, torch.from_numpy(g["image"]), cfg, homographies=torch.from_numpy(g["H"]))
-    assert np.array_equal(r["mean_prob"].numpy(), g["agg"])
-    assert np.array_equal(r["nms_prob"].numpy(), g["nms"])
+    assert_conv_close(r["mean_prob"].numpy(), g["agg"], "agg")
+    assert_conv_close(r["nms_prob"].numpy(), g["nms"], "nms")
     assert r["keypoints"].dtype == np.int64 and np.array_equal(r["keypoints"], g["keypoints"])
     # drawing the homographies from numpy's global RNG in the reference's order reproduces them too
     np.random.seed(int(g["np_seed"]))
@@ -205,14 +222,14 @@ def test_ha_export_variants_match_reference(golden):
     img = torch.from_numpy(g["image"])
     r = O.homography_adaptation(sd, img, {"homography_adaptation": dict(HA_CFG, aggregation="max"), "model": MP_MODEL},
                                 homographies=torch.from_numpy(g["max_H"]))
-    assert np.array_equal(r["mean_prob"].numpy(), g["max_agg"][0] if g["max_agg"].ndim == 3 else g["max_agg"])
+    assert_conv_close(r["mean_prob"].numpy(), g["max_agg"][0] if g["max_agg"].ndim == 3 else g["max_agg"], "max_agg")
     assert np.array_equal(r["keypoints"], g["max_keypoints"])
     np.random.seed(int(g["np_seed"]))           # the same homographies from numpy's global RNG in the reference's order
     r2 = O.homography_adaptation(sd, img, {"homography_adaptation": dict(HA_CFG, aggregation="max"), "model": MP_MODEL})
     assert np.array_equal(r2["homographies"].numpy(), g["max_H"]) and np.array_equal(r2["keypoints"], g["max_keypoints"])
     r3 = O.homography_adaptation(sd, img, {"homography_adaptation": dict(HA_CFG, num=1), "model": MP_MODEL})
     assert g["noha_H"].shape[0] == 0
-    assert np.array_equal(r3["mean_prob"].numpy(), g["noha_agg"][0] if g["noha_agg"].ndim == 3 else g["noha_agg"])
+    assert_conv_close(r3["mean_prob"].numpy(), g["noha_agg"][0] if g["noha_agg"].ndim == 3 else g["noha_agg"], "noha_agg")
     assert np.array_equal(r3["keypoints"], g["noha_keypoints"])
     assert len(g["max_keypoints"]) != len(g["noha_keypoints"])
 
@@ -242,6 +259,6 @@ def test_hpatches_export_values_match_reference(golden):
     pts = g["des_pts"]
     for img_key, prob_key, desc_key in (("image", "rep_prob", "des_desc_at_pts"), ("warped_image", "rep_warped_prob", "des_warped_desc_at_pts")):
         out = O.model_forward(sd, torch.from_numpy(g[img_key]), SP_MODEL)
-        assert np.array_equal(out["detector_output"]["prob_heatmap_nms"][0].numpy(), g[prob_key])
+        assert_conv_close(out["detector_output"]["prob_heatmap_nms"][0].numpy(), g[prob_key], prob_key)
         desc = out["descriptor_output"]["desc"][0].numpy().transpose(1, 2, 0)
-        assert np.array_equal(desc[pts[:, 0], pts[:, 1]], g[desc_key])
+        assert_conv_close(desc[pts[:, 0], pts[:, 1]], g[desc_key], desc_key)

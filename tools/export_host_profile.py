@@ -1,7 +1,7 @@
-import copy, sys, tempfile, time, cProfile, pstats, io
+import os, copy, sys, tempfile, time, cProfile, pstats, io
 from pathlib import Path
 import torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from superpoint_nerf_pytorch_b200 import settings
 from superpoint_nerf_pytorch_b200.engine import SyntheticLoader

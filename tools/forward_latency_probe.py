@@ -1,6 +1,6 @@
-import copy, sys, time, torch
-sys.path.insert(0, '/root/repo')
-sys.path.insert(0, '/root/repo/tests')
+import os, copy, sys, time, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'tests'))
 from conftest import SP_MODEL
 from superpoint_nerf_pytorch_b200.utils.get_model import get_model
 c = copy.deepcopy(SP_MODEL); c["precision"] = "f16"; c["detector_head"]["top_k"] = 1000

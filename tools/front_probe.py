@@ -1,6 +1,6 @@
 """Bottleneck experiments on front_tc_kernel: time it with parts of each role switched off (SPN_FRONT_DBG bits)."""
 import os, sys, copy, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from superpoint_nerf_pytorch_b200.utils.get_model import get_model
 dev = torch.device('cuda', 0)

@@ -1,6 +1,6 @@
 """Times (and, under ncu, exposes) the mask and aggregate kernels alone on the bench workload's geometry."""
-import sys, copy, time, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, copy, time, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from superpoint_nerf_pytorch_b200 import _native
 

@@ -1,6 +1,6 @@
 """Per-kernel time of box_nms (+ top-k) for a single image and for a batch, from the context's CUDA-event profile."""
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from superpoint_nerf_pytorch_b200 import _native
 ctx = _native.Context(0)
 dev = torch.device('cuda', 0)

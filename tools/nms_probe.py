@@ -1,5 +1,5 @@
-import sys, copy, torch, time
-sys.path.insert(0,'/root/repo')
+import os, sys, copy, torch, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from superpoint_nerf_pytorch_b200.engine_solvers.export import HomographyAdaptation
 from superpoint_nerf_pytorch_b200.utils.get_model import get_model
