@@ -62,12 +62,9 @@ SPN_API int spn_version(void);
 SPN_API int spn_create(spn_ctx** out, int device);
 SPN_API int spn_destroy(spn_ctx* ctx);
 
-/* A/B switches of the tensor-core path (read when a launch is planned, never from the environment): "fold" (3x3 layers
- * with the horizontal taps folded into N = 192), "fuse_front" (warp + block_1 + block_2 in one kernel), "fuse_head"
- * (convPb + softmax + depth-to-space in one kernel), "pdl" (programmatic dependent launch): all default to 1.
- * Kept for A/B, default 0 (both measured slower): "front_pair" (the fused front end as a 2-CTA cluster with
- * cta_group::2 MMAs), "fold_hybrid" (64-channel-input folded layers with kx = 2 as a separate shifted N = 64 MMA).
- * "ws_guard" (default 0): see spn_check_guards. */
+/* Options of the tensor-core path (read when a launch is planned, never from the environment): "fuse_front" (warp +
+ * block_1 + block_2 in one kernel) and "fuse_head" (convPb + softmax + depth-to-space in one kernel), both default 1;
+ * 0 selects the unfused kernels.  "ws_guard" (default 0): see spn_check_guards.  Any other name is SPN_E_INVALID. */
 SPN_API int spn_set_option(spn_ctx* ctx, const char* name, int value);
 
 /* BN fold + pack + upload of one VGG_Block (conv2d + BatchNorm2d eval, eps as given).

@@ -159,7 +159,7 @@ class Context:
             pass
 
     def set_option(self, name: str, value: int):
-        """A/B switches of the tensor-core path: 'fold', 'fuse_front', 'fuse_head', 'pdl' (all default 1)."""
+        """Options of the tensor-core path: 'fuse_front', 'fuse_head' (default 1), 'ws_guard' (default 0)."""
         self._call("spn_set_option", self.handle, name.encode(), int(value))
 
     @property

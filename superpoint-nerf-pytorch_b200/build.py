@@ -7,14 +7,13 @@ No torch involvement: plain `nvcc -shared`.  The .so is git-ignored but travels 
 from __future__ import annotations
 
 import subprocess
-import os
 import sys
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 CSRC = HERE / "csrc"
 SO = HERE / "libspn_b200.so"
-SOURCES = ["spn_api.cu", "conv_fp32.cu", "conv_tc.cu", "conv_fold.cu", "conv_split.cu", "front_tc.cu", "front2_tc.cu", "head_tc.cu", "geometry.cu", "nms.cu", "desc.cu", "eval.cu", "labels.cu"]
+SOURCES = ["spn_api.cu", "conv_fp32.cu", "conv_tc.cu", "conv_fold.cu", "conv_split.cu", "front_tc.cu", "head_tc.cu", "geometry.cu", "nms.cu", "desc.cu", "eval.cu", "labels.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 
@@ -37,8 +36,6 @@ def build(force: bool = False, verbose: bool = False) -> Path:
     for src in SOURCES:
         obj = bdir / (src + ".o")
         cmd = ["nvcc", *[f for f in NVCC_FLAGS if f != "--use_fast_math=false"], "-c", str(CSRC / src), "-o", str(obj)]
-        if os.environ.get("SPN_FRONT_DBG_BUILD"):   # extra front_tc_kernel instantiations for tools/front_probe.py
-            cmd.insert(1, "-DSPN_FRONT_DBG_BUILD")
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))

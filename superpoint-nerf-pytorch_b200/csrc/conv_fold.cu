@@ -49,15 +49,8 @@ struct FoldParams {
   const void* wimg;    // per slice: [cin block][ky 3][k-step 4][chunk 2][n = kx*64+co 192][8] + bias block [2][192][8]
 };
 
-// HYB (64-channel inputs): with one 64-channel block a tile is only 13 MMAs and the kernel is bound by the epilogues'
-// TMEM reads (3 x 64 fp32 columns per pixel = 96 KB per tile at 64 B/cycle = 1536 cycles against 1248 of MMA).  The
-// hybrid form keeps kx = 0, 1 folded (one N = 128 MMA on the unshifted pixel) and issues kx = 2 as a second N = 64 MMA on
-// the slab shifted by one pixel, accumulating straight into the kx = 1 columns:  out(x) = F0(x-1) + F1'(x).  12 x (64 +
-// 48) + 64 = 1408 MMA cycles, 64 KB of TMEM reads and one shuffle per value instead of two.
-template <bool HYB>
 __global__ void __launch_bounds__(kThreads, 1)
 conv_fold_kernel(const __grid_constant__ CUtensorMap tmap, const FoldParams p) {
-  constexpr uint32_t kAccCols = HYB ? 128u : 192u;   // TMEM columns per accumulator
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ __align__(8) uint64_t bar_full[kMaxStages], bar_empty[kMaxStages], bar_w, bar_tfull[2], bar_tempty[2];
   __shared__ uint32_t tmem_base_s;
@@ -125,8 +118,7 @@ conv_fold_kernel(const __grid_constant__ CUtensorMap tmap, const FoldParams p) {
     // tile = 12 MMAs) are therefore taken in the middle of the current unit's MMAs, and the commits at its end:
     // two short bookkeeping stretches per unit, each covered by the MMAs already queued.
     const uint32_t fmt = p.is_bf16 ? 1u : 0u;
-    const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((kAccCols >> 3) << 17) | ((128u >> 4) << 24);  // N 192 (128), M 128
-    const uint32_t idesc64 = (1u << 4) | (fmt << 7) | (fmt << 10) | ((64u >> 3) << 17) | ((128u >> 4) << 24);       // HYB: the kx = 2 MMA
+    const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((192u >> 3) << 17) | ((128u >> 4) << 24);  // N 192, M 128
     const uint32_t a_hi = (128u >> 4) | (1u << 14);                 // A: SBO = 128 B (8 consecutive pixels)
     const uint32_t a_lo_c = (kChStride >> 4) << 16;                 //    LBO = 8-channel group stride
     const uint32_t b_hi = (128u >> 4) | (1u << 14);                 // B: SBO = 128 B (8 consecutive n)
@@ -146,7 +138,7 @@ conv_fold_kernel(const __grid_constant__ CUtensorMap tmap, const FoldParams p) {
     for (int u = 0; u < n_units; ++u) {
       const int acc = i & 1;
       const bool last_cb = cb == p.cin_blocks - 1;
-      const uint32_t d_tmem = tmem_base + (uint32_t)acc * kAccCols;
+      const uint32_t d_tmem = tmem_base + (uint32_t)acc * 192;
       const uint32_t a_lo = ((slab_addr + (uint32_t)stage * kSlabBytes) >> 4) | a_lo_c;
       const uint32_t b_lo = ((w_addr + (uint32_t)cb * (12 * kBlkBytes)) >> 4) | b_lo_c;
       if (elect_one()) {
@@ -156,8 +148,6 @@ conv_fold_kernel(const __grid_constant__ CUtensorMap tmap, const FoldParams p) {
           const uint32_t aoff = ((uint32_t)ky * (kTWs * 16) + (uint32_t)kk * 2 * kChStride) >> 4;
           const uint32_t boff = ((uint32_t)(ky * 4 + kk) * kBlkBytes) >> 4;
           umma_f16_2w(d_tmem, a_lo + aoff, a_hi, b_lo + boff, b_hi, idesc, (cb | m) ? 1u : 0u);
-          // kx = 2 on the pixel to the right (+16 B in the slab), weights = rows 128..191 of the same block, into F1
-          if (HYB) umma_f16_2w(d_tmem + 64, a_lo + aoff + 1, a_hi, b_lo + boff + ((128u * 16u) >> 4), b_hi, idesc64, 1u);
         }
       }
       __syncwarp();
@@ -179,7 +169,6 @@ conv_fold_kernel(const __grid_constant__ CUtensorMap tmap, const FoldParams p) {
           const uint32_t aoff = ((uint32_t)ky * (kTWs * 16) + (uint32_t)kk * 2 * kChStride) >> 4;
           const uint32_t boff = ((uint32_t)(ky * 4 + kk) * kBlkBytes) >> 4;
           umma_f16_2w(d_tmem, a_lo + aoff, a_hi, b_lo + boff, b_hi, idesc, 1u);
-          if (HYB) umma_f16_2w(d_tmem + 64, a_lo + aoff + 1, a_hi, b_lo + boff + ((128u * 16u) >> 4), b_hi, idesc64, 1u);
         }
         umma_commit(&bar_empty[stage]);
         if (last_cb) {
@@ -214,25 +203,22 @@ conv_fold_kernel(const __grid_constant__ CUtensorMap tmap, const FoldParams p) {
       const int y = ty * kTH + r, gx = tx * kTWv - 1 + x;
       mbar_wait(&bar_tfull[acc], acc_phase);
       tc_fence_after();
-      const uint32_t taddr = tmem_base + (uint32_t)acc * kAccCols + ((uint32_t)(q * 32) << 16);
+      const uint32_t taddr = tmem_base + (uint32_t)acc * 192 + ((uint32_t)(q * 32) << 16);
       uint32_t h2[32];
 #pragma unroll
       for (int c0 = 0; c0 < 64; c0 += 32) {
-        uint32_t f0[32], f1[32], f2[HYB ? 1 : 32];
+        uint32_t f0[32], f1[32], f2[32];
         tmem_ld32(taddr + c0, f0);
         tmem_ld32(taddr + 64 + c0, f1);
-        if (!HYB) tmem_ld32(taddr + 128 + c0, f2);
+        tmem_ld32(taddr + 128 + c0, f2);
         tmem_ld_wait();
 #pragma unroll
         for (int c = 0; c < 32; c += 2) {
-          // out(x) = F(x-1, kx=0) + F(x, kx=1) + F(x+1, kx=2): neighbours are lane-1 / lane+1 (same tile row for x in 1..14);
-          // HYB: the kx = 2 term is already inside F1
+          // out(x) = F(x-1, kx=0) + F(x, kx=1) + F(x+1, kx=2): neighbours are lane-1 / lane+1 (same tile row for x in 1..14)
           float a = __shfl_up_sync(0xffffffffu, __uint_as_float(f0[c]), 1) + __uint_as_float(f1[c]);
           float b = __shfl_up_sync(0xffffffffu, __uint_as_float(f0[c + 1]), 1) + __uint_as_float(f1[c + 1]);
-          if (!HYB) {
-            a += __shfl_down_sync(0xffffffffu, __uint_as_float(f2[c]), 1);
-            b += __shfl_down_sync(0xffffffffu, __uint_as_float(f2[c + 1]), 1);
-          }
+          a += __shfl_down_sync(0xffffffffu, __uint_as_float(f2[c]), 1);
+          b += __shfl_down_sync(0xffffffffu, __uint_as_float(f2[c + 1]), 1);
           h2[(c0 + c) >> 1] = p.relu ? pack2_relu(a, b, p.is_bf16) : pack2(a, b, p.is_bf16);   // ReLU commutes with the pool below
         }
       }
@@ -267,23 +253,6 @@ conv_fold_kernel(const __grid_constant__ CUtensorMap tmap, const FoldParams p) {
   }
 }
 
-uint16_t to16h(float f, int bf16) {
-  if (bf16) {
-    __nv_bfloat16 h = __float2bfloat16_rn(f);
-    return *reinterpret_cast<uint16_t*>(&h);
-  }
-  __half h = __float2half_rn(f);
-  return *reinterpret_cast<uint16_t*>(&h);
-}
-float from16h(uint16_t h, int bf16) {
-  if (bf16) return __bfloat162float(*reinterpret_cast<__nv_bfloat16*>(&h));
-  return __half2float(*reinterpret_cast<__half*>(&h));
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 }  // namespace
 
 // operand-B image of a 3x3 layer for conv_fold_kernel (both 16-bit types)
@@ -306,16 +275,16 @@ int spn_fold_pack_layer(spn_ctx* ctx, int layer, const float* h_wfold, const flo
                   for (int e = 0; e < 8; ++e) {
                     const int c = sl * 64 + co, ci = cb * 64 + kk * 16 + j * 8 + e;
                     if (c < L.cout)
-                      blk[((size_t)j * 192 + kx * 64 + co) * 8 + e] = to16h(h_wfold[((size_t)c * L.cin + ci) * 9 + ky * 3 + kx], bf);
+                      blk[((size_t)j * 192 + kx * 64 + co) * 8 + e] = to16(h_wfold[((size_t)c * L.cin + ci) * 9 + ky * 3 + kx], bf);
                   }
           }
       uint16_t* bb = base + (size_t)cbs * 12 * (kBlkBytes / 2);  // bias block: n = 64 + co (kx = 1), k 0 / 1 = hi / lo
       for (int co = 0; co < 64; ++co) {
         const int c = sl * 64 + co;
         if (c < L.cout) {
-          const uint16_t hi = to16h(h_bfold[c], bf);
+          const uint16_t hi = to16(h_bfold[c], bf);
           bb[((size_t)64 + co) * 8] = hi;
-          bb[((size_t)64 + co) * 8 + 1] = to16h(h_bfold[c] - from16h(hi, bf), bf);
+          bb[((size_t)64 + co) * 8 + 1] = to16(h_bfold[c] - from16(hi, bf), bf);
         }
       }
     }
@@ -331,8 +300,6 @@ int spn_launch_conv_fold(spn_ctx* ctx, int layer, int mode, const void* in, void
   const SpnLayer& L = ctx->layers[layer];
   const int bf = mode == SPN_MODE_BF16 ? 1 : 0;
   if (!L.w16f[bf]) { spn_set_error("layer %d has no folded tensor-core weights", layer); return SPN_E_STATE; }
-  EncodeTiledFn encode = (EncodeTiledFn)spn_tc_encode_fn(ctx);
-  if (!encode) return SPN_E_CUDA;
   FoldParams p;
   memset(&p, 0, sizeof(p));
   p.n_img = n_img; p.H = H; p.W = W;
@@ -349,27 +316,16 @@ int spn_launch_conv_fold(spn_ctx* ctx, int layer, int mode, const void* in, void
   const size_t dyn = (size_t)wres + (size_t)p.stages * kSlabBytes + 1024;
 
   CUtensorMap tmap;
-  const cuuint64_t dims[4] = {(cuuint64_t)W * 8, (cuuint64_t)H, (cuuint64_t)(L.cin / 8), (cuuint64_t)n_img};
-  const cuuint64_t strides[3] = {(cuuint64_t)W * 16, (cuuint64_t)H * W * 16, (cuuint64_t)(L.cin / 8) * H * W * 16};
-  const cuuint32_t box[4] = {(cuuint32_t)kTWs * 8, (cuuint32_t)kPH, 8, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult cr = encode(&tmap, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(in), dims,
-                       strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) {
-    spn_set_error("cuTensorMapEncodeTiled failed (%d) for layer %d, %dx%dx%d", (int)cr, layer, L.cin, H, W);
-    return SPN_E_CUDA;
-  }
-  const bool hyb = p.cin_blocks == 1 && ctx->opt_fold_hybrid;
-  void (*kern)(const CUtensorMap, const FoldParams) = hyb ? conv_fold_kernel<true> : conv_fold_kernel<false>;
-  SPN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+  int rc = spn_c8_tensor_map(ctx, &tmap, in, n_img, L.cin, H, W, kTWs, kPH, bf);
+  if (rc) return rc;
+  SPN_CUDA(cudaFuncSetAttribute(conv_fold_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
   const long long work = (long long)n_img * p.tiles_x * p.tiles_y * p.cout_slices;
   int grid = ctx->sm_count;
   if (work < grid) grid = (int)work;
   grid = grid / p.cout_slices * p.cout_slices;
   if (grid < p.cout_slices) grid = p.cout_slices;
   SpnProfScope prof(ctx, layer, s);
-  SPN_CUDA(spn_launch_pdl(ctx->opt_pdl != 0, kern, dim3(grid), dim3(kThreads), dyn, s, tmap, p));
+  SPN_CUDA(spn_launch_pdl(conv_fold_kernel, dim3(grid), dim3(kThreads), dyn, s, tmap, p));
   SPN_CHECK_LAUNCH(ctx);
   return SPN_OK;
 }

@@ -3,7 +3,7 @@
 // conv: VGG_Block.forward = conv(k, stride 1, pad k/2) + BN(eval) + ReLU + MaxPool(2,2)
 //       (reference models/model_utils/VGG_Backbone.py:23-36) with BN folded into the weights.
 //       NCHW fp32 in and out, i.e. the reference's own layout.  This is the 1e-4 parity path; the
-//       throughput path is the tcgen05 implicit GEMM in conv_tc.cu.
+//       throughput path is the tcgen05 implicit GEMM in front_tc.cu / conv_fold.cu / conv_tc.cu.
 // softmax_d2s: Detector_head.forward lines heads.py:25-28 (softmax over 65, drop channel 64,
 //       pixel_shuffle(8), squeeze) optionally multiplied by the validity mask (export.py:70).
 #include "spn_common.cuh"

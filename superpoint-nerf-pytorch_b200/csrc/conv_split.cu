@@ -26,10 +26,6 @@ namespace {
 
 using namespace tcptx;
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
   const __half ha = __float2half_rn(a), hb = __float2half_rn(b);
   const __half la = __float2half_rn(a - __half2float(ha)), lb = __float2half_rn(b - __half2float(hb));
@@ -465,26 +461,7 @@ __global__ void c8_split_to_nchw_kernel(const void* __restrict__ hi, const void*
   }
 }
 
-uint16_t h16(float f) {
-  __half h = __float2half_rn(f);
-  return *reinterpret_cast<uint16_t*>(&h);
-}
-float f16(uint16_t h) { return __half2float(*reinterpret_cast<__half*>(&h)); }
-
 int fold_nco(const SpnLayer& L) { return L.cin == 64 ? 64 : 32; }
-
-int make_tmap(spn_ctx* ctx, CUtensorMap* tm, const void* base, int cin, int n_img, int H, int W, int box_w, int box_h) {
-  EncodeTiledFn encode = (EncodeTiledFn)spn_tc_encode_fn(ctx);
-  if (!encode) return SPN_E_CUDA;
-  const cuuint64_t dims[4] = {(cuuint64_t)W * 8, (cuuint64_t)H, (cuuint64_t)(cin / 8), (cuuint64_t)n_img};
-  const cuuint64_t strides[3] = {(cuuint64_t)W * 16, (cuuint64_t)H * W * 16, (cuuint64_t)(cin / 8) * H * W * 16};
-  const cuuint32_t box[4] = {(cuuint32_t)box_w * 8, (cuuint32_t)box_h, 8, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult cr = encode(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                       CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) { spn_set_error("cuTensorMapEncodeTiled failed (%d) in the split path", (int)cr); return SPN_E_CUDA; }
-  return SPN_OK;
-}
 
 // one 3x3 layer: (in_hi, in_lo) C8 -> (out_hi, out_lo) C8 (pooled or not)
 int launch_split_fold(spn_ctx* ctx, int layer, const void* in_hi, const void* in_lo, void* out_hi, void* out_lo, int n_img, int H, int W,
@@ -505,9 +482,9 @@ int launch_split_fold(spn_ctx* ctx, int layer, const void* in_hi, const void* in
   p.out_hi = out_hi; p.out_lo = out_lo; p.wimg = L.w16x;
   const size_t dyn = (size_t)wres + (size_t)p.stages * kSlabBytes + 1024;
   CUtensorMap th, tl;
-  int rc = make_tmap(ctx, &th, in_hi, L.cin, n_img, H, W, kTWs, kPH);
+  int rc = spn_c8_tensor_map(ctx, &th, in_hi, n_img, L.cin, H, W, kTWs, kPH, 0);
   if (rc) return rc;
-  if ((rc = make_tmap(ctx, &tl, in_lo, L.cin, n_img, H, W, kTWs, kPH))) return rc;
+  if ((rc = spn_c8_tensor_map(ctx, &tl, in_lo, n_img, L.cin, H, W, kTWs, kPH, 0))) return rc;
   const long long work = (long long)n_img * p.tiles_x * p.tiles_y * p.cout_slices;
   int grid = ctx->sm_count;
   if (work < grid) grid = (int)work;
@@ -541,9 +518,9 @@ int launch_split_1x1(spn_ctx* ctx, int layer, const void* in_hi, const void* in_
   p.out = out; p.wimg = L.w16x;
   const size_t dyn = (size_t)wres + (size_t)p.stages * kSlab1 + 1024;
   CUtensorMap th, tl;
-  int rc = make_tmap(ctx, &th, in_hi, L.cin, n_img, H, W, kTW1, kTH1);
+  int rc = spn_c8_tensor_map(ctx, &th, in_hi, n_img, L.cin, H, W, kTW1, kTH1, 0);
   if (rc) return rc;
-  if ((rc = make_tmap(ctx, &tl, in_lo, L.cin, n_img, H, W, kTW1, kTH1))) return rc;
+  if ((rc = spn_c8_tensor_map(ctx, &tl, in_lo, n_img, L.cin, H, W, kTW1, kTH1, 0))) return rc;
   const long long work = (long long)n_img * p.tiles_x * p.tiles_y * p.cout_slices;
   int grid = ctx->sm_count;
   if (work < grid) grid = (int)work;
@@ -579,8 +556,8 @@ int spn_split_pack_layer(spn_ctx* ctx, int layer, const float* w, const float* b
   if (L.w16x) { cudaFree(L.w16x); L.w16x = nullptr; }
   if (L.cin % 64 != 0) return SPN_OK;
   std::vector<uint16_t> img;
-  auto hi_of = [&](float v) { return h16(v); };
-  auto lo_of = [&](float v) { return h16(v - f16(h16(v))); };
+  auto hi_of = [&](float v) { return to16(v, 0); };
+  auto lo_of = [&](float v) { return to16(v - from16(to16(v, 0), 0), 0); };
   if (L.ks == 3) {
     const int nco = fold_nco(L), N = 3 * nco, blk = 2 * N * 8 /* halfs */, cbs = L.cin / 64, slices = (L.cout + nco - 1) / nco;
     const size_t per_slice = (size_t)(2 * cbs * 12 + 1) * blk;

@@ -1,24 +1,21 @@
-// tcgen05 implicit-GEMM convolutions (fast path): VGG_Block.forward (reference VGG_Backbone.py:23-36) for the 3x3
-// layers with Cin >= 64 and the 1x1 heads, fp16/bf16 operands, fp32 accumulation in TMEM.
+// tcgen05 1x1 convolution with fp32 NCHW output: the 1x1 heads convDb and, on the unfused path (option fuse_head = 0),
+// convPb, and the single-layer entry point spn_conv_layer for 1x1 layers.  fp16/bf16 operands, fp32 accumulation in TMEM.
+// The 3x3 layers run in conv_fold.cu (block_3..8, convPa, convDa) and front_tc.cu (block_1 + block_2).
 //
 // Data layout in HBM ("C8"): act[n][C/8][H][W][8] halfs - i.e. 16-byte channel groups, pixels contiguous along W.
 // This is exactly the UMMA no-swizzle K-major operand layout (core matrix = 8 rows x 16 bytes), so ONE TMA box
-//   (W: TW+2 pixels) x (H: TH+2 rows) x (8 channel groups)               [halo tile of 64 input channels]
-// lands in shared memory as slab[chunk][row][col][8] and all nine filter taps are read from it by nine UMMA
-// descriptors that differ only in their start address (+ (ky*PW + kx) * 16 bytes): the im2col matrix is never
-// materialised and each activation byte crosses L2->SMEM 1.4x (halo) instead of 9x.  TMA zero-fills outside the
-// image, which is the convolution's zero padding.
+//   (W: 8 pixels) x (H: 16 rows) x (8 channel groups)                    [tile of 64 input channels]
+// lands in shared memory as slab[chunk][row][col][8] and is read directly as operand A.
 //
 // GEMM view per CTA tile: M = 128 pixels (8 wide x 16 high; TMEM lane = pixel), N = 64 output channels (one
-// "slice"; a CTA keeps its slice's weights for all K resident in SMEM), K = 9 * Cin.  MMA = tcgen05.mma
+// "slice"; a CTA keeps its slice's weights for all K resident in SMEM), K = Cin.  MMA = tcgen05.mma
 // cta_group::1 kind::f16 M128 N64 K16, A and B from SMEM descriptors (SWIZZLE_NONE, LBO = channel-group stride,
 // SBO = 8-row-group stride), D = 64 fp32 TMEM columns, double buffered so the epilogue of tile i overlaps the MMAs
 // of tile i+1.
 //
 // Warp roles (192 threads, persistent, one CTA per SM): warp 0 = TMA producer (weights once via cp.async.bulk,
-// then one 23 KB slab per (tile, 64-channel block) through a ring of mbarriers), warp 1 = MMA issuer (one elected
-// lane) + TMEM allocator, warps 2-5 = epilogue (tcgen05.ld -> bias -> ReLU -> 2x2 max-pool by shuffles -> 16-byte
-// coalesced C8 stores, or fp32 NCHW stores for the heads).
+// then one 16 KB slab per (tile, 64-channel block) through a ring of mbarriers), warp 1 = MMA issuer (one elected
+// lane) + TMEM allocator, warps 2-5 = epilogue (tcgen05.ld -> optional ReLU -> fp32 NCHW stores).
 #include <cuda.h>
 
 #include <string>
@@ -33,7 +30,9 @@ using namespace tcptx;
 
 constexpr int kTW = 8, kTH = 16;              // output tile: 8 x 16 pixels = 128 GEMM rows
 constexpr int kThreads = 192;
-constexpr int kWBlockBytes = 8192;            // weights of one (cin block, tap): 4 k-steps x 2 chunks x 64 cout x 16 B
+constexpr int kWBlockBytes = 8192;            // weights of one cin block: 4 k-steps x 2 chunks x 64 cout x 16 B
+constexpr int kSlabBytes = 8 * kTH * kTW * 16;  // one TMA box: 8 channel groups x 16 rows x 8 pixels x 16 B
+constexpr uint32_t kChStride = (uint32_t)kTH * kTW * 16;  // bytes between 8-channel groups inside a slab
 constexpr int kMaxStages = 6;
 constexpr int kBiasBlockBytes = 2048;         // bias as operand B: [chunk 2][cout 64][8], k 0 / 1 = hi / lo halves
 constexpr int kOnesBytes = 4096;              // constant operand A of the bias MMA: [chunk 2][128 rows][8]
@@ -43,16 +42,12 @@ struct TcParams {
   int cin_blocks;         // Cin / 64
   int cout_slices;        // ceil(Cout / 64)
   int cout;               // real number of output channels
-  int taps;               // 9 (3x3, halo 1) or 1 (1x1)
-  int relu, pool;
-  int out_mode;           // 0: C8 half/bf16   1: NCHW fp32
+  int relu;
   int is_bf16;
   int tiles_x, tiles_y;
   int stages;
-  int stage_bytes;        // slab bytes rounded up to 1024
-  int slab_bytes;         // exact TMA transaction bytes
-  void* out;
-  const void* wimg;       // [cout_slices][cin_blocks][taps][4][2][64][8] halfs
+  float* out;             // NCHW fp32 [n][cout][H][W]
+  const void* wimg;       // [cout_slices][cin_blocks][4][2][64][8] halfs + per slice the bias block
 };
 
 // Constant A operand of the bias MMA: row r = (1, 1, 0, ..., 0) in K chunk 0, zeros in chunk 1.
@@ -64,18 +59,14 @@ __device__ __forceinline__ void fill_ones_operand(uint8_t* ones, int is_bf16, in
 }
 
 // ------------------------------------------------------------------------------------------------ main kernel
-template <int TAPS>
 __global__ void __launch_bounds__(kThreads, 1)
-conv_tc_kernel(const __grid_constant__ CUtensorMap tmap, const TcParams p) {
+conv1x1_tc_kernel(const __grid_constant__ CUtensorMap tmap, const TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ __align__(8) uint64_t bar_full[kMaxStages], bar_empty[kMaxStages], bar_w, bar_tfull[2], bar_tempty[2];
   __shared__ uint32_t tmem_base_s;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  constexpr int halo = TAPS == 9 ? 1 : 0;
-  constexpr int PW = kTW + 2 * halo, PH = kTH + 2 * halo;
-  constexpr uint32_t ch_stride = (uint32_t)PH * PW * 16;  // bytes between 8-channel groups inside a slab
-  const int wbytes = p.cin_blocks * TAPS * kWBlockBytes + kBiasBlockBytes;
+  const int wbytes = p.cin_blocks * kWBlockBytes + kBiasBlockBytes;
   uint8_t* wsm = smem;                                    // this CTA's weight slice (+ bias block), resident
   uint8_t* ones = smem + ((wbytes + 1023) & ~1023);       // constant A operand of the bias MMA
   uint8_t* slab0 = ones + kOnesBytes;
@@ -117,9 +108,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmap, const TcParams p) {
       for (int cb = 0; cb < p.cin_blocks; ++cb) {
         mbar_wait(&bar_empty[stage], phase ^ 1);
         if (elect_one()) {
-          mbar_expect_tx(&bar_full[stage], (uint32_t)p.slab_bytes);
-          tma_load_4d(slab0 + (size_t)stage * p.stage_bytes, &tmap, &bar_full[stage], (tx * kTW - halo) * 8,
-                      ty * kTH - halo, cb * 8, n);
+          mbar_expect_tx(&bar_full[stage], (uint32_t)kSlabBytes);
+          tma_load_4d(slab0 + (size_t)stage * kSlabBytes, &tmap, &bar_full[stage], tx * kTW * 8, ty * kTH, cb * 8, n);
         }
         __syncwarp();
         if (++stage == p.stages) { stage = 0; phase ^= 1; }
@@ -130,9 +120,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmap, const TcParams p) {
     // instruction descriptor: D=f32, A=B=f16|bf16, both K-major, N=64, M=128
     const uint32_t fmt = p.is_bf16 ? 1u : 0u;
     const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((64u >> 3) << 17) | ((128u >> 4) << 24);
-    // operand A (slab): LBO = stride between 8-channel groups, SBO = stride between 8-pixel rows of the halo tile;
+    // operand A (slab): LBO = stride between 8-channel groups, SBO = stride between 8-pixel rows of the tile;
     // operand B (weights): LBO = 1024 B between the two K chunks, SBO = 128 B between groups of 8 output channels
-    const uint32_t a_lbo = ch_stride, a_sbo = (uint32_t)PW * 16;
+    const uint32_t a_lbo = kChStride, a_sbo = (uint32_t)kTW * 16;
     const uint32_t b_lbo = 1024u, b_sbo = 128u;
     const uint32_t a_hi = (a_sbo >> 4) | (1u << 14), b_hi = (b_sbo >> 4) | (1u << 14);  // SBO | descriptor version 1
     const uint32_t a_lo_c = (a_lbo >> 4) << 16, b_lo_c = (b_lbo >> 4) << 16;
@@ -147,24 +137,20 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmap, const TcParams p) {
       for (int cb = 0; cb < p.cin_blocks; ++cb) {
         mbar_wait(&bar_full[stage], phase);
         tc_fence_after();
-        const uint32_t a_lo = ((slab_addr + (uint32_t)stage * p.stage_bytes) >> 4) | a_lo_c;
-        const uint32_t b_lo = ((w_addr + (uint32_t)cb * (TAPS * kWBlockBytes)) >> 4) | b_lo_c;
+        const uint32_t a_lo = ((slab_addr + (uint32_t)stage * kSlabBytes) >> 4) | a_lo_c;
+        const uint32_t b_lo = ((w_addr + (uint32_t)cb * kWBlockBytes) >> 4) | b_lo_c;
         if (elect_one()) {
 #pragma unroll
-          for (int tap = 0; tap < TAPS; ++tap) {
-            const int ky = TAPS == 9 ? tap / 3 : 0, kx = TAPS == 9 ? tap % 3 : 0;
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk) {
-              const uint32_t aoff = ((uint32_t)(ky * PW + kx) * 16 + (uint32_t)kk * 2 * ch_stride) >> 4;
-              const uint32_t boff = ((uint32_t)tap * kWBlockBytes + (uint32_t)kk * 2048) >> 4;
-              umma_f16_2w(d_tmem, a_lo + aoff, a_hi, b_lo + boff, b_hi, idesc, (cb | tap | kk) ? 1u : 0u);
-            }
+          for (int kk = 0; kk < 4; ++kk) {
+            const uint32_t aoff = ((uint32_t)kk * 2 * kChStride) >> 4;
+            const uint32_t boff = ((uint32_t)kk * 2048) >> 4;
+            umma_f16_2w(d_tmem, a_lo + aoff, a_hi, b_lo + boff, b_hi, idesc, (cb | kk) ? 1u : 0u);
           }
           umma_commit(&bar_empty[stage]);  // frees the slab once these MMAs have read it
           if (cb == p.cin_blocks - 1) {
             // + bias: D += ones[128 x 16] . biasB[64 x 16]  (k 0/1 = hi/lo halves of the folded bias)
             const uint32_t o_lo = (smem_u32(ones) >> 4) | ((2048u >> 4) << 16);
-            const uint32_t bb_lo = ((w_addr + (uint32_t)p.cin_blocks * (TAPS * kWBlockBytes)) >> 4) | b_lo_c;
+            const uint32_t bb_lo = ((w_addr + (uint32_t)p.cin_blocks * kWBlockBytes) >> 4) | b_lo_c;
             umma_f16_2w(d_tmem, o_lo, (128u >> 4) | (1u << 14), bb_lo, b_hi, idesc, 1u);
             umma_commit(&bar_tfull[acc]);  // accumulator complete -> epilogue
           }
@@ -195,48 +181,14 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmap, const TcParams p) {
       mbar_arrive(&bar_tempty[acc]);  // TMEM accumulator is free again
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
 
-      if (p.out_mode == 0) {
-        // bias + ReLU -> packed 16-bit pairs -> optional 2x2 max-pool -> 16-byte stores of 8 channels
-        uint32_t h2[32];
+      if (y < p.H && x < p.W) {
 #pragma unroll
-        for (int c = 0; c < 32; ++c) {
-          h2[c] = pack2(__uint_as_float(v[2 * c]), __uint_as_float(v[2 * c + 1]), p.is_bf16);  // bias is already in D
-        }
-        int oy = y, ox = x, Ho = p.H, Wo = p.W;
-        bool writer = (y < p.H) && (x < p.W);
-        if (p.pool) {
-#pragma unroll
-          for (int c = 0; c < 32; ++c) {
-            h2[c] = max2(h2[c], __shfl_xor_sync(0xffffffffu, h2[c], 1), p.is_bf16);
-            h2[c] = max2(h2[c], __shfl_xor_sync(0xffffffffu, h2[c], 8), p.is_bf16);
-          }
-          writer = writer && ((g & 1) == 0) && ((r & 1) == 0);
-          oy = y >> 1; ox = x >> 1; Ho = p.H >> 1; Wo = p.W >> 1;
-        }
-        if (p.relu) {  // after the pool: max commutes with ReLU
-#pragma unroll
-          for (int c = 0; c < 32; ++c) h2[c] = max2(h2[c], 0u, p.is_bf16);
-        }
-        if (writer) {
-          const int cgroups = p.cout_slices * 8;
-          uint4* o = reinterpret_cast<uint4*>(p.out);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            if (slice * 64 + j * 8 < p.cout)
-              o[(((size_t)n * cgroups + slice * 8 + j) * Ho + oy) * Wo + ox] = make_uint4(h2[4 * j], h2[4 * j + 1], h2[4 * j + 2], h2[4 * j + 3]);
-          }
-        }
-      } else {
-        if (y < p.H && x < p.W) {
-          float* o = reinterpret_cast<float*>(p.out);
-#pragma unroll
-          for (int c = 0; c < 64; ++c) {
-            const int co = slice * 64 + c;
-            if (co < p.cout) {
-              float a = __uint_as_float(v[c]);
-              if (p.relu) a = fmaxf(a, 0.f);
-              o[(((size_t)n * p.cout + co) * p.H + y) * p.W + x] = a;
-            }
+        for (int c = 0; c < 64; ++c) {
+          const int co = slice * 64 + c;
+          if (co < p.cout) {
+            float a = __uint_as_float(v[c]);  // bias is already in D
+            if (p.relu) a = fmaxf(a, 0.f);
+            p.out[(((size_t)n * p.cout + co) * p.H + y) * p.W + x] = a;
           }
         }
       }
@@ -362,8 +314,6 @@ struct TcState {
   EncodeTiledFn encode = nullptr;
   float* w1 = nullptr;      // block_1 weights [9][64] fp32 (BN folded)
   void* w1img[2] = {nullptr, nullptr};  // block_1 as tcgen05 operand B: [chunk 2][cout 64][8] (K = 9 taps padded to 16)
-  float* bias_pad[SPN_NUM_LAYERS] = {};  // [cout_slices*64]
-  bool smem_attr_set = false;
 };
 
 TcState* tc_state(spn_ctx* ctx) {
@@ -384,27 +334,13 @@ int get_encode(TcState* st) {
   return SPN_OK;
 }
 
-uint16_t to16(float f, int bf16) {
-  if (bf16) {
-    __nv_bfloat16 h = __float2bfloat16_rn(f);
-    return *reinterpret_cast<uint16_t*>(&h);
-  }
-  __half h = __float2half_rn(f);
-  return *reinterpret_cast<uint16_t*>(&h);
-}
-
-// One tensor-core conv layer: in (C8, [n][cin/8][H][W][8]) -> out (C8 pooled-or-not, or NCHW fp32).
-int launch_conv_tc(spn_ctx* ctx, int layer, int mode, const void* in, void* out, int n_img, int H, int W, bool relu, bool pool,
-                   int out_mode, cudaStream_t s) {
-  TcState* st = tc_state(ctx);
+// One 1x1 tensor-core conv layer: in (C8, [n][cin/8][H][W][8]) -> out (NCHW fp32 [n][cout][H][W]).
+int launch_conv1x1_tc(spn_ctx* ctx, int layer, int mode, const void* in, float* out, int n_img, int H, int W, bool relu,
+                      cudaStream_t s) {
   const SpnLayer& L = ctx->layers[layer];
   const int bf = mode == SPN_MODE_BF16 ? 1 : 0;
-  if (L.ks == 3 && out_mode == 0 && ctx->opt_fold)  // 3x3 layers: horizontal taps folded into N (conv_fold.cu)
-    return spn_launch_conv_fold(ctx, layer, mode, in, out, n_img, H, W, relu, pool, s);
-  if (!L.w16[bf] || !st->bias_pad[layer]) { spn_set_error("layer %d has no tensor-core weights", layer); return SPN_E_STATE; }
+  if (!L.w16[bf]) { spn_set_error("layer %d has no tensor-core weights", layer); return SPN_E_STATE; }
   SPN_REQUIRE(L.cin % 64 == 0, "tensor-core conv needs Cin %% 64 == 0 (layer %d has %d)", layer, L.cin);
-  int rc = get_encode(st);
-  if (rc) return rc;
 
   TcParams p;
   memset(&p, 0, sizeof(p));
@@ -412,43 +348,28 @@ int launch_conv_tc(spn_ctx* ctx, int layer, int mode, const void* in, void* out,
   p.cin_blocks = L.cin / 64;
   p.cout_slices = (L.cout + 63) / 64;
   p.cout = L.cout;
-  p.taps = L.ks * L.ks;
-  p.relu = relu; p.pool = pool; p.out_mode = out_mode; p.is_bf16 = bf;
+  p.relu = relu; p.is_bf16 = bf;
   p.tiles_x = spn_cdiv(W, kTW); p.tiles_y = spn_cdiv(H, kTH);
-  const int halo = L.ks == 3 ? 1 : 0;
-  const int PW = kTW + 2 * halo, PH = kTH + 2 * halo;
-  p.slab_bytes = 8 * PH * PW * 16;
-  p.stage_bytes = (p.slab_bytes + 1023) & ~1023;
-  const int wbytes = p.cin_blocks * p.taps * kWBlockBytes + kBiasBlockBytes;
+  const int wbytes = p.cin_blocks * kWBlockBytes + kBiasBlockBytes;
   const int wres = ((wbytes + 1023) & ~1023) + kOnesBytes;
   const int max_dyn = 227 * 1024 - 2048;  // leave room for the static barriers / bias
-  p.stages = (max_dyn - wres - 1024) / p.stage_bytes;
+  p.stages = (max_dyn - wres - 1024) / kSlabBytes;
   if (p.stages > kMaxStages) p.stages = kMaxStages;
   SPN_REQUIRE(p.stages >= 2, "layer %d does not fit in shared memory (weights %d bytes)", layer, wbytes);
   p.out = out; p.wimg = L.w16[bf];
-  const size_t dyn = (size_t)wres + (size_t)p.stages * p.stage_bytes + 1024;
+  const size_t dyn = (size_t)wres + (size_t)p.stages * kSlabBytes + 1024;
 
   CUtensorMap tmap;
-  const cuuint64_t dims[4] = {(cuuint64_t)W * 8, (cuuint64_t)H, (cuuint64_t)(L.cin / 8), (cuuint64_t)n_img};
-  const cuuint64_t strides[3] = {(cuuint64_t)W * 16, (cuuint64_t)H * W * 16, (cuuint64_t)(L.cin / 8) * H * W * 16};
-  const cuuint32_t box[4] = {(cuuint32_t)PW * 8, (cuuint32_t)PH, 8, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult cr = st->encode(&tmap, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(in),
-                           dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) {
-    spn_set_error("cuTensorMapEncodeTiled failed (%d) for layer %d, %dx%dx%d", (int)cr, layer, L.cin, H, W);
-    return SPN_E_CUDA;
-  }
-  auto kern = L.ks == 3 ? conv_tc_kernel<9> : conv_tc_kernel<1>;
-  SPN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+  int rc = spn_c8_tensor_map(ctx, &tmap, in, n_img, L.cin, H, W, kTW, kTH, bf);
+  if (rc) return rc;
+  SPN_CUDA(cudaFuncSetAttribute(conv1x1_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
   const long long work = (long long)n_img * p.tiles_x * p.tiles_y * p.cout_slices;
   int grid = ctx->sm_count;
   if (work < grid) grid = (int)work;
   grid = grid / p.cout_slices * p.cout_slices;
   if (grid < p.cout_slices) grid = p.cout_slices;
   SpnProfScope prof(ctx, layer, s);
-  kern<<<grid, kThreads, dyn, s>>>(tmap, p);
+  conv1x1_tc_kernel<<<grid, kThreads, dyn, s>>>(tmap, p);
   SPN_CHECK_LAUNCH(ctx);
   return SPN_OK;
 }
@@ -492,7 +413,6 @@ const float* spn_tc_block1_weights(spn_ctx* ctx) { return tc_state(ctx)->w1; }
 int spn_tc_pack_layer(spn_ctx* ctx, int layer, const float* h_wfold, const float* h_bfold, cudaStream_t s) {
   TcState* st = tc_state(ctx);
   SpnLayer& L = ctx->layers[layer];
-  const int taps = L.ks * L.ks;
   SPN_CUDA(cudaStreamSynchronize(s));
   if (layer == SPN_L_BLOCK1) {
     SPN_REQUIRE(L.cin == 1 && L.cout == 64 && L.ks == 3, "block_1 must be a 3x3 conv 1->64");
@@ -505,16 +425,11 @@ int spn_tc_pack_layer(spn_ctx* ctx, int layer, const float* h_wfold, const float
       // K = 16: k 0..8 = the nine taps, k 9 / 10 = the bias as a (hi, lo) pair of 16-bit values multiplied by the
       // constant-one columns the front end puts into A1 (so block_1's epilogue needs no bias add)
       std::vector<uint16_t> img(2 * 64 * 8, 0);
-      auto from16 = [&](uint16_t h) {
-        if (bf) { __nv_bfloat16 v = *reinterpret_cast<__nv_bfloat16*>(&h); return __bfloat162float(v); }
-        __half v = *reinterpret_cast<__half*>(&h);
-        return __half2float(v);
-      };
       for (int co = 0; co < 64; ++co) {
         for (int t = 0; t < 9; ++t) img[((size_t)(t / 8) * 64 + co) * 8 + (t % 8)] = to16(h_wfold[(size_t)co * 9 + t], bf);
         const uint16_t hi = to16(h_bfold[co], bf);
         img[((size_t)1 * 64 + co) * 8 + 1] = hi;
-        img[((size_t)1 * 64 + co) * 8 + 2] = to16(h_bfold[co] - from16(hi), bf);
+        img[((size_t)1 * 64 + co) * 8 + 2] = to16(h_bfold[co] - from16(hi, bf), bf);
       }
       if (!st->w1img[bf]) SPN_CUDA(cudaMalloc(&st->w1img[bf], img.size() * 2));
       SPN_CUDA(cudaMemcpy(st->w1img[bf], img.data(), img.size() * 2, cudaMemcpyHostToDevice));
@@ -522,58 +437,61 @@ int spn_tc_pack_layer(spn_ctx* ctx, int layer, const float* h_wfold, const float
     return SPN_OK;
   }
   if (L.cin % 64 != 0) return SPN_OK;  // not a tensor-core layer
-  const int slices = (L.cout + 63) / 64, cbs = L.cin / 64;
-  std::vector<float> bias((size_t)slices * 64, 0.f);
-  for (int co = 0; co < L.cout; ++co) bias[co] = h_bfold[co];
-  if (st->bias_pad[layer]) { cudaFree(st->bias_pad[layer]); st->bias_pad[layer] = nullptr; }
-  SPN_CUDA(cudaMalloc((void**)&st->bias_pad[layer], bias.size() * sizeof(float)));
-  SPN_CUDA(cudaMemcpy(st->bias_pad[layer], bias.data(), bias.size() * sizeof(float), cudaMemcpyHostToDevice));
-  // operand-B image: [slice][cin block][tap][k-step 4][chunk 2][cout 64][8 cin]  (SWIZZLE_NONE K-major core matrices)
-  // followed, per slice, by the bias block [chunk 2][cout 64][8]: k 0 = hi, k 1 = lo 16-bit halves of the folded bias
-  const size_t n16 = (size_t)slices * ((size_t)cbs * taps * 4 * 2 * 64 * 8 + 2 * 64 * 8);
-  for (int bf = 0; bf < 2; ++bf) {
-    std::vector<uint16_t> img(n16, 0);
-    size_t o = 0;
-    auto from16 = [&](uint16_t h) {
-      if (bf) { __nv_bfloat16 v = *reinterpret_cast<__nv_bfloat16*>(&h); return __bfloat162float(v); }
-      __half v = *reinterpret_cast<__half*>(&h);
-      return __half2float(v);
-    };
-    for (int sl = 0; sl < slices; ++sl) {
-      for (int cb = 0; cb < cbs; ++cb)
-        for (int t = 0; t < taps; ++t)
-          for (int kk = 0; kk < 4; ++kk)
-            for (int j = 0; j < 2; ++j)
-              for (int co = 0; co < 64; ++co)
-                for (int e = 0; e < 8; ++e, ++o) {
-                  const int c = sl * 64 + co, ci = cb * 64 + kk * 16 + j * 8 + e;
-                  if (c < L.cout) img[o] = to16(h_wfold[((size_t)c * L.cin + ci) * taps + t], bf);
-                }
-      for (int co = 0; co < 64; ++co) {
-        const int c = sl * 64 + co;
-        if (c < L.cout) {
-          const uint16_t hi = to16(h_bfold[c], bf);
-          img[o + (size_t)co * 8] = hi;
-          img[o + (size_t)co * 8 + 1] = to16(h_bfold[c] - from16(hi), bf);
+  if (L.ks == 1 || layer == SPN_L_BLOCK2) {  // the 1x1 kernel's weights, and block_2's that front_tc_kernel reads
+    const int taps = L.ks * L.ks, slices = (L.cout + 63) / 64, cbs = L.cin / 64;
+    // operand-B image: [slice][cin block][tap][k-step 4][chunk 2][cout 64][8 cin]  (SWIZZLE_NONE K-major core matrices)
+    // followed, per slice, by the bias block [chunk 2][cout 64][8]: k 0 = hi, k 1 = lo 16-bit halves of the folded bias
+    const size_t n16 = (size_t)slices * ((size_t)cbs * taps * 4 * 2 * 64 * 8 + 2 * 64 * 8);
+    for (int bf = 0; bf < 2; ++bf) {
+      std::vector<uint16_t> img(n16, 0);
+      size_t o = 0;
+      for (int sl = 0; sl < slices; ++sl) {
+        for (int cb = 0; cb < cbs; ++cb)
+          for (int t = 0; t < taps; ++t)
+            for (int kk = 0; kk < 4; ++kk)
+              for (int j = 0; j < 2; ++j)
+                for (int co = 0; co < 64; ++co)
+                  for (int e = 0; e < 8; ++e, ++o) {
+                    const int c = sl * 64 + co, ci = cb * 64 + kk * 16 + j * 8 + e;
+                    if (c < L.cout) img[o] = to16(h_wfold[((size_t)c * L.cin + ci) * taps + t], bf);
+                  }
+        for (int co = 0; co < 64; ++co) {
+          const int c = sl * 64 + co;
+          if (c < L.cout) {
+            const uint16_t hi = to16(h_bfold[c], bf);
+            img[o + (size_t)co * 8] = hi;
+            img[o + (size_t)co * 8 + 1] = to16(h_bfold[c] - from16(hi, bf), bf);
+          }
         }
+        o += 2 * 64 * 8;
       }
-      o += 2 * 64 * 8;
+      if (L.w16[bf]) { cudaFree(L.w16[bf]); L.w16[bf] = nullptr; }
+      SPN_CUDA(cudaMalloc(&L.w16[bf], n16 * 2));
+      SPN_CUDA(cudaMemcpy(L.w16[bf], img.data(), n16 * 2, cudaMemcpyHostToDevice));
     }
-    if (L.w16[bf]) { cudaFree(L.w16[bf]); L.w16[bf] = nullptr; }
-    SPN_CUDA(cudaMalloc(&L.w16[bf], n16 * 2));
-    SPN_CUDA(cudaMemcpy(L.w16[bf], img.data(), n16 * 2, cudaMemcpyHostToDevice));
   }
   int rc = spn_fold_pack_layer(ctx, layer, h_wfold, h_bfold);
   if (rc) return rc;
   return spn_head_pack_layer(ctx, layer, h_wfold, h_bfold);
 }
 
-const float* spn_tc_bias(spn_ctx* ctx, int layer) { return tc_state(ctx)->bias_pad[layer]; }
-
-void* spn_tc_encode_fn(spn_ctx* ctx) {
+int spn_c8_tensor_map(spn_ctx* ctx, CUtensorMap* map, const void* base, int n_img, int C, int H, int W, int box_w, int box_h,
+                      int bf16) {
   TcState* st = tc_state(ctx);
-  if (get_encode(st) != SPN_OK) return nullptr;
-  return (void*)st->encode;
+  int rc = get_encode(st);
+  if (rc) return rc;
+  const cuuint64_t dims[4] = {(cuuint64_t)W * 8, (cuuint64_t)H, (cuuint64_t)(C / 8), (cuuint64_t)n_img};
+  const cuuint64_t strides[3] = {(cuuint64_t)W * 16, (cuuint64_t)H * W * 16, (cuuint64_t)(C / 8) * H * W * 16};
+  const cuuint32_t box[4] = {(cuuint32_t)box_w * 8, (cuuint32_t)box_h, 8, 1};
+  const cuuint32_t estr[4] = {1, 1, 1, 1};
+  CUresult cr = st->encode(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(base),
+                           dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (cr != CUDA_SUCCESS) {
+    spn_set_error("cuTensorMapEncodeTiled failed (%d) for a C8 tensor of %d x %d x %d x %d", (int)cr, n_img, C, H, W);
+    return SPN_E_CUDA;
+  }
+  return SPN_OK;
 }
 
 // Encoder over `n_slots` forwards.  d_hinv == nullptr: slot i is image i (plain forward).  Otherwise slot =
@@ -599,19 +517,18 @@ int spn_tc_encoder_slots(spn_ctx* ctx, const float* d_images, const float* d_hin
       conv1_c8_kernel<<<g, 256, 0, s>>>(d_images + (size_t)slot_begin * H * W, st->w1, ctx->layers[0].bias, A, B, H, W, bf);
       SPN_CHECK_LAUNCH(ctx);
     }
-    if ((rc = launch_conv_tc(ctx, 1, mode, A, Bq, B, H, W, true, true, 0, s))) return rc;
+    if ((rc = spn_launch_conv_fold(ctx, 1, mode, A, Bq, B, H, W, true, true, s))) return rc;
   } else {
     // warp + block_1 + block_2 in one kernel (front_tc.cu): block_1's output never reaches HBM
-    rc = ctx->opt_front_pair ? spn_front2_tc_launch(ctx, d_images, d_hinv, n_h, slot_begin, n_slots, H, W, mode, st->w1img[bf], Bq, s)
-                             : spn_front_tc_launch(ctx, d_images, d_hinv, n_h, slot_begin, n_slots, H, W, mode, st->w1img[bf], Bq, s);
+    rc = spn_front_tc_launch(ctx, d_images, d_hinv, n_h, slot_begin, n_slots, H, W, mode, st->w1img[bf], Bq, s);
     if (rc) return rc;
   }
-  if ((rc = launch_conv_tc(ctx, 2, mode, Bq, A, B, H / 2, W / 2, true, false, 0, s))) return rc;
-  if ((rc = launch_conv_tc(ctx, 3, mode, A, Bq, B, H / 2, W / 2, true, true, 0, s))) return rc;
-  if ((rc = launch_conv_tc(ctx, 4, mode, Bq, A, B, H / 4, W / 4, true, false, 0, s))) return rc;
-  if ((rc = launch_conv_tc(ctx, 5, mode, A, Bq, B, H / 4, W / 4, true, true, 0, s))) return rc;
-  if ((rc = launch_conv_tc(ctx, 6, mode, Bq, A, B, H / 8, W / 8, true, false, 0, s))) return rc;
-  if ((rc = launch_conv_tc(ctx, 7, mode, A, F, B, H / 8, W / 8, true, false, 0, s))) return rc;
+  if ((rc = spn_launch_conv_fold(ctx, 2, mode, Bq, A, B, H / 2, W / 2, true, false, s))) return rc;
+  if ((rc = spn_launch_conv_fold(ctx, 3, mode, A, Bq, B, H / 2, W / 2, true, true, s))) return rc;
+  if ((rc = spn_launch_conv_fold(ctx, 4, mode, Bq, A, B, H / 4, W / 4, true, false, s))) return rc;
+  if ((rc = spn_launch_conv_fold(ctx, 5, mode, A, Bq, B, H / 4, W / 4, true, true, s))) return rc;
+  if ((rc = spn_launch_conv_fold(ctx, 6, mode, Bq, A, B, H / 8, W / 8, true, false, s))) return rc;
+  if ((rc = spn_launch_conv_fold(ctx, 7, mode, A, F, B, H / 8, W / 8, true, false, s))) return rc;
   ctx->feat = F;
   return SPN_OK;
 }
@@ -624,8 +541,8 @@ int spn_tc_detector_head(spn_ctx* ctx, int B, int H, int W, int mode, float* d_l
   const TcPlan pl = tc_plan(B, H, W);
   char* head = ctx->ws + pl.off_head;
   int rc;
-  if ((rc = launch_conv_tc(ctx, SPN_L_CONVPA, mode, ctx->feat, head, B, H / 8, W / 8, true, false, 0, s))) return rc;
-  return launch_conv_tc(ctx, SPN_L_CONVPB, mode, head, d_logits, B, H / 8, W / 8, false, false, 1, s);
+  if ((rc = spn_launch_conv_fold(ctx, SPN_L_CONVPA, mode, ctx->feat, head, B, H / 8, W / 8, true, false, s))) return rc;
+  return launch_conv1x1_tc(ctx, SPN_L_CONVPB, mode, head, d_logits, B, H / 8, W / 8, false, s);
 }
 
 // convPa, then convPb + softmax + depth-to-space + mask in one kernel (head_tc.cu)
@@ -634,7 +551,7 @@ int spn_tc_detector_head_fused(spn_ctx* ctx, int B, int H, int W, int mode, cons
   const TcPlan pl = tc_plan(B, H, W);
   char* head = ctx->ws + pl.off_head;
   int rc;
-  if ((rc = launch_conv_tc(ctx, SPN_L_CONVPA, mode, ctx->feat, head, B, H / 8, W / 8, true, false, 0, s))) return rc;
+  if ((rc = spn_launch_conv_fold(ctx, SPN_L_CONVPA, mode, ctx->feat, head, B, H / 8, W / 8, true, false, s))) return rc;
   return spn_launch_head_tc(ctx, mode, head, B, H / 8, W / 8, d_mask, d_logits, d_prob, s);
 }
 
@@ -642,8 +559,8 @@ int spn_tc_descriptor_head(spn_ctx* ctx, int B, int H, int W, int mode, float* d
   const TcPlan pl = tc_plan(B, H, W);
   char* head = ctx->ws + pl.off_head;
   int rc;
-  if ((rc = launch_conv_tc(ctx, SPN_L_CONVDA, mode, ctx->feat, head, B, H / 8, W / 8, true, false, 0, s))) return rc;
-  return launch_conv_tc(ctx, SPN_L_CONVDB, mode, head, d_desc_raw, B, H / 8, W / 8, false, false, 1, s);
+  if ((rc = spn_launch_conv_fold(ctx, SPN_L_CONVDA, mode, ctx->feat, head, B, H / 8, W / 8, true, false, s))) return rc;
+  return launch_conv1x1_tc(ctx, SPN_L_CONVDB, mode, head, d_desc_raw, B, H / 8, W / 8, false, s);
 }
 
 float* spn_tc_logits_scratch(spn_ctx* ctx, int B, int H, int W) {
@@ -666,8 +583,8 @@ int spn_tc_conv_layer(spn_ctx* ctx, int layer, int mode, const float* d_in, int 
   const size_t n_in = (size_t)B * (L.cin / 8) * H * W;
   nchw_to_c8_kernel<<<(unsigned)((n_in + 255) / 256), 256, 0, s>>>(d_in, cin8, B, L.cin, H, W, bf);
   SPN_CHECK_LAUNCH(ctx);
-  if (L.ks == 1) return launch_conv_tc(ctx, layer, mode, cin8, d_out, B, H, W, relu, false, 1, s);
-  if ((rc = launch_conv_tc(ctx, layer, mode, cin8, cout8, B, H, W, relu, pool, 0, s))) return rc;
+  if (L.ks == 1) return launch_conv1x1_tc(ctx, layer, mode, cin8, d_out, B, H, W, relu, s);
+  if ((rc = spn_launch_conv_fold(ctx, layer, mode, cin8, cout8, B, H, W, relu, pool, s))) return rc;
   // C8 buffer has cout_slices*64 channels; only the first cout are meaningful
   SPN_REQUIRE(L.cout % 64 == 0, "spn_conv_layer (tensor-core, 3x3) needs Cout %% 64 == 0");
   const size_t n_out = (size_t)B * (L.cout / 8) * Ho * Wo;
@@ -681,7 +598,6 @@ void spn_tc_destroy(spn_ctx* ctx) {
   if (!st) return;
   if (st->w1) cudaFree(st->w1);
   for (auto& w : st->w1img) if (w) cudaFree(w);
-  for (auto& b : st->bias_pad) if (b) cudaFree(b);
   delete st;
   ctx->tc = nullptr;
 }

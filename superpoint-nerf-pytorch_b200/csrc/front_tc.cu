@@ -9,7 +9,7 @@
 // Per CTA tile (8 x 16 output pixels of block_2 before pooling = M 128), pipelined over tiles by warp role:
 //   P  warps 10-17  bilinear-sample the 12 x 20 warped-image patch, build block_1's im2col operand A1
 //                   (256 rows = the 10 x 18 halo pixels (180 used), K = 9 taps padded to 16, fp16) in SMEM;
-//                   kPGroups groups of warps that take tiles round robin
+//                   four groups of two warps that take tiles round robin
 //   M  warps 0, 1   two issuers, one per tile parity, taking turns (bar_turn).  MMA1: D1 = A1 . W1 (2 x M128 N64 K16)
 //                   into TMEM, issued kAhead = 3 tiles AHEAD of
 //                   MMA2: D2 += slab(tap) . W2(tap) (36 x M128 N64 K16, weights resident in SMEM), rolled tap loop
@@ -20,7 +20,7 @@
 //                   max-pool (two shfl.xor) -> 16-byte C8 stores
 //   warp 0          also the weight loader (cp.async.bulk)
 // All hand-offs are mbarriers with one arrival per warp (generic-proxy SMEM writes are published to the tensor core
-// with fence.proxy.async).  How the role balance was found: DESIGN.md section 3.2, tools/front_probe_cycles.sh.
+// with fence.proxy.async).  How the role balance was found: DESIGN.md section 3.2.
 #include "spn_common.cuh"
 #include "spn_geom.cuh"
 #include "tc_ptx.cuh"
@@ -43,31 +43,13 @@ constexpr int kW1Bytes = 2 * 64 * 16;                 // block_1 weights as oper
 constexpr int kA1Rows = 256;
 constexpr int kA1Bytes = 2 * kA1Rows * 16;            // [chunk 2][row 256][8 halfs]
 constexpr int kStages = 4;
-constexpr int kNA1 = 3;                               // D1 buffers (TMEM): MMA1 runs two tiles ahead of MMA2
-#ifndef SPN_E2_GROUPS
-#define SPN_E2_GROUPS 1
-#endif
-constexpr int kE2Groups = SPN_E2_GROUPS;              // block_2 epilogue groups (2: warps 18-21 take the odd tiles)
-constexpr int kThreads = 576 + (kE2Groups - 1) * 128;  // 18 (22) warps
-#ifndef SPN_TURN_TAP
-#define SPN_TURN_TAP 9
-#endif
-constexpr int kTurnTap = SPN_TURN_TAP;               // the issue turn passes to the other issuer after this tap of block_2 (9 = after the bias MMA)
-#ifndef SPN_POLL_NS
-#define SPN_POLL_NS 0
-#endif
-constexpr uint32_t kPollNs = SPN_POLL_NS;             // back-off between barrier polls of the producer / epilogue roles
-#ifndef SPN_MMA1_AHEAD
-#define SPN_MMA1_AHEAD 3
-#endif
-constexpr int kAhead = SPN_MMA1_AHEAD;               // block_1's MMAs are issued this many tiles ahead of block_2's (2 or 3; 3 D1 buffers)
-#ifndef SPN_P_GROUPS
-#define SPN_P_GROUPS 4
-#endif
-constexpr int kPGroups = SPN_P_GROUPS;                // P role: the 8 warps 10-17 split into groups that take tiles round robin
+constexpr int kNA1 = 3;                               // D1 buffers (TMEM)
+constexpr int kThreads = 576;                         // 18 warps
+constexpr int kAhead = 3;                             // block_1's MMAs are issued this many tiles ahead of block_2's
+constexpr int kPGroups = 4;                           // P role: the 8 warps 10-17 split into groups that take tiles round robin
 constexpr int kPGroup = 256 / kPGroups;               // threads per group
 constexpr int kPSamples = (12 * 20 + kPGroup - 1) / kPGroup, kPRows = (10 * 18 + kPGroup - 1) / kPGroup;   // per thread and tile
-constexpr int kNA1s = kPGroups > 3 ? kPGroups : 3;    // A1 / patch buffers (SMEM)
+constexpr int kNA1s = kPGroups;                       // A1 / patch buffers (SMEM): one per P group
 
 struct FrontParams {
   const float* images;   // [n_src][H][W] fp32
@@ -91,8 +73,6 @@ __device__ __forceinline__ uint16_t to16(float v, int bf) {
   return *reinterpret_cast<uint16_t*>(&h);
 }
 
-// DBG != 0 instantiations switch parts of the roles off (bottleneck experiments, tools/front_probe.py; wrong results).
-template <int DBG>
 __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ __align__(8) uint64_t bar_w, bar_a1_full[kNA1s], bar_a1_empty[kNA1s], bar_d1_full[kNA1], bar_d1_empty[kNA1],
@@ -194,7 +174,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
     // block_2 (as far as the three D1 buffers and the four slab stages allow), so E1 has two tile times to turn D1 into
     // the slab (2117 -> 2069 cycles per tile against two tiles ahead).
     if ((int)(blockIdx.x + par * gridDim.x) < n_tiles) issue_mma1(par);
-    if (kAhead == 3 && par == 0 && (int)(blockIdx.x + 2 * gridDim.x) < n_tiles) issue_mma1(2);
+    if (par == 0 && (int)(blockIdx.x + 2 * gridDim.x) < n_tiles) issue_mma1(2);
     for (int i = par, t = blockIdx.x + par * gridDim.x; t < n_tiles; t += 2 * gridDim.x, i += 2) {
       const int stage = i % kStages, acc = i & 1;
       const uint32_t sph = (uint32_t)(i / kStages) & 1u, aph = (uint32_t)(i >> 1) & 1u;
@@ -203,7 +183,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
       // The two issuers take turns: block_2 of tile i+1 is not issued before the last MMA of tile i is in the queue.
       // Without the turn both warps issue at once whenever their operands are ready, the MMAs of two tiles interleave
       // (alternating accumulators), both accumulators complete together and the pipe then idles while they drain.
-      if (kTurnTap >= 0) mbar_wait(&bar_turn[par], aph);
+      mbar_wait(&bar_turn[par], aph);
       tc_fence_after();
       if (elect_one()) {
         // One ROLLED loop over the nine taps (4 MMAs per iteration, descriptors advanced by loop-carried adds).  Fully
@@ -216,12 +196,11 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
         const uint32_t d2 = tmem_base + (uint32_t)acc * 64;
         int kx = 0;
 #pragma unroll 1
-        for (int tap = 0; tap < ((DBG & 128) ? 1 : 9); ++tap) {
+        for (int tap = 0; tap < 9; ++tap) {
 #pragma unroll
           for (int kk = 0; kk < 4; ++kk)
             umma_f16_2w(d2, a_t + (uint32_t)kk * ((2 * kChStride) >> 4), hi_a2, b_t + (uint32_t)kk * (2048u >> 4), hi_b, idesc,
                         (tap | kk) ? 1u : 0u);
-          if (tap == kTurnTap) mbar_arrive(&bar_turn[par ^ 1]);   // a few MMAs early: covers the other warp's wake-up
           b_t += 8192u >> 4;
           if (++kx == 3) { kx = 0; a_t += kPW - 2; } else { a_t += 1; }   // next tap: +1 pixel, or the next halo row
         }
@@ -230,7 +209,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
         umma_f16_2w(d2, (smem_u32(ones) >> 4) | ((2048u >> 4) << 16), (128u >> 4) | (1u << 14), w2_lo + ((9u * 8192u) >> 4), hi_b,
                     idesc, 1u);
         umma_commit(&bar_d2_full[acc]);
-        if (kTurnTap >= 9 || (kTurnTap >= 0 && (DBG & 128))) mbar_arrive(&bar_turn[par ^ 1]);
+        mbar_arrive(&bar_turn[par ^ 1]);   // the bias MMA is in the queue: the other issuer's turn
       }
       __syncwarp();
       if (t + kAhead * (int)gridDim.x < n_tiles) issue_mma1(i + kAhead);   // kAhead == 3: the other issuer's next tile
@@ -240,7 +219,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
     // kPGroups groups of warps take tiles round robin.  A tile's P work is one long dependent chain (coordinates ->
     // four L2 loads -> interpolation -> patch -> barrier -> im2col rows -> fence), ~2300 cycles when all eight warps
     // work on the same tile in lock step, which made P the pace of the kernel (ncu source page: P never waited for a
-    // free A1 buffer while the MMA issuers waited for operands; role knock-outs in SM cycles, tools/front_probe_cycles.sh:
+    // free A1 buffer while the MMA issuers waited for operands; role knock-outs in SM cycles, DESIGN.md section 3.2:
     // 2230 cycles per tile with P, 1971 without, 1969 for the MMA stream alone).  With g groups each has g tile times
     // per tile and the samples of a thread overlap their loads.
     const int grp = (warp - 10) / (8 / kPGroups);
@@ -273,7 +252,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
         const int py = s / kQW, px = s - py * kQW;
         const int y = ty * kTH - 2 + py, x = tx * kTW - 2 + px;
         float v = 0.f;
-        if (s < kQH * kQW && y >= 0 && y < p.H && x >= 0 && x < p.W && !(DBG & 1)) {
+        if (s < kQH * kQW && y >= 0 && y < p.H && x >= 0 && x < p.W) {
           if (j == 0) {
             v = __ldg(&img[(size_t)y * p.W + x]);
           } else {
@@ -284,7 +263,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
         }
         pv[k] = v;
       }
-      mbar_wait_backoff(&bar_a1_empty[b], ph ^ 1u, kPollNs * 2);
+      mbar_wait(&bar_a1_empty[b], ph ^ 1u);
 #pragma unroll
       for (int k = 0; k < kPSamples; ++k)
         if (pt + k * kPGroup < kQH * kQW) patch_s[b][pt + k * kPGroup] = to16(pv[k], p.is_bf16);
@@ -301,7 +280,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
 #pragma unroll
       for (int k = 0; k < kPRows; ++k) {
         const int r = pt + k * kPGroup;
-        if (r >= ((DBG & 2) ? 0 : kHalo)) break;
+        if (r >= kHalo) break;
         const int hy = r / kPW, hx = r - hy * kPW;
         const int gy = ty * kTH - 1 + hy, gx = tx * kTW - 1 + hx;
         uint4 c0 = make_uint4(0u, 0u, 0u, 0u), c1 = make_uint4(0u, 0u, 0u, 0u);
@@ -329,7 +308,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
     for (int t = blockIdx.x; t < n_tiles; t += gridDim.x, ++i) {
       const int b = i % kNA1, stage = i % kStages;
       const uint32_t ph = (uint32_t)(i / kNA1) & 1u, sph = (uint32_t)(i / kStages) & 1u;
-      mbar_wait_backoff(&bar_d1_full[b], ph, kPollNs);
+      mbar_wait(&bar_d1_full[b], ph);
       mbar_wait(&bar_slab_empty[stage], sph ^ 1u);
       tc_fence_after();
       uint8_t* slab = slab0 + (size_t)stage * kStageBytes;
@@ -339,12 +318,10 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
         const int r = h * 128 + q * 32 + lane;
         uint32_t v[64];
         const uint32_t taddr = tmem_base + 128 + (uint32_t)(b * 2 + h) * 64 + ((uint32_t)(q * 32) << 16);
-        if (!(DBG & 8)) {
-          tmem_ld32(taddr, v);
-          tmem_ld32(taddr + 32, v + 32);
-          tmem_ld_wait();
-        }
-        if (r < kHalo && !(DBG & 4)) {  // bias is already inside D1 (ones columns of A1): ReLU + 16-bit pack + 8 x 16-byte stores
+        tmem_ld32(taddr, v);
+        tmem_ld32(taddr + 32, v + 32);
+        tmem_ld_wait();
+        if (r < kHalo) {  // bias is already inside D1 (ones columns of A1): ReLU + 16-bit pack + 8 x 16-byte stores
 #pragma unroll
           for (int c8 = 0; c8 < 8; ++c8) {
             uint32_t w[4];
@@ -370,26 +347,22 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
     const int q = warp & 3;
     const int g = q * 4 + (lane >> 3), r = lane & 7;
     const int Ho = p.H >> 1, Wo = p.W >> 1;
-    const int e2g = warp >= 18 ? 1 : 0;   // with two groups each owns one accumulator / tile parity
-    for (int i = e2g, t = blockIdx.x + e2g * gridDim.x; t < n_tiles; t += kE2Groups * gridDim.x, i += kE2Groups) {
+    for (int i = 0, t = blockIdx.x; t < n_tiles; t += gridDim.x, ++i) {
       const int acc = i & 1;
       const uint32_t aph = (uint32_t)(i >> 1) & 1u;
       const int ls = fast_div(t, p.magic_tpi), rr = t - ls * tiles_per_img;
       const int ty = fast_div(rr, p.magic_tx), tx = rr - ty * p.tiles_x;
       const int y = ty * kTH + g, x = tx * kTW + r;
-      mbar_wait_backoff(&bar_d2_full[acc], aph, kPollNs);
+      mbar_wait(&bar_d2_full[acc], aph);
       tc_fence_after();
       uint32_t v[64];
       const uint32_t taddr = tmem_base + (uint32_t)acc * 64 + ((uint32_t)(q * 32) << 16);
-      if (!(DBG & 64)) {
-        tmem_ld32(taddr, v);
-        tmem_ld32(taddr + 32, v + 32);
-        tmem_ld_wait();
-      }
+      tmem_ld32(taddr, v);
+      tmem_ld32(taddr + 32, v + 32);
+      tmem_ld_wait();
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&bar_d2_empty[acc]);
-      if (DBG & 32) continue;
       uint32_t h2[32];
 #pragma unroll
       for (int c = 0; c < 32; ++c) h2[c] = pack2_relu(__uint_as_float(v[2 * c]), __uint_as_float(v[2 * c + 1]), p.is_bf16);
@@ -398,7 +371,7 @@ __global__ void __launch_bounds__(kThreads, 1) front_tc_kernel(const FrontParams
         h2[c] = max2(h2[c], __shfl_xor_sync(0xffffffffu, h2[c], 1), p.is_bf16);
         h2[c] = max2(h2[c], __shfl_xor_sync(0xffffffffu, h2[c], 8), p.is_bf16);
       }
-      if (y < p.H && x < p.W && (g & 1) == 0 && (r & 1) == 0 && !(DBG & 16)) {
+      if (y < p.H && x < p.W && (g & 1) == 0 && (r & 1) == 0) {
         uint4* o = reinterpret_cast<uint4*>(p.out);
         const int oy = y >> 1, ox = x >> 1;
 #pragma unroll
@@ -436,28 +409,9 @@ int spn_front_tc_launch(spn_ctx* ctx, const float* d_images, const float* d_hinv
   const size_t dyn = (size_t)kW2Bytes + kW1Bytes + kNA1s * kA1Bytes + kOnesBytes + (size_t)kStages * kStageBytes + 1024;
   const long long tiles = (long long)n_slots * p.tiles_x * p.tiles_y;
   const int grid = (int)(tiles < ctx->sm_count ? tiles : ctx->sm_count);
-  void (*kern)(const FrontParams) = front_tc_kernel<0>;
-#ifdef SPN_FRONT_DBG_BUILD  // diagnostic build only (tools/front_probe.py): role knock-out instantiations, wrong results
-  switch (ctx->opt_front_variant) {
-    case 0: break;
-    case 1: kern = front_tc_kernel<1>; break;
-    case 2: kern = front_tc_kernel<2>; break;
-    case 3: kern = front_tc_kernel<3>; break;
-    case 12: kern = front_tc_kernel<12>; break;
-    case 16: kern = front_tc_kernel<16>; break;
-    case 32: kern = front_tc_kernel<32>; break;
-    case 96: kern = front_tc_kernel<96>; break;
-    case 128: kern = front_tc_kernel<128>; break;
-    case 15: kern = front_tc_kernel<15>; break;
-    case 108: kern = front_tc_kernel<108>; break;
-    case 99: kern = front_tc_kernel<99>; break;
-    case 111: kern = front_tc_kernel<111>; break;
-    default: spn_set_error("front_variant %d is not compiled in", ctx->opt_front_variant); return SPN_E_INVALID;
-  }
-#endif
-  SPN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+  SPN_CUDA(cudaFuncSetAttribute(front_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
   SpnProfScope prof(ctx, SPN_L_BLOCK2, s);
-  SPN_CUDA(spn_launch_pdl(ctx->opt_pdl != 0, kern, dim3(grid), dim3(kThreads), dyn, s, p));
+  SPN_CUDA(spn_launch_pdl(front_tc_kernel, dim3(grid), dim3(kThreads), dyn, s, p));
   SPN_CHECK_LAUNCH(ctx);
   return SPN_OK;
 }

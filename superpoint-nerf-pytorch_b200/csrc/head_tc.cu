@@ -211,23 +211,6 @@ head_tc_kernel(const __grid_constant__ CUtensorMap tmap, const HeadParams p) {
   }
 }
 
-uint16_t to16h(float f, int bf16) {
-  if (bf16) {
-    __nv_bfloat16 h = __float2bfloat16_rn(f);
-    return *reinterpret_cast<uint16_t*>(&h);
-  }
-  __half h = __float2half_rn(f);
-  return *reinterpret_cast<uint16_t*>(&h);
-}
-float from16h(uint16_t h, int bf16) {
-  if (bf16) return __bfloat162float(*reinterpret_cast<__nv_bfloat16*>(&h));
-  return __half2float(*reinterpret_cast<__half*>(&h));
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 }  // namespace
 
 // operand-B image of convPb for head_tc_kernel (1x1, 256 -> 65): [cb 4][kk 4][chunk 2][n 80][8] + bias block
@@ -242,13 +225,13 @@ int spn_head_pack_layer(spn_ctx* ctx, int layer, const float* h_wfold, const flo
           for (int co = 0; co < 65; ++co)
             for (int e = 0; e < 8; ++e) {
               const int ci = cb * 64 + kk * 16 + j * 8 + e;
-              img[(size_t)(cb * 4 + kk) * (kBlk / 2) + ((size_t)j * kN + co) * 8 + e] = to16h(h_wfold[(size_t)co * 256 + ci], bf);
+              img[(size_t)(cb * 4 + kk) * (kBlk / 2) + ((size_t)j * kN + co) * 8 + e] = to16(h_wfold[(size_t)co * 256 + ci], bf);
             }
     uint16_t* bb = img.data() + (size_t)16 * (kBlk / 2);
     for (int co = 0; co < 65; ++co) {
-      const uint16_t hi = to16h(h_bfold[co], bf);
+      const uint16_t hi = to16(h_bfold[co], bf);
       bb[(size_t)co * 8] = hi;
-      bb[(size_t)co * 8 + 1] = to16h(h_bfold[co] - from16h(hi, bf), bf);
+      bb[(size_t)co * 8 + 1] = to16(h_bfold[co] - from16(hi, bf), bf);
     }
     if (L.w16f[bf]) { cudaFree(L.w16f[bf]); L.w16f[bf] = nullptr; }
     SPN_CUDA(cudaMalloc(&L.w16f[bf], img.size() * 2));
@@ -263,27 +246,19 @@ int spn_launch_head_tc(spn_ctx* ctx, int mode, const void* in, int n_img, int Hc
   const SpnLayer& L = ctx->layers[SPN_L_CONVPB];
   const int bf = mode == SPN_MODE_BF16 ? 1 : 0;
   if (!L.w16f[bf]) { spn_set_error("convPb has no fused-head weights"); return SPN_E_STATE; }
-  EncodeTiledFn encode = (EncodeTiledFn)spn_tc_encode_fn(ctx);
-  if (!encode) return SPN_E_CUDA;
   HeadParams p;
   memset(&p, 0, sizeof(p));
   p.n_img = n_img; p.Hc = Hc; p.Wc = Wc; p.tiles_x = spn_cdiv(Wc, kTW); p.tiles_y = spn_cdiv(Hc, kTH); p.is_bf16 = bf;
   p.wimg = L.w16f[bf]; p.mask = d_mask; p.logits = d_logits; p.prob = d_prob;
   const size_t dyn = (size_t)((kWBytes + 1023) & ~1023) + kOnesBytes + (size_t)kStages * kSlabBytes + 1024;
   CUtensorMap tmap;
-  const cuuint64_t dims[4] = {(cuuint64_t)Wc * 8, (cuuint64_t)Hc, 32, (cuuint64_t)n_img};
-  const cuuint64_t strides[3] = {(cuuint64_t)Wc * 16, (cuuint64_t)Hc * Wc * 16, (cuuint64_t)32 * Hc * Wc * 16};
-  const cuuint32_t box[4] = {(cuuint32_t)kTW * 8, (cuuint32_t)kTH, 8, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult cr = encode(&tmap, bf ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(in), dims,
-                       strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) { spn_set_error("cuTensorMapEncodeTiled failed (%d) for the fused head", (int)cr); return SPN_E_CUDA; }
+  int rc = spn_c8_tensor_map(ctx, &tmap, in, n_img, 256, Hc, Wc, kTW, kTH, bf);
+  if (rc) return rc;
   SPN_CUDA(cudaFuncSetAttribute(head_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
   const long long tiles = (long long)n_img * p.tiles_x * p.tiles_y;
   const int grid = (int)(tiles < ctx->sm_count ? tiles : ctx->sm_count);
   SpnProfScope prof(ctx, SPN_L_CONVPB, s);
-  SPN_CUDA(spn_launch_pdl(ctx->opt_pdl != 0, head_tc_kernel, dim3(grid), dim3(kThreads), dyn, s, tmap, p));
+  SPN_CUDA(spn_launch_pdl(head_tc_kernel, dim3(grid), dim3(kThreads), dyn, s, tmap, p));
   SPN_CHECK_LAUNCH(ctx);
   return SPN_OK;
 }

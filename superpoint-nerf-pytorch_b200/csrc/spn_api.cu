@@ -90,13 +90,11 @@ extern "C" int spn_destroy(spn_ctx* ctx) {
 
 extern "C" int spn_set_option(spn_ctx* ctx, const char* name, int value) {
   SPN_REQUIRE(ctx && name, "spn_set_option: null pointer");
-  struct { const char* n; int* v; } opts[] = {{"fold", &ctx->opt_fold}, {"fold_hybrid", &ctx->opt_fold_hybrid}, {"fuse_front", &ctx->opt_fuse_front},
-                                               {"fuse_head", &ctx->opt_fuse_head}, {"pdl", &ctx->opt_pdl},
-                                               {"front_variant", &ctx->opt_front_variant}, {"front_pair", &ctx->opt_front_pair},
+  struct { const char* n; int* v; } opts[] = {{"fuse_front", &ctx->opt_fuse_front}, {"fuse_head", &ctx->opt_fuse_head},
                                                {"ws_guard", &ctx->opt_ws_guard}};
   for (auto& o : opts)
     if (!strcmp(o.n, name)) { *o.v = value; return SPN_OK; }
-  spn_set_error("spn_set_option: unknown option '%s' (fold, fold_hybrid, fuse_front, fuse_head, pdl, front_pair, ws_guard)", name);
+  spn_set_error("spn_set_option: unknown option '%s' (fuse_front, fuse_head, ws_guard)", name);
   return SPN_E_INVALID;
 }
 

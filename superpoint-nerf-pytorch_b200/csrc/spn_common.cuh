@@ -1,5 +1,6 @@
 // Shared declarations for the sm_100a kernels behind include/spn_b200.h.
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
@@ -15,7 +16,7 @@ struct SpnLayer {
   int cin = 0, cout = 0, ks = 0, cout_pad = 0;
   float* w32 = nullptr;    // [cin][ks*ks][cout_pad] fp32, BN folded
   float* bias = nullptr;   // [cout_pad] fp32, BN folded
-  void* w16[2] = {nullptr, nullptr};  // tcgen05 operand-B images (fp16, bf16), see conv_tc.cu
+  void* w16[2] = {nullptr, nullptr};  // tcgen05 operand-B images (fp16, bf16) of the 1x1 layers and block_2, see conv_tc.cu
   void* w16f[2] = {nullptr, nullptr}; // same for the kx-folded 3x3 kernel (N = 192), see conv_fold.cu
   void* w16x = nullptr;               // (hi, lo) fp16 operand-B images of the split strict mode, see conv_split.cu
 };
@@ -59,14 +60,9 @@ struct spn_ctx {
   void* feat = nullptr;     // points into ws
   int64_t launches = 0;
   void* tc = nullptr;       // tcgen05 path state (conv_tc.cu)
-  // options (spn_set_option): A/B switches of the tensor-core path, all on by default
-  int opt_fold = 1;         // 3x3 layers: horizontal taps folded into N (conv_fold.cu) instead of nine descriptors
-  int opt_fold_hybrid = 0;  // A/B: 64-channel-input folded layers with kx = 2 as a separate shifted N = 64 MMA (conv_fold.cu, HYB; measured 15 % slower)
+  // options (spn_set_option)
   int opt_fuse_front = 1;   // warp + block_1 + block_2 in one kernel (front_tc.cu)
   int opt_fuse_head = 1;    // convPb + softmax + depth-to-space in one kernel (head_tc.cu)
-  int opt_pdl = 1;          // programmatic dependent launch along the tensor-core chain
-  int opt_front_variant = 0;  // diagnostic build only (tools/front_probe.py)
-  int opt_front_pair = 0;   // fused front end as a 2-CTA cluster with cta_group::2 MMAs (front2_tc.cu)
   int opt_ws_guard = 0;     // paint the gaps between the carved workspace regions before every encoder pass (spn_check_guards)
   std::vector<std::pair<char*, size_t>> guard_gaps;   // the gaps painted by the last pass
 };
@@ -121,10 +117,9 @@ struct SpnProfScope {
 
 // Launch with programmatic stream serialization: the kernel may begin (prologue: barriers, TMEM, weights) while the
 // previous kernel of the stream drains; it must execute griddepcontrol.wait before touching anything that kernel
-// wrote or read.  pdl == false (spn_set_option "pdl" 0) falls back to a plain launch.
+// wrote or read.
 template <typename... KArgs, typename... Args>
-inline cudaError_t spn_launch_pdl(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t dyn, cudaStream_t s, Args&&... args) {
-  const bool off = !pdl;
+inline cudaError_t spn_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t dyn, cudaStream_t s, Args&&... args) {
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = grid;
@@ -135,7 +130,7 @@ inline cudaError_t spn_launch_pdl(bool pdl, void (*kernel)(KArgs...), dim3 grid,
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = off ? 0 : 1;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
@@ -147,6 +142,20 @@ constexpr size_t kSpnGuard = 64 * 1024, kSpnGap = 4096;
 constexpr int kSpnGuardByte = 0xA5;
 int spn_ensure_ws(spn_ctx* ctx, size_t bytes, cudaStream_t s);
 int spn_ensure_aux(spn_ctx* ctx, size_t bytes, cudaStream_t s);
+
+// Host-side 16-bit conversions for packing operand images (bf16 != 0: bfloat16, else fp16), round to nearest even.
+inline uint16_t to16(float f, int bf16) {
+  if (bf16) {
+    __nv_bfloat16 h = __float2bfloat16_rn(f);
+    return *reinterpret_cast<uint16_t*>(&h);
+  }
+  __half h = __float2half_rn(f);
+  return *reinterpret_cast<uint16_t*>(&h);
+}
+inline float from16(uint16_t h, int bf16) {
+  if (bf16) return __bfloat162float(*reinterpret_cast<__nv_bfloat16*>(&h));
+  return __half2float(*reinterpret_cast<__half*>(&h));
+}
 
 // ---- kernels implemented in the other translation units ----
 int spn_conv_fp32(spn_ctx* ctx, int layer, const float* in, float* out, int B, int H, int W, bool relu, bool pool,
@@ -160,13 +169,15 @@ int spn_tc_encoder(spn_ctx* ctx, const float* d_images, int B, int H, int W, int
 int spn_tc_detector_head(spn_ctx* ctx, int B, int H, int W, int mode, float* d_logits, cudaStream_t s);
 int spn_tc_descriptor_head(spn_ctx* ctx, int B, int H, int W, int mode, float* d_desc_raw, cudaStream_t s);
 void spn_tc_destroy(spn_ctx* ctx);
-const float* spn_tc_bias(spn_ctx* ctx, int layer);
 int spn_head_pack_layer(spn_ctx* ctx, int layer, const float* h_wfold, const float* h_bfold);
 int spn_launch_head_tc(spn_ctx* ctx, int mode, const void* in, int n_img, int Hc, int Wc, const uint8_t* d_mask, float* d_logits,
                        float* d_prob, cudaStream_t s);
 int spn_tc_detector_head_fused(spn_ctx* ctx, int B, int H, int W, int mode, const uint8_t* d_mask, float* d_logits, float* d_prob,
                                cudaStream_t s);
-void* spn_tc_encode_fn(spn_ctx* ctx);  // cuTensorMapEncodeTiled, or nullptr (error set)
+// TMA map of a C8 activation tensor [n_img][C/8][H][W][8] (fp16, or bf16 if bf16 != 0) whose box is box_w pixels x
+// box_h rows x 64 channels of one image; reads outside the tensor are zero-filled (the convolutions' padding).
+int spn_c8_tensor_map(spn_ctx* ctx, CUtensorMap* map, const void* base, int n_img, int C, int H, int W, int box_w, int box_h,
+                      int bf16);
 int spn_fold_pack_layer(spn_ctx* ctx, int layer, const float* h_wfold, const float* h_bfold);
 int spn_launch_conv_fold(spn_ctx* ctx, int layer, int mode, const void* in, void* out, int n_img, int H, int W, bool relu,
                          bool pool, cudaStream_t s);
@@ -174,8 +185,6 @@ int spn_tc_encoder_slots(spn_ctx* ctx, const float* d_images, const float* d_hin
                          int H, int W, int mode, cudaStream_t s);
 int spn_front_tc_launch(spn_ctx* ctx, const float* d_images, const float* d_hinv, int n_h, int slot_begin, int n_slots, int H,
                         int W, int mode, const void* w1img, void* d_out, cudaStream_t s);
-int spn_front2_tc_launch(spn_ctx* ctx, const float* d_images, const float* d_hinv, int n_h, int slot_begin, int n_slots, int H,
-                         int W, int mode, const void* w1img, void* d_out, cudaStream_t s);
 // split strict mode on the tensor cores (conv_split.cu)
 int spn_split_pack_layer(spn_ctx* ctx, int layer, const float* w, const float* b);
 int spn_split_encoder(spn_ctx* ctx, const float* d_images, int B, int H, int W, cudaStream_t s);

@@ -33,25 +33,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
         : "memory");
   }
 }
-// Same wait for roles with slack: sleeps between polls so that a waiting warp does not spend shared-memory wavefronts
-// (each failed try_wait is one) that the tensor core's operand fetch needs.
-__device__ __forceinline__ void mbar_wait_backoff(uint64_t* bar, uint32_t parity, uint32_t ns) {
-  const uint32_t addr = smem_u32(bar);
-  for (;;) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}"
-        : "=r"(ok)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (ok) break;
-    if (ns) __nanosleep(ns);
-  }
-}
 __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3) {
   asm volatile(
       "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"

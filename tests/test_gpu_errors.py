@@ -24,8 +24,9 @@ def test_cabi_argument_and_state_errors():
         ctx.encoder_forward(x, MODE_FP32)
     with pytest.raises(P.NativeError, match="no feature map"):
         ctx.detector_head_forward(1, 16, 24, MODE_FP32)
-    with pytest.raises(P.NativeError, match="unknown option"):
-        ctx.set_option("no_such_switch", 1)
+    for name in ("no_such_switch", "fold", "fold_hybrid", "front_pair", "front_variant", "pdl"):
+        with pytest.raises(P.NativeError, match="unknown option"):
+            ctx.set_option(name, 1)
     with pytest.raises(P.NativeError, match="CUDA tensor"):
         ctx.encoder_forward(x.cpu(), MODE_FP32)
     with pytest.raises(P.NativeError, match="float32"):

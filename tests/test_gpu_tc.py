@@ -34,7 +34,8 @@ def sp_model():
     ("backbone.block_8", (3, 128, 30, 40), 1), ("detector_head.convPa", (2, 128, 30, 40), 1),
     ("detector_head.convPb", (2, 256, 30, 40), 1), ("descriptor_head.convDb", (1, 256, 15, 20), 1),
     ("backbone.block_2", (1, 64, 240, 320), 1), ("backbone.block_4", (1, 64, 16, 8), 2),
-    ("backbone.block_7", (1, 128, 5, 6), 1)])
+    ("backbone.block_7", (1, 128, 5, 6), 1), ("backbone.block_3", (2, 64, 48, 40), 1),
+    ("backbone.block_4", (1, 64, 40, 72), 1), ("backbone.block_5", (1, 64, 30, 44), 1)])
 def test_tc_conv_layer_vs_fp32(sp_model, name, shape, mode):
     m, sd = sp_model
     ctx = m.native()
@@ -133,7 +134,7 @@ def test_ha_fast_mode_headline_workload_vs_oracle(weights):
 
 def test_fused_front_end_matches_unfused(monkeypatch):
     """warp + block_1 + block_2 fused in one tcgen05 kernel (front_tc.cu) vs the unfused kernels (warp_batch ->
-    conv1_c8 -> conv_tc): same heatmaps within fp16 rounding, for plain forwards and for warped HA slots, including
+    conv1_c8 -> conv_fold): same heatmaps within fp16 rounding, for plain forwards and for warped HA slots, including
     image sizes that are not multiples of the 8x16 tile."""
     from superpoint_nerf_pytorch_b200.utils.get_model import get_model
     sd = O.make_state_dict("magicpoint", seed=7, logit_gain=8.0)
@@ -183,7 +184,7 @@ def test_forward_fast_other_sizes_vs_oracle(shape):
 
 
 def test_fused_head_matches_unfused(monkeypatch):
-    """convPb + softmax + depth-to-space + mask in one kernel (head_tc.cu) vs conv_tc<1> + softmax_d2s_kernel:
+    """convPb + softmax + depth-to-space + mask in one kernel (head_tc.cu) vs conv1x1_tc_kernel + softmax_d2s_kernel:
     same 16-bit operands and fp32 accumulation, so logits and heatmaps agree to fp32 rounding."""
     from superpoint_nerf_pytorch_b200.utils.get_model import get_model
     sd = O.make_state_dict("magicpoint", seed=7, logit_gain=8.0)
@@ -205,48 +206,6 @@ def test_fused_head_matches_unfused(monkeypatch):
             outs[tag] = (prob.clone(), logits.clone(), prob2.clone())
         for a, b in zip(outs["fused"], outs["unfused"]):
             assert rel_err(a.cpu().numpy(), b.cpu().numpy()) < 2e-5   # fast exp in the fused kernel: ~1e-6 relative
-
-
-@pytest.mark.parametrize("name,shape", [("backbone.block_3", (2, 64, 48, 40)), ("backbone.block_6", (1, 128, 60, 80))])
-def test_unfolded_conv_kernel_still_correct(sp_model, monkeypatch, name, shape):
-    """conv_tc_kernel<9> (nine shifted descriptors, N = 64) is the formulation used inside front_tc_kernel and the
-    SPN_TC_FOLD=0 fallback for the other 3x3 layers: keep it covered."""
-    m, sd = sp_model
-    ctx = m.native()
-    lid = LAYER_ID[name]
-    _n, cin, cout, k, relu, pool = O.layer_table(superpoint=True)[lid]
-    rng = np.random.RandomState(lid + 100)
-    x = torch.from_numpy(np.maximum(rng.randn(*shape), 0).astype(np.float32))
-    want = O.vgg_block(sd, name, x.half().float(), k, relu, pool).numpy()
-    ctx.set_option("fold", 0)
-    a = ctx.conv_layer(lid, x.cuda(), 1, relu=relu, pool=pool, cout=cout).cpu().numpy()
-    ctx.set_option("fold", 1)
-    b = ctx.conv_layer(lid, x.cuda(), 1, relu=relu, pool=pool, cout=cout).cpu().numpy()
-    assert rel_err(a, want) < FAST and rel_err(b, want) < FAST
-    assert rel_err(a, b) < 2e-3      # same operands, different summation order + one fp16 rounding
-
-
-@pytest.mark.parametrize("name,shape", [("backbone.block_3", (2, 64, 48, 40)), ("backbone.block_4", (1, 64, 40, 72)),
-                                        ("backbone.block_5", (1, 64, 30, 44))])
-def test_hybrid_fold_option(sp_model, name, shape):
-    """Option fold_hybrid (conv_fold_kernel<true>: kx = 0, 1 folded into one N = 128 MMA, kx = 2 as a shifted N = 64 MMA
-    accumulating into the same columns) is an A/B variant for the 64-channel-input layers (measured slower, off by
-    default): it must stay correct."""
-    m, sd = sp_model
-    ctx = m.native()
-    lid = LAYER_ID[name]
-    _n, cin, cout, k, relu, pool = O.layer_table(superpoint=True)[lid]
-    rng = np.random.RandomState(lid + 300)
-    x = torch.from_numpy(np.maximum(rng.randn(*shape), 0).astype(np.float32))
-    want = O.vgg_block(sd, name, x.half().float(), k, relu, pool).numpy()
-    b = ctx.conv_layer(lid, x.cuda(), 1, relu=relu, pool=pool, cout=cout).cpu().numpy()
-    ctx.set_option("fold_hybrid", 1)
-    try:
-        a = ctx.conv_layer(lid, x.cuda(), 1, relu=relu, pool=pool, cout=cout).cpu().numpy()
-    finally:
-        ctx.set_option("fold_hybrid", 0)
-    assert rel_err(a, want) < FAST and rel_err(b, want) < FAST
-    assert rel_err(a, b) < 2e-3      # same operands, the kx = 2 term is summed inside the accumulator instead of after it
 
 
 def test_workspace_guard_bands_stay_intact():
