@@ -1,4 +1,4 @@
-"""ctypes binding of include/spn_b200.h.  PyTorch is used only for device memory and streams."""
+"""ctypes binding of include/spn_b200.h and include/spn_jpeg.h.  PyTorch is used only for device memory and streams."""
 from __future__ import annotations
 
 import ctypes as C
@@ -69,6 +69,14 @@ PROTOTYPES = {
     "spn_profile_read": (_i, [_vp, _vp, _vp]),
 }
 
+# name -> (restype, argtypes); must list every symbol include/spn_jpeg.h declares
+JPEG_PROTOTYPES = {
+    "spn_jpeg_plan": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
+    "spn_jpeg_decode_gray": (_i, [_vp, _vp, _vp, _i, _vp, C.c_int64, _vp, _vp, _vp]),
+}
+JPEG_OK, JPEG_UNSUPPORTED, JPEG_MALFORMED = 0, 1, 2
+JPEG_INFO_FIELDS = 5
+
 _lib = None
 _lock = threading.Lock()
 
@@ -94,7 +102,7 @@ def load_library():
                     raise NativeError(f"{_LIB_PATH} not found and building it failed ({e}); build it with "
                                       "`python superpoint-nerf-pytorch_b200/build.py` (there is no CPU/PyTorch fallback)")
             lib = C.CDLL(str(_LIB_PATH))
-            for name, (res, args) in PROTOTYPES.items():
+            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES).items():
                 fn = getattr(lib, name)
                 fn.restype, fn.argtypes = res, args
             _lib = lib
@@ -124,6 +132,29 @@ def _chk_dev(t: torch.Tensor, dtype, name, device=None):
 def _dense(t):
     """Row-major dense view of a tensor (copies only if needed) - the C ABI takes dense arrays."""
     return None if t is None else t.contiguous()
+
+
+def jpeg_plan(data, offsets):
+    """spn_jpeg_plan (host only, no GPU needed): data = the files back to back (contiguous uint8 numpy), offsets (n+1,)
+    int64 -> (plan blob uint8 numpy, info (n, 5) int64 numpy {status, height, width, luma blocks, output offset},
+    coef_bytes, out_bytes)."""
+    import numpy as np
+    lib = load_library()
+    data = np.ascontiguousarray(data, dtype=np.uint8)
+    offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+    n = len(offsets) - 1
+    info = np.zeros((n, JPEG_INFO_FIELDS), np.int64)
+    totals = np.zeros(2, np.int64)
+    size = C.c_int64(0)
+    args = (C.c_void_p(data.ctypes.data) if data.size else None, C.c_void_p(offsets.ctypes.data), n)
+    tail = (C.c_void_p(info.ctypes.data), C.c_void_p(totals.ctypes.data))
+    for plan in (None, True):
+        if plan is not None:
+            plan = np.empty(size.value, np.uint8)
+        rc = lib.spn_jpeg_plan(*args, None if plan is None else C.c_void_p(plan.ctypes.data), C.byref(size), *tail)
+        if rc != 0:
+            raise NativeError(f"spn_jpeg_plan failed ({rc}): {lib.spn_last_error().decode(errors='replace')}")
+    return plan, info, int(totals[0]), int(totals[1])
 
 
 class Context:
@@ -460,6 +491,18 @@ class Context:
         self._call("spn_resize_crop", self.handle, _ptr(src), int(src.dtype == torch.uint8), src.shape[0], src.shape[1], int(new_h),
                    int(new_w), int(crop_top), int(crop_left), int(H), int(W), C.c_float(divisor), _ptr(out), self._s())
         return out
+
+    def jpeg_decode_gray(self, plan, data, n, coef, out, status):
+        """Enqueue spn_jpeg_decode_gray on the current stream: plan (uint8), data (uint8 file bytes), coef (int16 scratch of
+        at least the plan's coef_bytes), out (uint8 planes of at least out_bytes), status (int32, n) - all CUDA tensors
+        of this context's device.  Images whose status ends up non-zero must be decoded on the host."""
+        for t, dt, name in ((plan, torch.uint8, "plan"), (data, torch.uint8, "data"), (coef, torch.int16, "coef"),
+                            (out, torch.uint8, "out"), (status, torch.int32, "status")):
+            _chk_dev(t, dt, name, self.device)
+        if status.numel() < n:
+            raise NativeError(f"status holds {status.numel()} entries, {n} needed")
+        self._call("spn_jpeg_decode_gray", self.handle, _ptr(plan), _ptr(data), int(n), _ptr(coef), C.c_int64(coef.numel() * 2),
+                   _ptr(out), _ptr(status), self._s())
 
     def invert3x3(self, m):
         m = _dense(m)

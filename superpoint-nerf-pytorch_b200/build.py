@@ -1,4 +1,4 @@
-"""Build libspn_b200.so (the C-ABI library of include/spn_b200.h) in-tree with nvcc for sm_100a.
+"""Build libspn_b200.so (the C-ABI library of include/spn_b200.h and include/spn_jpeg.h) in-tree with nvcc for sm_100a.
 
     python superpoint-nerf-pytorch_b200/build.py [--force]
 
@@ -13,7 +13,7 @@ from pathlib import Path
 HERE = Path(__file__).resolve().parent
 CSRC = HERE / "csrc"
 SO = HERE / "libspn_b200.so"
-SOURCES = ["spn_api.cu", "conv_fp32.cu", "conv_tc.cu", "conv_fold.cu", "conv_split.cu", "front_tc.cu", "head_tc.cu", "geometry.cu", "nms.cu", "desc.cu", "eval.cu", "labels.cu"]
+SOURCES = ["spn_api.cu", "conv_fp32.cu", "conv_tc.cu", "conv_fold.cu", "conv_split.cu", "front_tc.cu", "head_tc.cu", "geometry.cu", "nms.cu", "desc.cu", "eval.cu", "labels.cu", "jpeg.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 
@@ -22,7 +22,8 @@ def needs_build() -> bool:
     if not SO.exists():
         return True
     t = SO.stat().st_mtime
-    deps = list(CSRC.glob("*.cu")) + list(CSRC.glob("*.cuh")) + [HERE.parent / "include" / "spn_b200.h", Path(__file__)]
+    deps = list(CSRC.glob("*.cu")) + list(CSRC.glob("*.cuh")) + [HERE.parent / "include" / "spn_b200.h",
+                                                                HERE.parent / "include" / "spn_jpeg.h", Path(__file__)]
     return any(d.stat().st_mtime > t for d in deps)
 
 

@@ -3,12 +3,15 @@
     ratio_preserving_resize      <- data/COCO.py:66-76, data/HPatches.py:64-72 (+ the "/= 255." of COCO.py:135)
     adapt_homography_to_resize   <- data/HPatches.py:74-100
 
-Image decoding stays with torchvision on the host (as in the reference); everything after the decode is one kernel
-(spn_resize_crop) that takes the decoded uint8 image, so the host->device copy is 1 byte/pixel.
+Image decoding runs with torchvision on the host (as in the reference), or, with ``data.decode: device``, for a batch
+of baseline JPEG files on the GPU (``launch_jpeg_decode`` / ``finish_jpeg_decode``, bit-identical to the host decode); everything after
+the decode is one kernel (spn_resize_crop) that takes the decoded uint8 image, so the host->device copy is 1
+byte/pixel (or the compressed file).
 """
+import numpy as np
 import torch
 
-from .._native import get_context
+from .._native import get_context, jpeg_plan
 
 
 def resize_geometry(src_shape, target):
@@ -77,6 +80,72 @@ def ratio_preserving_resize(image, target, normalize=True, device=None):
         image = image.to(dev, non_blocking=True)
         out = get_context(dev).resize_crop(image, nh, nw, top, left, int(target[0]), int(target[1]), scale)
     out.record_stream(cur)
+    cur.wait_stream(side)
+    return out
+
+
+def _resolve(device):
+    dev = torch.device(device) if device is not None else torch.device("cuda")
+    return torch.device("cuda", torch.cuda.current_device()) if dev.index is None else dev
+
+
+_decode_streams = {}
+
+
+def launch_jpeg_decode(files, device=None):
+    """Start the device decode of JPEG files (uint8 numpy arrays of the file bytes) -> handle for finish_jpeg_decode.
+
+    One plan (host header parse), one pinned upload of the concatenated files, one spn_jpeg_decode_gray and one status
+    read-back on a decode stream of its own, so a decode in flight never delays the resizes the loader's side stream
+    runs for the consumer.  Nothing here waits for the GPU."""
+    dev = _resolve(device)
+    offsets = np.zeros(len(files) + 1, np.int64)
+    np.cumsum([len(f) for f in files], out=offsets[1:])
+    host = torch.empty(int(offsets[-1]), dtype=torch.uint8, pin_memory=True)
+    np.concatenate(files, out=host.numpy())
+    plan, info, coef_bytes, out_bytes = jpeg_plan(host.numpy(), offsets)
+    n = len(files)
+    ctx = get_context(dev)
+    if dev.index not in _decode_streams:
+        _decode_streams[dev.index] = torch.cuda.Stream(device=dev)
+    stream = _decode_streams[dev.index]
+    with torch.cuda.stream(stream):
+        d_data = host.to(dev, non_blocking=True)
+        d_plan = torch.from_numpy(plan).pin_memory().to(dev, non_blocking=True)
+        coef = torch.empty(coef_bytes // 2, dtype=torch.int16, device=dev)
+        planes = torch.empty(max(out_bytes, 1), dtype=torch.uint8, device=dev)
+        status = torch.empty(n, dtype=torch.int32, device=dev)
+        ctx.jpeg_decode_gray(d_plan, d_data, n, coef, planes, status)
+        status_host = torch.empty(n, dtype=torch.int32, pin_memory=True)
+        status_host.copy_(status, non_blocking=True)
+        done = torch.cuda.Event()
+        done.record(stream)
+    return {"dev": dev, "ctx": ctx, "info": info, "planes": planes, "status": status_host, "done": done, "stream": stream}
+
+
+def finish_jpeg_decode(handle, target, normalize=True):
+    """-> list of (H,W) fp32 CUDA images (ratio_preserving_resize of the grayscale decode), None where the device decoder
+    did not decode the file (the caller decodes it on the host).  Waits for the decode's event only (never for the
+    consumer's stream); the resizes run on the loader's side stream after that event, and the consumer's stream waits
+    for the side stream."""
+    dev, ctx, info, planes = handle["dev"], handle["ctx"], handle["info"], handle["planes"]
+    handle["done"].synchronize()
+    status = handle["status"].numpy()
+    cur, side = torch.cuda.current_stream(dev), _upload_stream(dev)
+    side.wait_event(handle["done"])
+    planes.record_stream(side)
+    scale = 255.0 if normalize else 1.0
+    out = []
+    with torch.cuda.stream(side):
+        for i in range(len(status)):
+            if status[i] != 0:
+                out.append(None)
+                continue
+            h, w, off = int(info[i, 1]), int(info[i, 2]), int(info[i, 4])
+            nh, nw, top, left = resize_geometry((h, w), target)
+            img = ctx.resize_crop(planes[off:off + h * w].view(h, w), nh, nw, top, left, int(target[0]), int(target[1]), scale)
+            img.record_stream(cur)
+            out.append(img)
     cur.wait_stream(side)
     return out
 
