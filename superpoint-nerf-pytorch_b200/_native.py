@@ -1,4 +1,4 @@
-"""ctypes binding of include/spn_b200.h and include/spn_jpeg.h.  PyTorch is used only for device memory and streams."""
+"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h and include/spn_nerf.h.  PyTorch is used only for device memory and streams."""
 from __future__ import annotations
 
 import ctypes as C
@@ -74,6 +74,10 @@ JPEG_PROTOTYPES = {
     "spn_jpeg_plan": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "spn_jpeg_decode_gray": (_i, [_vp, _vp, _vp, _i, _vp, C.c_int64, _vp, _vp, _vp]),
 }
+# name -> (restype, argtypes); must list every symbol include/spn_nerf.h declares
+NERF_PROTOTYPES = {
+    "spn_nerf_fuse": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+}
 JPEG_OK, JPEG_UNSUPPORTED, JPEG_MALFORMED = 0, 1, 2
 JPEG_INFO_FIELDS = 5
 
@@ -102,7 +106,7 @@ def load_library():
                     raise NativeError(f"{_LIB_PATH} not found and building it failed ({e}); build it with "
                                       "`python superpoint-nerf-pytorch_b200/build.py` (there is no CPU/PyTorch fallback)")
             lib = C.CDLL(str(_LIB_PATH))
-            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES).items():
+            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES).items():
                 fn = getattr(lib, name)
                 fn.restype, fn.argtypes = res, args
             _lib = lib
@@ -431,6 +435,39 @@ class Context:
         out = torch.empty((H, W), dtype=torch.float32, device=prob_src.device)
         self._call("spn_nerf_splat", self.handle, _ptr(prob_src), _ptr(dst_pts) if n else None, _ptr(src_pts) if n else None, n, H, W,
                    _ptr(out), self._s())
+        return out
+
+    def nerf_fuse(self, prob, kp, kp_count, depth, K, R, t, targets, offsets, sources):
+        """Fused NeRF label heatmaps of one batch (spn_nerf_fuse): prob (V,H,W) fp32, kp (V,max_kp,2) int32 (row, col),
+        kp_count (V,) int32, depth (V,H,W) fp32, K / R (V,3,3) fp32, t (V,3,1) or (V,3) fp32, all CUDA; targets (n,)
+        view indices, offsets (n+1,) and sources (offsets[n],) the CSR list of each target's source views (host
+        sequences).  -> (n,H,W): out[i] = (prob[targets[i]] + sum of the source splats, in order) / (1 + n_sources)."""
+        import numpy as np
+        prob, kp, kp_count, depth = _dense(prob), _dense(kp), _dense(kp_count), _dense(depth)
+        for x, dt, name in ((prob, torch.float32, "prob"), (kp, torch.int32, "kp"), (kp_count, torch.int32, "kp_count"),
+                            (depth, torch.float32, "depth")):
+            _chk_dev(x, dt, name, self.device)
+        V, H, W = prob.shape
+        if kp.dim() != 3 or kp.shape[0] != V or kp.shape[2] != 2 or tuple(kp_count.shape) != (V,) or tuple(depth.shape) != (V, H, W):
+            raise NativeError(f"nerf_fuse: kp {tuple(kp.shape)}, kp_count {tuple(kp_count.shape)}, depth {tuple(depth.shape)} "
+                              f"do not match prob {(V, H, W)}")
+        mats = []
+        for x, n, name in ((K, 9, "K"), (R, 9, "R"), (t, 3, "t")):
+            x = _dense(x)
+            _chk_dev(x, torch.float32, name, self.device)
+            if x.numel() != V * n:
+                raise NativeError(f"nerf_fuse: {name} has shape {tuple(x.shape)}, expected {V} x {n} values")
+            mats.append(x)
+        tg = np.ascontiguousarray(np.asarray(targets, dtype=np.int64).reshape(-1).astype(np.int32))
+        off = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(-1).astype(np.int32))
+        src = np.ascontiguousarray(np.asarray(sources, dtype=np.int64).reshape(-1).astype(np.int32))
+        if len(off) != len(tg) + 1 or (len(off) and int(off[-1]) != len(src)):
+            raise NativeError(f"nerf_fuse: {len(tg)} targets need {len(tg) + 1} offsets ending at len(sources) = {len(src)}, "
+                              f"got {off.tolist()[:8]}{'...' if len(off) > 8 else ''}")
+        out = torch.empty((len(tg), H, W), dtype=torch.float32, device=prob.device)
+        hp = lambda a: C.c_void_p(a.ctypes.data) if a.size else None  # noqa: E731
+        self._call("spn_nerf_fuse", self.handle, _ptr(prob), _ptr(kp), _ptr(kp_count), int(kp.shape[1]), _ptr(depth), *map(_ptr, mats),
+                   V, H, W, len(tg), hp(tg), hp(off), hp(src), _ptr(out), self._s())
         return out
 
     # ---- on-GPU evaluation (evaluations/*.py of the reference) -----------------------------------

@@ -9,8 +9,10 @@ Same YAML schema as the reference (``data``, ``homography_adaptation``, ``model`
   * ``get_loader`` is this package's (utils/data_loaders.py): the reference's COCO / HPatches dataset classes mirrored for
     the export tasks, decoding on host threads and resizing on the GPU; ``--synthetic N`` feeds N synthetic images of
     the configured size instead;
-  * ``train`` and ``export_NeRF_labels`` are out of scope: their flags (``--training.*``) parse exactly as in the
-    reference, the task itself is rejected at dispatch;
+  * ``export_NeRF_labels`` reads posed multi-view scenes in this package's own layout (data/PosedViews.py, config
+    ``configs/magicpoint_nerf_export.yaml``, not the reference's NeRF dataset layout) and runs ExportNeRFDetections;
+  * ``train`` is out of scope: its flags (``--training.*``) parse exactly as in the reference, the task itself is
+    rejected at dispatch;
   * under ``torchrun`` (WORLD_SIZE > 1) every rank selects ``cuda:LOCAL_RANK``, joins the NCCL process group and takes
     the dataset items with index = rank (mod world): no two ranks write the same file (SURVEY.md section 8e).
 """
@@ -26,7 +28,8 @@ import tyro
 import yaml
 
 from . import settings
-from .engine_solvers.export import Export_Hpatches_Descriptors, Export_Hpatches_Repeatability, ExportDetections
+from .engine_solvers.export import (Export_Hpatches_Descriptors, Export_Hpatches_Repeatability, ExportDetections,
+                                   ExportNeRFDetections)
 from .utils.get_model import get_model
 from .utils.sharding import shard_indices
 
@@ -141,9 +144,10 @@ def main(config_path: str,
         synthetic: feed this many synthetic images instead of the dataset loader.
         random_init: skip loading `pretrained` (benchmarking with random-init weights, torch.manual_seed(0) on every rank).
     """
-    if task in ("train", "export_NeRF_labels"):   # ExportNeRFDetections is available as a class (engine_solvers/export.py); the NeRF
-        # dataset loader that feeds it is not part of this package
+    if task == "train":
         raise SystemExit(f"task {task!r} is outside the B200 hot path (SURVEY.md section 8); use the reference for it")
+    if task == "export_NeRF_labels" and synthetic:
+        raise SystemExit("--synthetic feeds single images; export_NeRF_labels needs posed views (data/PosedViews.py)")
     with open(config_path, "r") as f:
         config = yaml.safe_load(f)
     if not torch.cuda.is_available():
@@ -164,6 +168,8 @@ def main(config_path: str,
         if world > 1:   # device-sampler key = global dataset index: rank-strided items, see ExportDetections
             config.setdefault("homography_adaptation", {}).update(index_stride=world, index_offset=rank)
         ExportDetections(config, model, loader, pseudo_labels.split, pseudo_labels.enable_Homography_Adaptation, device)
+    elif task == "export_NeRF_labels":
+        ExportNeRFDetections(config, model, loader, pseudo_labels.split, device)
     elif task == "export_HPatches_Repeatability":
         Export_Hpatches_Repeatability(config, model, loader, device)
     else:

@@ -418,10 +418,13 @@ class ExportNeRFDetections:
     ``<EXPER_PATH>/outputs/<experiment>/<split>/<name>.npy``.
 
     What changes underneath: the reference runs the model once per (j, k) pair; here every view is forwarded ONCE through
-    the one-call path (heatmap + NMS + keypoint list, spn_detect_describe), the sequential 3x3 patch copies of
-    export.py:271-283 are one order-preserving kernel (spn_nerf_splat) and the final NMS is the bit-exact box_nms kernel.
-    The pairing quirk of export.py:269-271 (the border filter shortens ``unwarped_pts`` but the loop zips it with the
-    unfiltered ``warped_pts``) is reproduced as is."""
+    the one-call path (heatmap + NMS + keypoint list, spn_detect_describe), the source views are drawn with python's
+    ``random.choices`` exactly as in export.py:320-321, and then ONE spn_nerf_fuse call builds the averaged heatmaps of
+    every target view of the batch (re-projection, border filter, ordered 3x3 patch copies and the running sum in two
+    kernels), followed by one batched bit-exact box_nms and one copy to the host.  The pairing quirk of export.py:269-271
+    (the border filter shortens ``unwarped_pts`` but the loop zips it with the unfiltered ``warped_pts``) is reproduced
+    as is.  ``reproject`` is the per-pair composition (warp_points_NeRF -> filter_points -> spn_nerf_splat) that the
+    fused kernel is tested against."""
 
     def __init__(self, config, model, dataloader, split, device):
         self.config = config
@@ -448,6 +451,20 @@ class ExportNeRFDetections:
         return ctx.nerf_splat(prob_k, unwarped.to(torch.float32).contiguous(), pts_k[:n].contiguous())
 
     @torch.no_grad()
+    def fuse_per_pair(self, prob, kp, cnt, data, targets, offsets, sources):
+        """What spn_nerf_fuse computes, one ``reproject`` per (target, source) pair as export.py:322-325 does:
+        -> (n_targets,H,W) = stack([prob[j]] + splats).sum(0) / (1 + n) per target."""
+        raw, K = data["raw"], data["camera_intrinsic_matrix"]
+        out = []
+        for t, j in enumerate(targets):
+            maps = [prob[j]]
+            for k in sources[offsets[t]:offsets[t + 1]]:
+                maps.append(self.reproject(prob[k], kp[k, :cnt[k]], raw["input_depth"][k], K[j], raw["input_rotation"][k],
+                                           raw["input_translation"][k], raw["input_rotation"][j], raw["input_translation"][j]))
+            out.append(torch.stack(maps).sum(0) / float(len(maps)))
+        return torch.stack(out)
+
+    @torch.no_grad()
     def export_NeRF(self):
         import random
         dh = self.config["model"]["detector_head"]
@@ -461,27 +478,47 @@ class ExportNeRFDetections:
             prob, kp, cnt = out["prob_heatmap"], out["keypoints"], out["keypoint_count"].cpu().numpy()
             if cnt.max(initial=0) > kp.shape[1]:
                 raise RuntimeError("keypoint list overflow: set detector_head.top_k")
+            # the targets and their source views, drawn in the reference's order (export.py:316-321); a view whose file
+            # exists - or that an earlier view of the batch with the same name will write - is skipped without a draw
+            targets, offsets, sources, paths, planned = [], [0], [], [], set()
             for j in range(len(names)):
                 save_path = Path(self.output_dir, f"{names[j]}.npy")
-                if save_path.exists():
+                if save_path.exists() or save_path in planned:
                     continue
                 other_index = [k for k in range(len(names)) if k != j]
                 other_index = random.choices(other_index, k=int(0.75 * len(other_index)))     # export.py:320-321, python's RNG
-                maps = [prob[j]]
-                for k in other_index:
-                    maps.append(self.reproject(prob[k], kp[k, :cnt[k]], data["raw"]["input_depth"][k], data["camera_intrinsic_matrix"][j],
-                                               data["raw"]["input_rotation"][k], data["raw"]["input_translation"][k],
-                                               data["raw"]["input_rotation"][j], data["raw"]["input_translation"][j]))
-                mean = torch.stack(maps).sum(0) / float(len(maps))
-                ctx = self.model.native()
-                cap = min(mean.numel(), 16384)
-                r = ctx.box_nms(mean.unsqueeze(0), float(dh["nms"]), 0.1, float(dh["det_thresh"]), int(dh["top_k"]),
-                                det_thresh=float(dh["det_thresh"]), want_map=False, max_kp=cap)
-                n = int(r["kp_count"][0])
-                if n > cap:                            # more keypoints than the list holds: redo with the true size
-                    r = ctx.box_nms(mean.unsqueeze(0), float(dh["nms"]), 0.1, float(dh["det_thresh"]), int(dh["top_k"]),
-                                    det_thresh=float(dh["det_thresh"]), want_map=False, max_kp=n)
-                np.save(save_path, r["kp"][0, :n].cpu().numpy().astype(np.int64))
+                targets.append(j)
+                sources += other_index
+                offsets.append(len(sources))
+                paths.append(save_path)
+                planned.add(save_path)
+            raw = data["raw"]
+            ctx = self.model.native()
+            mean = ctx.nerf_fuse(prob, kp, out["keypoint_count"], raw["input_depth"].to(torch.float32),
+                                 data["camera_intrinsic_matrix"].to(torch.float32), raw["input_rotation"].to(torch.float32),
+                                 raw["input_translation"].to(torch.float32), targets, offsets, sources)
+            for path, kp_t in zip(paths, self._keypoints(ctx, mean, dh)):
+                np.save(path, kp_t)
+
+    @staticmethod
+    def _keypoints(ctx, heat, dh):
+        """box_nms + threshold + nonzero of every fused heatmap (export.py:326-334): one batched call, one copy to the
+        host (-> list of (N,2) int64 arrays)."""
+        cap = min(heat[0].numel(), 16384)
+        for _ in range(2):
+            r = ctx.box_nms(heat, float(dh["nms"]), 0.1, float(dh["det_thresh"]), int(dh["top_k"]),
+                            det_thresh=float(dh["det_thresh"]), want_map=False, max_kp=cap)
+            kp_h = torch.empty(r["kp"].shape, dtype=torch.int32, pin_memory=True)
+            cnt_h = torch.empty(r["kp_count"].shape, dtype=torch.int32, pin_memory=True)
+            kp_h.copy_(r["kp"], non_blocking=True)
+            cnt_h.copy_(r["kp_count"], non_blocking=True)
+            torch.cuda.current_stream(heat.device).synchronize()
+            counts = cnt_h.numpy()
+            if counts.max(initial=0) <= cap:
+                break
+            cap = int(counts.max())                   # more keypoints than the list holds: redo with the true size
+        kp = kp_h.numpy()
+        return [kp[i, :counts[i]].astype(np.int64) for i in range(len(counts))]
 
 
 def load_packed_labels(directory):

@@ -6,7 +6,8 @@ decoded at a time on the loop's thread) it returns a ``PrefetchLoader``: the hos
 JPEG/PPM decode, which release the GIL) runs on a thread pool a bounded number of items ahead, the device part (one
 resize/crop/normalise kernel per image on the uint8 pixels) runs on the consumer's thread and stream.  It yields the
 same collated batch dictionaries in the same order; rank sharding (``rank``/``world``) takes items with
-index = rank (mod world) BEFORE anything is decoded.  A dataset that has ``finish_batch`` (COCO with ``data.decode:
+index = rank (mod world) BEFORE anything is decoded.  ``export_NeRF_labels`` items are whole chunks of posed views
+(data/PosedViews.py), loaded one per batch.  A dataset that has ``finish_batch`` (COCO with ``data.decode:
 device``) gets up to ``device_batch`` ready items at a time, in order, for one batched device stage.  The stage is
 launched when its items are ready and its results are taken one batch later, so the wait for one batch overlaps the
 gathering and launch of the next.  Items before one that fails are yielded before the exception, as without the stage.
@@ -74,8 +75,11 @@ def get_loader(config, task, device="cuda", validate_training=False, export_spli
     name, class_name = config["data"]["name"], config["data"]["class_name"]
     batch_size = config["data"]["batch_size"]
     cls = getattr(importlib.import_module(f"{_DATA_PACKAGE}.{name}"), class_name)
-    if task in ("train", "test", "export_NeRF_labels") or validate_training or nerf_train:
+    if task in ("train", "test") or validate_training or nerf_train:
         raise NotImplementedError(f"task {task!r} is outside the B200 hot path (SURVEY.md section 8): use the reference's loader")
+    if task == "export_NeRF_labels":              # one item = one chunk of posed views (data/PosedViews.py)
+        dataset = cls(config["data"], task=export_split, device=device)
+        return PrefetchLoader(dataset, 1, workers=config["data"].get("loader_workers"), rank=rank, world=world)
     if task == "export_pseudo_labels":
         dataset = cls(config["data"], task=export_split, device=device)
     elif task in ("export_HPatches_Repeatability", "export_HPatches_Descriptors"):
