@@ -1,4 +1,4 @@
-"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h and include/spn_nerf.h.  PyTorch is used only for device memory and streams."""
+"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h and include/spn_posed.h.  PyTorch is used only for device memory and streams."""
 from __future__ import annotations
 
 import ctypes as C
@@ -78,6 +78,11 @@ JPEG_PROTOTYPES = {
 NERF_PROTOTYPES = {
     "spn_nerf_fuse": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
 }
+# name -> (restype, argtypes); must list every symbol include/spn_posed.h declares
+POSED_PROTOTYPES = {
+    "spn_posed_reproject": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, C.c_double, _vp, _vp, _vp, _vp, _vp,
+                                 _vp]),
+}
 JPEG_OK, JPEG_UNSUPPORTED, JPEG_MALFORMED = 0, 1, 2
 JPEG_INFO_FIELDS = 5
 
@@ -106,7 +111,7 @@ def load_library():
                     raise NativeError(f"{_LIB_PATH} not found and building it failed ({e}); build it with "
                                       "`python superpoint-nerf-pytorch_b200/build.py` (there is no CPU/PyTorch fallback)")
             lib = C.CDLL(str(_LIB_PATH))
-            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES).items():
+            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES | POSED_PROTOTYPES).items():
                 fn = getattr(lib, name)
                 fn.restype, fn.argtypes = res, args
             _lib = lib
@@ -471,6 +476,44 @@ class Context:
         return out
 
     # ---- on-GPU evaluation (evaluations/*.py of the reference) -----------------------------------
+    def posed_reproject(self, kp, kp_count, depth, K, R, t, pairs, depth_tol):
+        """Keypoints of view a reprojected into view b for every pair (spn_posed_reproject): kp (V,max_kp,2) int32 (row,
+        col), kp_count (V,) int32, depth (V,H,W) fp32 ray depth, K / R (V,3,3) fp32, t (V,3,1) or (V,3) fp32, all CUDA;
+        pairs (P,2) host (a, b) view indices.  -> dict with proj (P,max_kp,2) float64 (a's keypoints in b, NaN where
+        undefined), vis (P,2,max_kp) int32 (a visible in b, b visible in a), set1 / set2 (P,max_kp,2) float64 (the
+        compacted visible points, both in b's frame) and set_count (P,2) int32."""
+        import numpy as np
+        kp, kp_count, depth = _dense(kp), _dense(kp_count), _dense(depth)
+        for x, dt, name in ((kp, torch.int32, "kp"), (kp_count, torch.int32, "kp_count"), (depth, torch.float32, "depth")):
+            _chk_dev(x, dt, name, self.device)
+        if depth.dim() != 3 or kp.dim() != 3 or kp.shape[0] != depth.shape[0] or kp.shape[2] != 2 or \
+                tuple(kp_count.shape) != (depth.shape[0],):
+            raise NativeError(f"posed_reproject: kp {tuple(kp.shape)}, kp_count {tuple(kp_count.shape)} do not match depth "
+                              f"{tuple(depth.shape)} (V,H,W)")
+        V, H, W = depth.shape
+        mats = []
+        for x, n, name in ((K, 9, "K"), (R, 9, "R"), (t, 3, "t")):
+            x = _dense(x)
+            _chk_dev(x, torch.float32, name, self.device)
+            if x.numel() != V * n:
+                raise NativeError(f"posed_reproject: {name} has shape {tuple(x.shape)}, expected {V} x {n} values")
+            mats.append(x)
+        pr = np.asarray(pairs, dtype=np.int64)
+        if pr.size == 0:
+            pr = pr.reshape(0, 2)
+        if pr.ndim != 2 or pr.shape[1] != 2:
+            raise NativeError(f"posed_reproject: pairs must be (P, 2), got shape {pr.shape}")
+        pr = np.ascontiguousarray(pr.astype(np.int32))
+        P, max_kp = len(pr), int(kp.shape[1])
+        f64 = dict(dtype=torch.float64, device=depth.device)
+        out = {"proj": torch.empty((P, max_kp, 2), **f64), "vis": torch.empty((P, 2, max_kp), dtype=torch.int32, device=depth.device),
+               "set1": torch.empty((P, max_kp, 2), **f64), "set2": torch.empty((P, max_kp, 2), **f64),
+               "set_count": torch.empty((P, 2), dtype=torch.int32, device=depth.device)}
+        self._call("spn_posed_reproject", self.handle, _ptr(kp), _ptr(kp_count), max_kp, _ptr(depth), *map(_ptr, mats), V, H, W, P,
+                   C.c_void_p(pr.ctypes.data) if P else None, C.c_double(float(depth_tol)),
+                   *[_ptr(out[k]) if P else None for k in ("proj", "vis", "set1", "set2", "set_count")], self._s())
+        return out
+
     SELECT_CAP = 16384
 
     def select_keypoints(self, prob, warp=None, bounds=None, emit_warped=False, keep_k=300):

@@ -1,4 +1,4 @@
-"""Build libspn_b200.so (the C-ABI library of include/spn_b200.h, include/spn_jpeg.h and include/spn_nerf.h) in-tree with nvcc for sm_100a.
+"""Build libspn_b200.so (the C-ABI library of include/spn_b200.h, spn_jpeg.h, spn_nerf.h and spn_posed.h) in-tree with nvcc for sm_100a.
 
     python superpoint-nerf-pytorch_b200/build.py [--force]
 
@@ -24,7 +24,8 @@ def needs_build() -> bool:
     t = SO.stat().st_mtime
     deps = list(CSRC.glob("*.cu")) + list(CSRC.glob("*.cuh")) + [HERE.parent / "include" / "spn_b200.h",
                                                                 HERE.parent / "include" / "spn_jpeg.h",
-                                                                HERE.parent / "include" / "spn_nerf.h", Path(__file__)]
+                                                                HERE.parent / "include" / "spn_nerf.h",
+                                                                HERE.parent / "include" / "spn_posed.h", Path(__file__)]
     return any(d.stat().st_mtime > t for d in deps)
 
 

@@ -15,10 +15,14 @@
 //                             accumulator row and publishes the row-wise arg-min with one 64-bit atomicMin
 //                             (distance bits, index): ties go to the lower index like cv2.
 //   cross_check_kernel        crossCheck=True: keep (i, j) iff j is i's nearest and i is j's nearest
+//   posed_reproject_kernel    spn_posed_reproject (include/spn_posed.h): one CTA per (pair, direction); every keypoint
+//                             through depth and both poses in explicitly rounded fp64, the visibility / occlusion test,
+//                             the visible points compacted in keypoint order with a ballot and block scan
 #include <math.h>
 
 #include "spn_common.cuh"
 #include "tc_ptx.cuh"
+#include "../../include/spn_posed.h"
 
 namespace {
 
@@ -318,6 +322,136 @@ __global__ void cross_check_kernel(const unsigned long long* __restrict__ bq, co
   dist[(size_t)b * qcap + i] = d;
 }
 
+// ------------------------------------------------------------------------------------------------ posed reprojection
+// Every operation is a separately rounded intrinsic so that a numpy restatement in the same order (oracle/posed_oracle.py)
+// gives the same bits: nvcc would otherwise contract a * b + c into an FMA.
+constexpr int kPosedThreads = 256;
+
+__device__ __forceinline__ double dmul(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ double dadd(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ double dsub(double a, double b) { return __dsub_rn(a, b); }
+
+// row of a 3x3 product: (m0 x + m1 y) + m2 z
+__device__ __forceinline__ double drow(const double* m, double x, double y, double z) {
+  return dadd(dadd(dmul(m[0], x), dmul(m[1], y)), dmul(m[2], z));
+}
+
+__device__ __forceinline__ double dnorm3(double x, double y, double z) {
+  return __dsqrt_rn(dadd(dadd(dmul(x, x), dmul(y, y)), dmul(z, z)));
+}
+
+// inverse of a 3x3 fp32 matrix: the adjugate divided by the determinant, in fp64 (labels.cu inverse3x3 without the
+// final rounding to float)
+__device__ void inverse3x3_d(const float* m, double* o) {
+  const double a = m[0], b = m[1], c = m[2], d = m[3], e = m[4], f = m[5], g = m[6], h = m[7], i = m[8];
+  const double c00 = dsub(dmul(e, i), dmul(f, h)), c01 = dsub(dmul(f, g), dmul(d, i)), c02 = dsub(dmul(d, h), dmul(e, g));
+  const double det = dadd(dadd(dmul(a, c00), dmul(b, c01)), dmul(c, c02));
+  o[0] = __ddiv_rn(c00, det); o[1] = __ddiv_rn(dsub(dmul(c, h), dmul(b, i)), det); o[2] = __ddiv_rn(dsub(dmul(b, f), dmul(c, e)), det);
+  o[3] = __ddiv_rn(c01, det); o[4] = __ddiv_rn(dsub(dmul(a, i), dmul(c, g)), det); o[5] = __ddiv_rn(dsub(dmul(c, d), dmul(a, f)), det);
+  o[6] = __ddiv_rn(c02, det); o[7] = __ddiv_rn(dsub(dmul(b, g), dmul(a, h)), det); o[8] = __ddiv_rn(dsub(dmul(a, e), dmul(b, d)), det);
+}
+
+struct PosedParams {
+  const int32_t* kp;        // [V][max_kp][2] (row, col)
+  const int32_t* kp_count;  // [V]
+  const float* depth;       // [V][H][W]
+  const float* K;           // [V][9]
+  const float* R;           // [V][9]
+  const float* t;           // [V][3]
+  const int* pairs;         // [P][2] (a, b), uploaded
+  int H, W, max_kp;
+  double depth_tol;
+  double* proj;             // [P][max_kp][2]
+  int* vis;                 // [P][2][max_kp]
+  double* set1;             // [P][max_kp][2]
+  double* set2;             // [P][max_kp][2]
+  int* set_count;           // [P][2]
+};
+
+// blockIdx.x = 2 q + dir.  dir 0: keypoints of a into b (proj, vis[q][0], set 1 at the projected positions); dir 1:
+// keypoints of b into a (vis[q][1], set 2 at b's own integer positions).
+__global__ void __launch_bounds__(kPosedThreads) posed_reproject_kernel(const PosedParams p) {
+  __shared__ double Ks[9], Kinv[9], Rs[9], Rinv[9], ts[3], tdst[3];
+  __shared__ int warp_n[kPosedThreads / 32];
+  __shared__ int base;
+  const int q = blockIdx.x >> 1, dir = blockIdx.x & 1;
+  const int a = p.pairs[2 * q], b = p.pairs[2 * q + 1];
+  const int src = dir ? b : a, dst = dir ? a : b;
+  if (threadIdx.x == 0) {
+    inverse3x3_d(p.K + src * 9, Kinv);
+    inverse3x3_d(p.R + dst * 9, Rinv);
+    for (int e = 0; e < 9; ++e) { Ks[e] = p.K[dst * 9 + e]; Rs[e] = p.R[src * 9 + e]; }
+    for (int e = 0; e < 3; ++e) { ts[e] = p.t[src * 3 + e]; tdst[e] = p.t[dst * 3 + e]; }
+    base = 0;
+  }
+  __syncthreads();
+  const int H = p.H, W = p.W, max_kp = p.max_kp;
+  const int n = min(max(p.kp_count[src], 0), max_kp);
+  const int32_t* P = p.kp + (size_t)src * max_kp * 2;
+  const float* Dsrc = p.depth + (size_t)src * H * W;
+  const float* Ddst = p.depth + (size_t)dst * H * W;
+  int* vis = p.vis + ((size_t)q * 2 + dir) * max_kp;
+  double* proj = p.proj + (size_t)q * max_kp * 2;
+  double* set = (dir ? p.set2 : p.set1) + (size_t)q * max_kp * 2;
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int c0 = 0; c0 < max_kp; c0 += kPosedThreads) {   // slots past n are written too (vis 0, proj NaN)
+    const int i = c0 + threadIdx.x;
+    bool visible = false;
+    int r = 0, c = 0;
+    double row = nan, col = nan;
+    if (i < n) {
+      r = P[2 * i];
+      c = P[2 * i + 1];
+      if (r >= 0 && r < H && c >= 0 && c < W) {
+        const double d = (double)Dsrc[(size_t)r * W + c];
+        const double x = (double)c, y = (double)r;
+        const double ray0 = dadd(dadd(dmul(Kinv[0], x), dmul(Kinv[1], y)), Kinv[2]);
+        const double ray1 = dadd(dadd(dmul(Kinv[3], x), dmul(Kinv[4], y)), Kinv[5]);
+        const double ray2 = dadd(dadd(dmul(Kinv[6], x), dmul(Kinv[7], y)), Kinv[8]);
+        const double nrm = dnorm3(ray0, ray1, ray2);
+        const double X0 = dmul(__ddiv_rn(ray0, nrm), d), X1 = dmul(__ddiv_rn(ray1, nrm), d), X2 = dmul(__ddiv_rn(ray2, nrm), d);
+        const double w0 = dsub(dadd(drow(Rs, X0, X1, X2), ts[0]), tdst[0]);
+        const double w1 = dsub(dadd(drow(Rs + 3, X0, X1, X2), ts[1]), tdst[1]);
+        const double w2 = dsub(dadd(drow(Rs + 6, X0, X1, X2), ts[2]), tdst[2]);
+        const double Y0 = drow(Rinv, w0, w1, w2), Y1 = drow(Rinv + 3, w0, w1, w2), Y2 = drow(Rinv + 6, w0, w1, w2);
+        const double p0 = drow(Ks, Y0, Y1, Y2), p1 = drow(Ks + 3, Y0, Y1, Y2), p2 = drow(Ks + 6, Y0, Y1, Y2);
+        row = __ddiv_rn(p1, p2);
+        col = __ddiv_rn(p0, p2);
+        if (!isfinite(row) || !isfinite(col)) { row = nan; col = nan; }
+        if (isfinite(d) && d > 0.0 && Y2 > 0.0 && row >= 0.0 && row <= (double)(H - 1) && col >= 0.0 && col <= (double)(W - 1)) {
+          const int nr = (int)floor(dadd(row, 0.5)), nc = (int)floor(dadd(col, 0.5));
+          const double db = (double)Ddst[(size_t)nr * W + nc];
+          visible = isfinite(db) && db > 0.0 && fabs(dsub(dnorm3(Y0, Y1, Y2), db)) <= dmul(p.depth_tol, db);
+        }
+      }
+    }
+    if (i < max_kp) {
+      vis[i] = visible ? 1 : 0;
+      if (dir == 0) { proj[2 * i] = row; proj[2 * i + 1] = col; }
+    }
+    // ordered compaction of the visible points (block-wide exclusive scan of the flags)
+    const unsigned ballot = __ballot_sync(0xffffffffu, visible);
+    if (lane == 0) warp_n[warp] = __popc(ballot);
+    __syncthreads();
+    int s = base + __popc(ballot & ((1u << lane) - 1u)), total = 0;
+    for (int w = 0; w < kPosedThreads / 32; ++w) {
+      s += w < warp ? warp_n[w] : 0;
+      total += warp_n[w];
+    }
+    if (visible) {
+      set[2 * s] = dir ? (double)r : row;
+      set[2 * s + 1] = dir ? (double)c : col;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) base += total;
+    __syncthreads();
+  }
+  const int count = base;
+  for (int i = count + threadIdx.x; i < max_kp; i += kPosedThreads) { set[2 * i] = nan; set[2 * i + 1] = nan; }
+  if (threadIdx.x == 0) p.set_count[2 * q + dir] = count;
+}
+
 }  // namespace
 
 extern "C" int spn_select_keypoints(spn_ctx* ctx, const float* d_prob, int B, int H, int W, const double* h_warp, int bound_h,
@@ -378,6 +512,36 @@ extern "C" int spn_mutual_nn_match(spn_ctx* ctx, const float* d_desc1, const int
   nn_match_tc_kernel<<<dim3(spn_cdiv(cap1, kNT), spn_cdiv(cap2, kMT), B), 128, dyn, s>>>(p);   // and the other direction
   SPN_CHECK_LAUNCH(ctx);
   cross_check_kernel<<<dim3(spn_cdiv(cap1, 128), B), 128, 0, s>>>(bq, bt, d_n1, d_n2, cap1, cap2, d_match, d_dist);
+  SPN_CHECK_LAUNCH(ctx);
+  return SPN_OK;
+}
+
+extern "C" int spn_posed_reproject(spn_ctx* ctx, const int32_t* d_kp, const int32_t* d_kp_count, int max_kp, const float* d_depth,
+                                   const float* d_K, const float* d_R, const float* d_t, int V, int H, int W, int P,
+                                   const int32_t* h_pairs, double depth_tol, double* d_proj, int32_t* d_vis, double* d_set1,
+                                   double* d_set2, int32_t* d_set_count, spn_stream stream) {
+  SPN_REQUIRE(ctx && d_kp && d_kp_count && d_depth && d_K && d_R && d_t, "spn_posed_reproject: null pointer");
+  SPN_REQUIRE(V > 0 && H > 0 && W > 0 && H <= 32767 && W <= 32767, "spn_posed_reproject: bad shape V=%d H=%d W=%d (need V > 0, 0 < H, W <= 32767)", V, H, W);
+  SPN_REQUIRE(max_kp > 0, "spn_posed_reproject: max_kp must be > 0 (got %d)", max_kp);
+  SPN_REQUIRE(P >= 0 && P <= 65535, "spn_posed_reproject: P = %d pairs outside [0, 65535]", P);
+  SPN_REQUIRE(isfinite(depth_tol) && depth_tol >= 0.0, "spn_posed_reproject: depth_tol must be finite and >= 0 (got %g)", depth_tol);
+  if (P == 0) return SPN_OK;
+  SPN_REQUIRE(h_pairs && d_proj && d_vis && d_set1 && d_set2 && d_set_count, "spn_posed_reproject: null pointer (h_pairs / outputs)");
+  for (int q = 0; q < P; ++q)
+    SPN_REQUIRE(h_pairs[2 * q] >= 0 && h_pairs[2 * q] < V && h_pairs[2 * q + 1] >= 0 && h_pairs[2 * q + 1] < V,
+                "spn_posed_reproject: pair %d = (%d, %d) has a view index outside [0, %d)", q, h_pairs[2 * q], h_pairs[2 * q + 1], V);
+  SpnDeviceGuard guard(ctx->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t bytes = (size_t)P * 2 * sizeof(int32_t);
+  int rc = spn_ensure_aux(ctx, bytes, s);
+  if (rc) return rc;
+  // pageable source: the call returns once the bytes are staged
+  SPN_CUDA(cudaMemcpyAsync(ctx->aux, h_pairs, bytes, cudaMemcpyHostToDevice, s));
+  PosedParams p;
+  p.kp = d_kp; p.kp_count = d_kp_count; p.depth = d_depth; p.K = d_K; p.R = d_R; p.t = d_t; p.pairs = (const int*)ctx->aux;
+  p.H = H; p.W = W; p.max_kp = max_kp; p.depth_tol = depth_tol;
+  p.proj = d_proj; p.vis = d_vis; p.set1 = d_set1; p.set2 = d_set2; p.set_count = d_set_count;
+  posed_reproject_kernel<<<2 * P, kPosedThreads, 0, s>>>(p);
   SPN_CHECK_LAUNCH(ctx);
   return SPN_OK;
 }
