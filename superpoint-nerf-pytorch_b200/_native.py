@@ -1,4 +1,4 @@
-"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h and include/spn_posed.h.  PyTorch is used only for device memory and streams."""
+"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h, include/spn_posed.h and include/spn_match.h.  PyTorch is used only for device memory and streams."""
 from __future__ import annotations
 
 import ctypes as C
@@ -83,6 +83,10 @@ POSED_PROTOTYPES = {
     "spn_posed_reproject": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, C.c_double, _vp, _vp, _vp, _vp, _vp,
                                  _vp]),
 }
+# name -> (restype, argtypes); must list every symbol include/spn_match.h declares
+MATCH_PROTOTYPES = {
+    "spn_match_pairs": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _i, _i, _f, _f, _vp, _vp, _vp]),
+}
 JPEG_OK, JPEG_UNSUPPORTED, JPEG_MALFORMED = 0, 1, 2
 JPEG_INFO_FIELDS = 5
 
@@ -111,7 +115,7 @@ def load_library():
                     raise NativeError(f"{_LIB_PATH} not found and building it failed ({e}); build it with "
                                       "`python superpoint-nerf-pytorch_b200/build.py` (there is no CPU/PyTorch fallback)")
             lib = C.CDLL(str(_LIB_PATH))
-            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES | POSED_PROTOTYPES).items():
+            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES | POSED_PROTOTYPES | MATCH_PROTOTYPES).items():
                 fn = getattr(lib, name)
                 fn.restype, fn.argtypes = res, args
             _lib = lib
@@ -560,6 +564,35 @@ class Context:
         dist = torch.empty((B, c1), dtype=torch.float32, device=desc1.device)
         self._call("spn_mutual_nn_match", self.handle, _ptr(desc1), _ptr(_dense(n1)), _ptr(desc2), _ptr(_dense(n2)), B, c1, c2, Cc,
                    _ptr(match), _ptr(dist), self._s())
+        return match, dist
+
+    MATCH_MAX_PAIRS = 65535
+
+    def match_pairs(self, desc, count, pairs, mutual=True, ratio=0.0, max_dist=float("inf")):
+        """Matches of pairs of a descriptor pool (spn_match_pairs, include/spn_match.h): desc (N,cap,C) fp32 and count
+        (N,) int32 CUDA (detect_describe's desc_sparse / kp_count), pairs (P,2) host (a, b) set indices, at most
+        MATCH_MAX_PAIRS.  -> (match (P,cap) int32 index into b or -1, dist (P,cap) fp32, 0 where there is no match)."""
+        import numpy as np
+        desc, count = _dense(desc), _dense(count)
+        _chk_dev(desc, torch.float32, "desc", self.device)
+        _chk_dev(count, torch.int32, "count", self.device)
+        if desc.dim() != 3 or tuple(count.shape) != (desc.shape[0],):
+            raise NativeError(f"match_pairs: desc {tuple(desc.shape)} must be (N,cap,C) and count {tuple(count.shape)} (N,)")
+        pr = np.asarray(pairs, dtype=np.int64)
+        if pr.size == 0:
+            pr = pr.reshape(0, 2)
+        if pr.ndim != 2 or pr.shape[1] != 2:
+            raise NativeError(f"match_pairs: pairs must be (P, 2), got shape {pr.shape}")
+        if pr.size and (pr.min() < np.iinfo(np.int32).min or pr.max() > np.iinfo(np.int32).max):
+            raise NativeError("match_pairs: a pair index does not fit int32")
+        pr = np.ascontiguousarray(pr.astype(np.int32))
+        N, cap, Cc = desc.shape
+        P = len(pr)
+        match = torch.empty((P, cap), dtype=torch.int32, device=desc.device)
+        dist = torch.empty((P, cap), dtype=torch.float32, device=desc.device)
+        self._call("spn_match_pairs", self.handle, _ptr(desc), _ptr(count), N, cap, Cc, C.c_void_p(pr.ctypes.data) if P else None, P,
+                   int(bool(mutual)), C.c_float(ratio), C.c_float(max_dist), _ptr(match) if P else None, _ptr(dist) if P else None,
+                   self._s())
         return match, dist
 
     def resize_crop(self, src: torch.Tensor, new_h, new_w, crop_top, crop_left, H, W, divisor=255.0):

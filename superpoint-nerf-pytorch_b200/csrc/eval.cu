@@ -8,7 +8,8 @@
 //                             numpy) + select_k_best (ascending by probability, last k): one CTA per map, candidates
 //                             compacted into shared memory and bitonic-sorted as 64-bit (prob bits, pixel index) keys
 //   repeat_count_kernel       N1 x N2 Euclidean distances in fp64, nearest-neighbour counts within the threshold
-//   nn_match_tc_kernel        cv2.BFMatcher(NORM_L2): the N1 x N2 x 256 distance matrix as a tcgen05 GEMM.  The fp32
+//   nn_match_tc_kernel        cv2.BFMatcher(NORM_L2): the N1 x N2 x 256 distance matrix as a tcgen05 GEMM (the tile is
+//                             in nn_tc.cuh, shared with match.cu).  The fp32
 //                             descriptors are split into fp16 (hi, lo) halves on the way into shared memory and the dot
 //                             product is accumulated as hi*hi + hi*lo + lo*hi in fp32 TMEM (error ~2^-22, i.e. fp32
 //                             quality on L2-normalised descriptors); the epilogue forms |a|^2 + |b|^2 - 2 a.b per
@@ -21,6 +22,7 @@
 #include <math.h>
 
 #include "spn_common.cuh"
+#include "nn_tc.cuh"
 #include "tc_ptx.cuh"
 #include "../../include/spn_posed.h"
 
@@ -167,11 +169,7 @@ __global__ void __launch_bounds__(256) repeat_count_kernel(const double* __restr
 }
 
 // ------------------------------------------------------------------------------------------------ NN matching on tcgen05
-constexpr int kMT = 128;            // query rows per CTA (TMEM lanes)
-constexpr int kNT = 128;            // train rows per CTA (accumulator columns)
-constexpr int kKC = 64;             // K elements staged per step (4 MMA K-steps of 16)
-constexpr int kPlane = kMT * 16;    // bytes of one 8-element K chunk for 128 rows: [row][8 halfs]
-constexpr int kOpBytes = (kKC / 8) * kPlane;   // 16 KB: one operand (hi or lo) of one K step
+using namespace nntc;
 
 struct MatchParams {
   const float* q;        // [B][qcap][C] query descriptors
@@ -181,39 +179,6 @@ struct MatchParams {
   int qcap, tcap, C;
   unsigned long long* best;   // [B][qcap]: (distance^2 bits << 32) | train index, initialised to ~0
 };
-
-// rows [row0, row0 + 128) x K [k0, k0 + 64) of src (row-major fp32, `n` valid rows) -> hi / lo fp16 operand images
-// [chunk 8][row 128][8]; returns this thread's partial |row|^2 (thread = row).
-__device__ __forceinline__ float stage_operand(const float* __restrict__ src, int n, int C, int row0, int k0, uint8_t* hi, uint8_t* lo) {
-  const int r = threadIdx.x;
-  const bool live = row0 + r < n;
-  const float4* g = reinterpret_cast<const float4*>(src + (size_t)(row0 + r) * C + k0);
-  float ss = 0.f;
-#pragma unroll
-  for (int c = 0; c < kKC / 8; ++c) {
-    float v[8];
-    if (live) {
-      const float4 a = __ldg(g + 2 * c), b = __ldg(g + 2 * c + 1);
-      v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
-    } else {
-#pragma unroll
-      for (int e = 0; e < 8; ++e) v[e] = 0.f;
-    }
-    uint32_t h[4], l[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const __half h0 = __float2half_rn(v[2 * e]), h1 = __float2half_rn(v[2 * e + 1]);
-      const __half l0 = __float2half_rn(v[2 * e] - __half2float(h0)), l1 = __float2half_rn(v[2 * e + 1] - __half2float(h1));
-      h[e] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-      l[e] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
-      ss = fmaf(v[2 * e], v[2 * e], ss);
-      ss = fmaf(v[2 * e + 1], v[2 * e + 1], ss);
-    }
-    *reinterpret_cast<uint4*>(hi + (size_t)c * kPlane + (size_t)r * 16) = make_uint4(h[0], h[1], h[2], h[3]);
-    *reinterpret_cast<uint4*>(lo + (size_t)c * kPlane + (size_t)r * 16) = make_uint4(l[0], l[1], l[2], l[3]);
-  }
-  return ss;
-}
 
 __global__ void __launch_bounds__(128, 1) nn_match_tc_kernel(const MatchParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];   // A hi, A lo, B hi, B lo: 4 x 16 KB
@@ -225,10 +190,6 @@ __global__ void __launch_bounds__(128, 1) nn_match_tc_kernel(const MatchParams p
   const int nq = p.nq[b], nt = p.nt[b];
   if (q0 >= nq || t0 >= nt) return;   // uniform per CTA
   const int warp = threadIdx.x >> 5;
-  uint8_t* a_hi = smem;
-  uint8_t* a_lo = smem + kOpBytes;
-  uint8_t* b_hi = smem + 2 * kOpBytes;
-  uint8_t* b_lo = smem + 3 * kOpBytes;
   if (threadIdx.x == 0) {
     mbar_init(&bar, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -243,34 +204,9 @@ __global__ void __launch_bounds__(128, 1) nn_match_tc_kernel(const MatchParams p
   const uint32_t tmem_base = tmem_base_s;
   const float* qb = p.q + (size_t)b * p.qcap * p.C;
   const float* tb = p.t + (size_t)b * p.tcap * p.C;
-  // instruction descriptor: fp16 x fp16 -> fp32, M = 128, N = 128, both operands K-major
-  const uint32_t idesc = (1u << 4) | ((uint32_t)(kNT >> 3) << 17) | ((uint32_t)(kMT >> 4) << 24);
-  const uint32_t d_hi = (128u >> 4) | (1u << 14);                    // SBO: 8 rows x 16 B
-  const uint32_t lbo = ((uint32_t)kPlane >> 4) << 16;               // LBO: next 8-element K chunk
-  float na = 0.f, nb = 0.f;
+  float na, nb;
   uint32_t phase = 0;
-  for (int k0 = 0; k0 < p.C; k0 += kKC) {
-    na += stage_operand(qb, nq, p.C, q0, k0, a_hi, a_lo);
-    nb += stage_operand(tb, nt, p.C, t0, k0, b_hi, b_lo);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");    // generic-proxy stores -> tensor-core reads
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      tc_fence_after();
-#pragma unroll
-      for (int kk = 0; kk < kKC / 16; ++kk) {
-        const uint32_t off = ((uint32_t)kk * 2 * kPlane) >> 4;
-        const uint32_t ah = ((smem_u32(a_hi) >> 4) + off) | lbo, al = ((smem_u32(a_lo) >> 4) + off) | lbo;
-        const uint32_t bh = ((smem_u32(b_hi) >> 4) + off) | lbo, bl = ((smem_u32(b_lo) >> 4) + off) | lbo;
-        umma_f16_2w(tmem_base, ah, d_hi, bh, d_hi, idesc, (k0 | kk) ? 1u : 0u);   // hi . hi
-        umma_f16_2w(tmem_base, ah, d_hi, bl, d_hi, idesc, 1u);                    // hi . lo
-        umma_f16_2w(tmem_base, al, d_hi, bh, d_hi, idesc, 1u);                    // lo . hi
-      }
-      umma_commit(&bar);
-    }
-    mbar_wait(&bar, phase);   // the MMAs have read this step's operands: the buffers may be refilled
-    phase ^= 1;
-  }
-  tc_fence_after();
+  dot_tile(qb, nq, q0, tb, nt, t0, p.C, smem, &bar, phase, tmem_base, na, nb);
   nb_s[threadIdx.x] = nb;
   __syncthreads();
   // epilogue: thread = query row = TMEM lane; arg-min of |a|^2 + |b|^2 - 2 a.b over this CTA's 128 train rows
@@ -284,7 +220,7 @@ __global__ void __launch_bounds__(128, 1) nn_match_tc_kernel(const MatchParams p
 #pragma unroll
     for (int c = 0; c < 32; ++c) {
       const int j = t0 + c0 + c;
-      const float d2 = fmaxf(fmaf(-2.0f, __uint_as_float(v[c]), na + nb_s[c0 + c]), 0.f);
+      const float d2 = dist2(v[c], na, nb_s[c0 + c]);
       if (j < nt && d2 < best) { best = d2; best_j = j; }
     }
   }
@@ -502,7 +438,7 @@ extern "C" int spn_mutual_nn_match(spn_ctx* ctx, const float* d_desc1, const int
   unsigned long long* bt = bq + n1;
   fill_u64_kernel<<<(unsigned)((n1 + n2 + 255) / 256), 256, 0, s>>>(bq, n1 + n2, ~0ull);
   SPN_CHECK_LAUNCH(ctx);
-  const size_t dyn = 4 * (size_t)kOpBytes + 1024;
+  const size_t dyn = kSmemBytes;
   SPN_CUDA(cudaFuncSetAttribute(nn_match_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
   MatchParams p;
   p.q = d_desc1; p.t = d_desc2; p.nq = d_n1; p.nt = d_n2; p.qcap = cap1; p.tcap = cap2; p.C = C; p.best = bq;

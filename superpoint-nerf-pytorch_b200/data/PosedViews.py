@@ -45,6 +45,17 @@ def _matrix(value, shape, where):
     return m.reshape(shape).astype(np.float32)
 
 
+def read_image(path):
+    """-> (H, W) uint8 grayscale (colour images are converted); ValueError naming the file if it cannot be decoded."""
+    import cv2
+    img = cv2.imread(str(path), cv2.IMREAD_GRAYSCALE)
+    if img is None:
+        raise ValueError(f"{path}: cannot be decoded as an image")
+    if img.dtype != np.uint8:
+        raise ValueError(f"{path}: expected 8-bit samples, got {img.dtype}")
+    return img
+
+
 class PosedViews(Dataset):
     def __init__(self, data_config, task="training", device="cuda") -> None:
         super().__init__()
@@ -111,20 +122,11 @@ class PosedViews(Dataset):
     def __len__(self):
         return len(self.items)
 
-    def _read_image(self, path):
-        import cv2
-        img = cv2.imread(str(path), cv2.IMREAD_GRAYSCALE)
-        if img is None:
-            raise ValueError(f"{path}: cannot be decoded as an image")
-        if img.dtype != np.uint8:
-            raise ValueError(f"{path}: expected 8-bit samples, got {img.dtype}")
-        return img
-
     def __getitem__(self, index):
         """Host only (thread-safe): decode and check one chunk -> the item dictionary (CPU tensors)."""
         images, depths, shape = [], [], None
         for fr in self.items[index]:
-            img = self._read_image(fr["image"])
+            img = read_image(fr["image"])
             H, W = img.shape
             if H % 8 or W % 8:
                 raise ValueError(f"{fr['image']}: size {H}x{W} is not a multiple of 8")

@@ -36,11 +36,9 @@ the frame names) and ``summary.json``; the same inputs give byte-identical files
 from __future__ import annotations
 
 import concurrent.futures as cf
-import io
 import json
 import math
 import os
-import zipfile
 from pathlib import Path
 from typing import Literal
 
@@ -48,6 +46,7 @@ import numpy as np
 import torch
 
 from .. import settings
+from ..utils.npz import write_npz as _write_npz
 
 AUC_THRESHOLDS = (5.0, 10.0, 20.0)
 MATCH_GROUP = 64          # pairs per mutual_nn_match call: bounds the gathered descriptors to 2 x 64 x max_kp x 256 fp32
@@ -257,15 +256,6 @@ def summarize(per_pair, sp, pose, ev, model_name):
     else:
         s["note"] = "pose not evaluated (evaluation.pose: false)"
     return s
-
-
-def _write_npz(path, arrays):
-    """np.savez without the zip members' wall-clock timestamps, so that equal arrays give equal bytes."""
-    with zipfile.ZipFile(path, "w", zipfile.ZIP_STORED) as z:
-        for k in sorted(arrays):
-            buf = io.BytesIO()
-            np.lib.format.write_array(buf, np.asanyarray(arrays[k]), allow_pickle=False)
-            z.writestr(zipfile.ZipInfo(f"{k}.npy", date_time=(1980, 1, 1, 0, 0, 0)), buf.getvalue())
 
 
 def evaluate_posed_views(config, model, loader, split="training", workers=None):
