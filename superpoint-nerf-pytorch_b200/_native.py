@@ -1,4 +1,4 @@
-"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h, include/spn_posed.h and include/spn_match.h.  PyTorch is used only for device memory and streams."""
+"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h, include/spn_posed.h, include/spn_match.h and include/spn_retrieval.h.  PyTorch is used only for device memory and streams."""
 from __future__ import annotations
 
 import ctypes as C
@@ -87,6 +87,11 @@ POSED_PROTOTYPES = {
 MATCH_PROTOTYPES = {
     "spn_match_pairs": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _i, _i, _f, _f, _vp, _vp, _vp]),
 }
+# name -> (restype, argtypes); must list every symbol include/spn_retrieval.h declares
+RETRIEVAL_PROTOTYPES = {
+    "spn_knn": (_i, [_vp, _vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "spn_residual_sums": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
+}
 JPEG_OK, JPEG_UNSUPPORTED, JPEG_MALFORMED = 0, 1, 2
 JPEG_INFO_FIELDS = 5
 
@@ -115,7 +120,8 @@ def load_library():
                     raise NativeError(f"{_LIB_PATH} not found and building it failed ({e}); build it with "
                                       "`python superpoint-nerf-pytorch_b200/build.py` (there is no CPU/PyTorch fallback)")
             lib = C.CDLL(str(_LIB_PATH))
-            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES | POSED_PROTOTYPES | MATCH_PROTOTYPES).items():
+            for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES | POSED_PROTOTYPES | MATCH_PROTOTYPES |
+                                       RETRIEVAL_PROTOTYPES).items():
                 fn = getattr(lib, name)
                 fn.restype, fn.argtypes = res, args
             _lib = lib
@@ -594,6 +600,43 @@ class Context:
                    int(bool(mutual)), C.c_float(ratio), C.c_float(max_dist), _ptr(match) if P else None, _ptr(dist) if P else None,
                    self._s())
         return match, dist
+
+    def knn(self, query, train, k, exclude_self=False):
+        """The k nearest train rows of every query row (spn_knn, include/spn_retrieval.h): query (nq,C) and train (nt,C)
+        fp32 CUDA.  -> (index (nq,k) int32, ascending distance, -1 in slots past the usable train rows; dist2 (nq,k)
+        fp32, +inf there).  exclude_self: query and train are the same set and row i is not its own neighbour."""
+        query, train = _dense(query), _dense(train)
+        _chk_dev(query, torch.float32, "query", self.device)
+        _chk_dev(train, torch.float32, "train", self.device)
+        if query.dim() != 2 or train.dim() != 2 or query.shape[1] != train.shape[1]:
+            raise NativeError(f"knn: query {tuple(query.shape)} and train {tuple(train.shape)} must be (n, C) with the same C")
+        nq, Cc = query.shape
+        nt = train.shape[0]
+        index = torch.empty((nq, k), dtype=torch.int32, device=query.device)
+        dist2 = torch.empty((nq, k), dtype=torch.float32, device=query.device)
+        self._call("spn_knn", self.handle, _ptr(query) if nq else None, nq, _ptr(train) if nt else None, nt, Cc, int(k),
+                   int(bool(exclude_self)), _ptr(index) if nq else None, _ptr(dist2) if nq else None, self._s())
+        return index, dist2
+
+    def residual_sums(self, desc, count, assign, words):
+        """Per-image, per-word residual sums (spn_residual_sums, include/spn_retrieval.h): desc (N,cap,C) fp32 and count
+        (N,) int32 (detect_describe's desc_sparse / kp_count), assign (N,cap) int32 word per row, words (K,C) fp32, all
+        CUDA.  -> (sums (N,K,C) fp32: sum of x_i - c_w over the rows assigned to w, in row order; n (N,K) int32)."""
+        desc, count, assign, words = _dense(desc), _dense(count), _dense(assign), _dense(words)
+        for x, dt, name in ((desc, torch.float32, "desc"), (count, torch.int32, "count"), (assign, torch.int32, "assign"),
+                            (words, torch.float32, "words")):
+            _chk_dev(x, dt, name, self.device)
+        if desc.dim() != 3 or tuple(count.shape) != (desc.shape[0],) or tuple(assign.shape) != tuple(desc.shape[:2]) or \
+                words.dim() != 2 or words.shape[1] != desc.shape[2]:
+            raise NativeError(f"residual_sums: desc {tuple(desc.shape)} (N,cap,C), count {tuple(count.shape)} (N,), assign "
+                              f"{tuple(assign.shape)} (N,cap) and words {tuple(words.shape)} (K,C) do not fit together")
+        N, cap, Cc = desc.shape
+        K = words.shape[0]
+        sums = torch.empty((N, K, Cc), dtype=torch.float32, device=desc.device)
+        n = torch.empty((N, K), dtype=torch.int32, device=desc.device)
+        self._call("spn_residual_sums", self.handle, *[_ptr(x) if N else None for x in (desc, count, assign, words)], N, cap, Cc, K,
+                   _ptr(sums) if N else None, _ptr(n) if N else None, self._s())
+        return sums, n
 
     def resize_crop(self, src: torch.Tensor, new_h, new_w, crop_top, crop_left, H, W, divisor=255.0):
         """src (H0,W0) uint8 or fp32 CUDA -> (H,W) fp32: bilinear resize + centre crop + /divisor (loader pre-processing)."""

@@ -5,14 +5,22 @@
 The images are the ``data/ImageFolder.py`` listing of ``<DATA_PATH>/<data.name>/``.  Per run, in one process:
   1. one ``model(x, keypoints=True)`` per group of at most ``data.batch_size`` images of the same network input size;
      keypoints, counts and sparse descriptors are copied into one pool on the device ([N][top_k][256]);
-  2. ``spn_match_pairs`` calls over the pool (include/spn_match.h), at most ``Context.MATCH_MAX_PAIRS`` pairs each:
+  2. with ``pairs: retrieval`` only: the pair list from image retrieval (``retrieval.py``): a k-means vocabulary of the
+     pool (or the ``words`` of an earlier run's ``retrieval.npz``), VLAD vectors and each image's nearest images;
+  3. ``spn_match_pairs`` calls over the pool (include/spn_match.h), at most ``Context.MATCH_MAX_PAIRS`` pairs each:
      nearest neighbour of every keypoint of a among the keypoints of b, filtered by the ``matching`` block's mutual
      check, ratio test and distance threshold;
-  3. the kept matches compacted in (pair, keypoint of a) order on the device and one copy to the host.
+  4. the kept matches compacted in (pair, keypoint of a) order on the device and one copy to the host.
 
 ``matching`` keys: ``pairs`` (``exhaustive``: every i < j; ``sequential``: 0 < j - i <= ``window``; ``file``: the
-``pairs_file``, one ``name_a name_b`` per line, blank lines and lines starting with ``#`` skipped), ``mutual`` (bool),
+``pairs_file``, one ``name_a name_b`` per line, blank lines and lines starting with ``#`` skipped; ``retrieval``: each
+image with its ``retrieval.num_neighbors`` nearest images by VLAD), ``mutual`` (bool),
 ``ratio`` (0 = off, else in (0, 1]: keep iff d1 < ratio d2) and ``max_dist`` (keep iff d1 <= max_dist; ``.inf`` = off).
+
+``retrieval`` keys (a top-level block, read only with ``pairs: retrieval``): ``num_neighbors`` (1..128, default 20),
+``vocab_size`` (1..256 words, default 64), ``kmeans_iters`` (>= 1, default 20) and ``vocabulary`` (the path of an
+earlier run's ``retrieval.npz``, whose words are reused instead of running k-means; exclusive with the two k-means
+keys).
 
 Outputs, under ``<EXPER_PATH>/matches/<data.experiment_name>/``; the same inputs give byte-identical files:
   features.npz   names (N,), shapes (N,2) decoded (H, W), resize_geometry (N,4) (new_h, new_w, crop_top, crop_left;
@@ -20,6 +28,8 @@ Outputs, under ``<EXPER_PATH>/matches/<data.experiment_name>/``; the same inputs
                  the network's input size: image n's keypoints are keypoints[offsets[n]:offsets[n+1]]
   matches.npz    pairs (P,2) int32 image indices, offsets (P+1,) int64, matches (M,2) int32 (keypoint of a, keypoint
                  of b), distances (M,) fp32 and the settings mutual, ratio, max_dist
+  retrieval.npz  (``pairs: retrieval`` only) words (K,256) fp32, neighbors (N,k) int32 (-1: none), dist2 (N,k) fp32
+                 squared VLAD distances, num_neighbors and kmeans_iters (-1 when the vocabulary was loaded)
 """
 from __future__ import annotations
 
@@ -31,12 +41,13 @@ from pathlib import Path
 import numpy as np
 import torch
 
-from . import settings
+from . import retrieval, settings
 from ._native import Context
 from .utils.npz import write_npz
 
-PAIR_MODES = ("exhaustive", "sequential", "file")
+PAIR_MODES = ("exhaustive", "sequential", "file", "retrieval")
 MATCH_DEFAULTS = {"pairs": "exhaustive", "window": None, "pairs_file": None, "mutual": True, "ratio": 0.0, "max_dist": math.inf}
+RETRIEVAL_DEFAULTS = {"num_neighbors": 20, "vocab_size": 64, "kmeans_iters": 20, "vocabulary": None}
 
 
 def match_config(config) -> dict:
@@ -86,6 +97,50 @@ def match_config(config) -> dict:
     return m
 
 
+def retrieval_config(config) -> dict:
+    """The top-level ``retrieval`` block with defaults filled in (consulted with ``matching.pairs: retrieval`` only).
+    Unknown or out-of-range keys raise ValueError naming the key; the vocabulary file is checked by load_vocabulary."""
+    block = config.get("retrieval") or {}
+    if not isinstance(block, dict):
+        raise ValueError(f"retrieval: expected a mapping, got {block!r}")
+    for k in block:
+        if k not in RETRIEVAL_DEFAULTS:
+            raise ValueError(f"retrieval.{k}: unknown key (known: {', '.join(RETRIEVAL_DEFAULTS)})")
+    r = dict(RETRIEVAL_DEFAULTS, **block)
+    for k, lo, hi in (("num_neighbors", 1, 128), ("vocab_size", 1, 256), ("kmeans_iters", 1, None)):
+        v = r[k]
+        if isinstance(v, bool) or not isinstance(v, int) or v < lo or (hi is not None and v > hi):
+            what = f"in [{lo}, {hi}]" if hi is not None else f">= {lo}"
+            raise ValueError(f"retrieval.{k}: must be an integer {what}, got {v!r}")
+    if r["vocabulary"] is not None:
+        if not isinstance(r["vocabulary"], str) or not r["vocabulary"]:
+            raise ValueError(f"retrieval.vocabulary: must be the path of a retrieval.npz, got {r['vocabulary']!r}")
+        both = [k for k in ("vocab_size", "kmeans_iters") if block.get(k) is not None]
+        if both:
+            raise ValueError(f"retrieval.vocabulary: a loaded vocabulary takes no retrieval.{both[0]} (it would be ignored)")
+    return r
+
+
+def load_vocabulary(path):
+    """The ``words`` of a retrieval.npz -> (K, 256) fp32 numpy array; ValueError naming ``retrieval.vocabulary`` and
+    the file unless it holds a finite (K, 256) fp32 array with 1 <= K <= 256."""
+    where = f"retrieval.vocabulary: {path}"
+    try:
+        with np.load(path, allow_pickle=False) as z:
+            members = {k: z[k] for k in z.files}
+    except Exception as e:
+        raise ValueError(f"{where}: cannot be read as an .npz file ({e})") from None
+    if "words" not in members:
+        raise ValueError(f"{where}: no 'words' array (members: {', '.join(members)})")
+    words = members["words"]
+    if words.dtype != np.float32 or words.ndim != 2 or words.shape[1] != 256 or not 1 <= words.shape[0] <= 256:
+        raise ValueError(f"{where}: words must be a (K, 256) float32 array with 1 <= K <= 256, got {words.dtype} "
+                         f"{words.shape}")
+    if not np.isfinite(words).all():
+        raise ValueError(f"{where}: words hold non-finite values")
+    return words
+
+
 def pair_list(names, mode, window=None, pairs_file=None):
     """Image index pairs (a, b) of ``names``: ``exhaustive`` every a < b in order, ``sequential`` 0 < b - a <= window,
     ``file`` the ``name_a name_b`` lines of pairs_file in file order."""
@@ -96,6 +151,8 @@ def pair_list(names, mode, window=None, pairs_file=None):
         if isinstance(window, bool) or not isinstance(window, int) or window < 1:
             raise ValueError(f"sequential pairs need an integer window >= 1, got {window!r}")
         return [(a, b) for a in range(n) for b in range(a + 1, min(n, a + window + 1))]
+    if mode == "retrieval":
+        raise ValueError("pair mode retrieval needs the descriptors: use retrieval.neighbors and retrieval.retrieval_pairs")
     if mode != "file":
         raise ValueError(f"pair mode must be one of {', '.join(PAIR_MODES)}, got {mode!r}")
     index = {name: i for i, name in enumerate(names)}
@@ -174,12 +231,26 @@ def extract_features(model, dataset, batch_size):
 
 def match_folder(config, model, dataset):
     """Extract and match every image of ``dataset`` (data.ImageFolder) with the ``matching`` block of ``config`` ->
-    summary dictionary; writes ``<EXPER_PATH>/matches/<data.experiment_name>/features.npz`` and ``matches.npz``."""
+    summary dictionary; writes ``<EXPER_PATH>/matches/<data.experiment_name>/features.npz`` and ``matches.npz`` (and
+    ``retrieval.npz`` with ``pairs: retrieval``)."""
     m = match_config(config)
+    r = retrieval_config(config) if m["pairs"] == "retrieval" else None
+    vocabulary = load_vocabulary(r["vocabulary"]) if r and r["vocabulary"] else None
     model = model.eval()
     items, kp, counts, desc = extract_features(model, dataset, int(config["data"].get("batch_size", 1)))
     names = [it["name"] for it in items]
-    pairs = pair_list(names, m["pairs"], m["window"], m["pairs_file"])
+    if r:
+        if vocabulary is not None:
+            words = torch.from_numpy(vocabulary).to(desc.device)
+        else:
+            words = retrieval.kmeans(desc, counts, r["vocab_size"], r["kmeans_iters"])
+        index, dist2 = retrieval.neighbors(retrieval.vlad(desc, counts, words), counts, r["num_neighbors"])
+        pairs = retrieval.retrieval_pairs(index)
+        found = {"words": words.cpu().numpy(), "neighbors": index.cpu().numpy(), "dist2": dist2.cpu().numpy(),
+                 "num_neighbors": np.array(r["num_neighbors"]),
+                 "kmeans_iters": np.array(-1 if vocabulary is not None else r["kmeans_iters"])}
+    else:
+        pairs = pair_list(names, m["pairs"], m["window"], m["pairs_file"])
     offsets, matches, distances = match_pairs(desc, counts, pairs, m["mutual"], m["ratio"], m["max_dist"])
     cap, N, P, M = kp.shape[1], len(items), len(pairs), len(matches)
     valid = torch.arange(cap, device=kp.device)[None] < counts[:, None].clamp(0, cap)
@@ -201,8 +272,12 @@ def match_folder(config, model, dataset):
     out_dir.mkdir(parents=True, exist_ok=True)
     write_npz(out_dir / "features.npz", features)
     write_npz(out_dir / "matches.npz", result)
-    return {"n_images": N, "n_keypoints": int(cnt.sum()), "n_pairs": P, "n_matches": M, "output": str(out_dir),
-            **{k: m[k] for k in ("pairs", "mutual", "ratio", "max_dist")}}
+    summary = {"n_images": N, "n_keypoints": int(cnt.sum()), "n_pairs": P, "n_matches": M, "output": str(out_dir),
+               **{k: m[k] for k in ("pairs", "mutual", "ratio", "max_dist")}}
+    if r:
+        write_npz(out_dir / "retrieval.npz", found)
+        summary["n_retrieval_pairs"] = P
+    return summary
 
 
 def main(config_path: str, random_init: bool = False) -> None:
@@ -217,7 +292,8 @@ def main(config_path: str, random_init: bool = False) -> None:
         raise SystemExit("matching runs as a single process: run it without torchrun (WORLD_SIZE > 1)")
     with open(config_path, "r") as f:
         config = yaml.safe_load(f)
-    match_config(config)
+    if match_config(config)["pairs"] == "retrieval":
+        retrieval_config(config)
     if not torch.cuda.is_available():
         raise SystemExit("CUDA is not available: this implementation has no CPU fallback")
     from .data.ImageFolder import ImageFolder
