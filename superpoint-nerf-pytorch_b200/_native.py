@@ -1,4 +1,4 @@
-"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h, include/spn_posed.h, include/spn_match.h and include/spn_retrieval.h.  PyTorch is used only for device memory and streams."""
+"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h, include/spn_posed.h, include/spn_match.h, include/spn_retrieval.h and include/spn_verify.h.  PyTorch is used only for device memory and streams."""
 from __future__ import annotations
 
 import ctypes as C
@@ -92,6 +92,11 @@ RETRIEVAL_PROTOTYPES = {
     "spn_knn": (_i, [_vp, _vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "spn_residual_sums": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
 }
+# name -> (restype, argtypes); must list every symbol include/spn_verify.h declares
+VERIFY_PROTOTYPES = {
+    "spn_verify_pairs": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _vp, C.c_int64, _i, C.c_double, C.c_double, _i, C.c_uint64, _vp, _vp,
+                              _vp, _vp, _vp, _vp]),
+}
 JPEG_OK, JPEG_UNSUPPORTED, JPEG_MALFORMED = 0, 1, 2
 JPEG_INFO_FIELDS = 5
 
@@ -121,7 +126,7 @@ def load_library():
                                       "`python superpoint-nerf-pytorch_b200/build.py` (there is no CPU/PyTorch fallback)")
             lib = C.CDLL(str(_LIB_PATH))
             for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES | POSED_PROTOTYPES | MATCH_PROTOTYPES |
-                                       RETRIEVAL_PROTOTYPES).items():
+                                       RETRIEVAL_PROTOTYPES | VERIFY_PROTOTYPES).items():
                 fn = getattr(lib, name)
                 fn.restype, fn.argtypes = res, args
             _lib = lib
@@ -600,6 +605,47 @@ class Context:
                    int(bool(mutual)), C.c_float(ratio), C.c_float(max_dist), _ptr(match) if P else None, _ptr(dist) if P else None,
                    self._s())
         return match, dist
+
+    VERIFY_MAX_PAIRS = 65535
+    VERIFY_MODELS = {"fundamental": 0, "homography": 1}
+
+    def verify_pairs(self, kp, offsets, matches, pairs, model="fundamental", threshold=3.0, confidence=0.999, max_iters=10000,
+                     seed=0):
+        """RANSAC per pair (spn_verify_pairs, include/spn_verify.h): kp (N,cap,2) int32 (row, col) keypoint pool, offsets
+        (P+1,) int64 and matches (M,2) int32 CUDA (matching.match_pairs' output), pairs (P,2) host (a, b), at most
+        VERIFY_MAX_PAIRS; model 'fundamental' or 'homography'.  -> (models (P,3,3) fp64, num_inliers (P,) int32 (-1: the
+        pair's offsets or indices are out of range), hypotheses (P,) int32, best (P,) int32, inliers (M,) uint8); inlier
+        rows of pairs with out-of-range offsets stay 0."""
+        import numpy as np
+        if model not in self.VERIFY_MODELS:
+            raise NativeError(f"verify_pairs: model must be one of {', '.join(self.VERIFY_MODELS)}, got {model!r}")
+        kp, offsets, matches = _dense(kp), _dense(offsets), _dense(matches)
+        for x, dt, name in ((kp, torch.int32, "kp"), (offsets, torch.int64, "offsets"), (matches, torch.int32, "matches")):
+            _chk_dev(x, dt, name, self.device)
+        if kp.dim() != 3 or kp.shape[2] != 2 or matches.dim() != 2 or matches.shape[1] != 2 or offsets.dim() != 1:
+            raise NativeError(f"verify_pairs: kp {tuple(kp.shape)} must be (N,cap,2), matches {tuple(matches.shape)} (M,2) and "
+                              f"offsets {tuple(offsets.shape)} (P+1,)")
+        pr = np.asarray(pairs, dtype=np.int64)
+        if pr.size == 0:
+            pr = pr.reshape(0, 2)
+        if pr.ndim != 2 or pr.shape[1] != 2:
+            raise NativeError(f"verify_pairs: pairs must be (P, 2), got shape {pr.shape}")
+        if pr.size and (pr.min() < np.iinfo(np.int32).min or pr.max() > np.iinfo(np.int32).max):
+            raise NativeError("verify_pairs: a pair index does not fit int32")
+        pr = np.ascontiguousarray(pr.astype(np.int32))
+        P, M = len(pr), int(matches.shape[0])
+        if offsets.shape[0] != P + 1:
+            raise NativeError(f"verify_pairs: {P} pairs need {P + 1} offsets, got {offsets.shape[0]}")
+        N, cap, _ = kp.shape
+        dev = kp.device
+        models = torch.zeros((P, 3, 3), dtype=torch.float64, device=dev)
+        num, hyp, best = (torch.zeros((P,), dtype=torch.int32, device=dev) for _ in range(3))
+        inliers = torch.zeros((M,), dtype=torch.uint8, device=dev)
+        self._call("spn_verify_pairs", self.handle, _ptr(kp), N, cap, C.c_void_p(pr.ctypes.data) if P else None, P, _ptr(offsets),
+                   _ptr(matches) if M else None, M, self.VERIFY_MODELS[model], C.c_double(threshold), C.c_double(confidence),
+                   int(max_iters), C.c_uint64(seed), *[_ptr(x) if P else None for x in (models, num, hyp, best)],
+                   _ptr(inliers) if M else None, self._s())
+        return models, num, hyp, best, inliers
 
     def knn(self, query, train, k, exclude_self=False):
         """The k nearest train rows of every query row (spn_knn, include/spn_retrieval.h): query (nq,C) and train (nt,C)

@@ -1,4 +1,4 @@
-"""Build libspn_b200.so (the C-ABI library of include/spn_b200.h, spn_jpeg.h, spn_nerf.h, spn_posed.h, spn_match.h and spn_retrieval.h) in-tree with nvcc for sm_100a.
+"""Build libspn_b200.so (the C-ABI library of include/spn_b200.h, spn_jpeg.h, spn_nerf.h, spn_posed.h, spn_match.h, spn_retrieval.h and spn_verify.h) in-tree with nvcc for sm_100a.
 
     python superpoint-nerf-pytorch_b200/build.py [--force]
 
@@ -13,7 +13,7 @@ from pathlib import Path
 HERE = Path(__file__).resolve().parent
 CSRC = HERE / "csrc"
 SO = HERE / "libspn_b200.so"
-SOURCES = ["spn_api.cu", "conv_fp32.cu", "conv_tc.cu", "conv_fold.cu", "conv_split.cu", "front_tc.cu", "head_tc.cu", "geometry.cu", "nms.cu", "desc.cu", "eval.cu", "labels.cu", "jpeg.cu", "match.cu", "retrieval.cu"]
+SOURCES = ["spn_api.cu", "conv_fp32.cu", "conv_tc.cu", "conv_fold.cu", "conv_split.cu", "front_tc.cu", "head_tc.cu", "geometry.cu", "nms.cu", "desc.cu", "eval.cu", "labels.cu", "jpeg.cu", "match.cu", "retrieval.cu", "verify.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 
@@ -27,7 +27,8 @@ def needs_build() -> bool:
                                                                 HERE.parent / "include" / "spn_nerf.h",
                                                                 HERE.parent / "include" / "spn_posed.h",
                                                                 HERE.parent / "include" / "spn_match.h",
-                                                                HERE.parent / "include" / "spn_retrieval.h", Path(__file__)]
+                                                                HERE.parent / "include" / "spn_retrieval.h",
+                                                                HERE.parent / "include" / "spn_verify.h", Path(__file__)]
     return any(d.stat().st_mtime > t for d in deps)
 
 

@@ -358,13 +358,6 @@ ha_aggregate_kernel(const float* __restrict__ probs, const float* __restrict__ h
 
 // ---------------- device homography sampler (homographic_augmentation.py:21-106) ----------------
 
-__device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
-  x += 0x9E3779B97F4A7C15ull;
-  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-  return x ^ (x >> 31);
-}
-
 struct Rng {
   uint64_t key, ctr;
   __device__ double uniform() {  // (0,1)

@@ -197,3 +197,12 @@ int spn_tc_conv_layer(spn_ctx* ctx, int layer, int mode, const float* d_in, int 
                       float* d_out, cudaStream_t s);
 
 static inline int spn_cdiv(int a, int b) { return (a + b - 1) / b; }
+
+// SplitMix64 finaliser (Steele, Lea & Flood 2014): the counter-based random streams of the homography sampler
+// (geometry.cu) and of the RANSAC minimal samples (verify.cu).
+__device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
+  x += 0x9E3779B97F4A7C15ull;
+  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+  return x ^ (x >> 31);
+}

@@ -10,7 +10,8 @@ The images are the ``data/ImageFolder.py`` listing of ``<DATA_PATH>/<data.name>/
   3. ``spn_match_pairs`` calls over the pool (include/spn_match.h), at most ``Context.MATCH_MAX_PAIRS`` pairs each:
      nearest neighbour of every keypoint of a among the keypoints of b, filtered by the ``matching`` block's mutual
      check, ratio test and distance threshold;
-  4. the kept matches compacted in (pair, keypoint of a) order on the device and one copy to the host.
+  4. the kept matches compacted in (pair, keypoint of a) order on the device and one copy to the host;
+  5. with a ``verification`` block only: RANSAC per pair over those matches (``verify.verify_pairs``).
 
 ``matching`` keys: ``pairs`` (``exhaustive``: every i < j; ``sequential``: 0 < j - i <= ``window``; ``file``: the
 ``pairs_file``, one ``name_a name_b`` per line, blank lines and lines starting with ``#`` skipped; ``retrieval``: each
@@ -22,6 +23,14 @@ image with its ``retrieval.num_neighbors`` nearest images by VLAD), ``mutual`` (
 earlier run's ``retrieval.npz``, whose words are reused instead of running k-means; exclusive with the two k-means
 keys).
 
+``verification`` keys (an optional top-level block; without it nothing is verified and geometry.npz is not written):
+``model`` (required: ``fundamental``, 7-point RANSAC with the Sampson error, or ``homography``, 4-point RANSAC with the
+forward transfer error), ``threshold`` (pixels > 0, default 3.0), ``confidence`` (in (0, 1), default 0.999),
+``max_iters`` (1..16777216, default 10000), ``min_inliers`` (>= 0, default 15: a pair is verified iff its model has at
+least this many inliers) and ``seed`` (integer >= 0, default 0).  With the block, step 5 runs ``verify.verify_pairs``
+(include/spn_verify.h) on the matches of step 4; features.npz, matches.npz and retrieval.npz are the same bytes as
+without it.
+
 Outputs, under ``<EXPER_PATH>/matches/<data.experiment_name>/``; the same inputs give byte-identical files:
   features.npz   names (N,), shapes (N,2) decoded (H, W), resize_geometry (N,4) (new_h, new_w, crop_top, crop_left;
                  with ``data.preprocessing.resize`` only), offsets (N+1,) int64 and keypoints (K,2) int32 (row, col) at
@@ -30,6 +39,11 @@ Outputs, under ``<EXPER_PATH>/matches/<data.experiment_name>/``; the same inputs
                  of b), distances (M,) fp32 and the settings mutual, ratio, max_dist
   retrieval.npz  (``pairs: retrieval`` only) words (K,256) fp32, neighbors (N,k) int32 (-1: none), dist2 (N,k) fp32
                  squared VLAD distances, num_neighbors and kmeans_iters (-1 when the vocabulary was loaded)
+  geometry.npz   (with a ``verification`` block only) pairs (P,2) int32, models (P,3,3) fp64 (F: x_b^T F x_a = 0,
+                 ||F|| = 1; H: x_b ~ H x_a, H[2][2] = 1; x = (col, row, 1); zeros without a model), num_inliers,
+                 hypotheses and best (P,) int32, inliers (M,) bool row-aligned with matches.npz, verified (P,) bool
+                 (num_inliers >= min_inliers) and the settings model, threshold, confidence, max_iters, min_inliers,
+                 seed
 """
 from __future__ import annotations
 
@@ -41,13 +55,15 @@ from pathlib import Path
 import numpy as np
 import torch
 
-from . import retrieval, settings
+from . import retrieval, settings, verify
 from ._native import Context
 from .utils.npz import write_npz
 
 PAIR_MODES = ("exhaustive", "sequential", "file", "retrieval")
 MATCH_DEFAULTS = {"pairs": "exhaustive", "window": None, "pairs_file": None, "mutual": True, "ratio": 0.0, "max_dist": math.inf}
 RETRIEVAL_DEFAULTS = {"num_neighbors": 20, "vocab_size": 64, "kmeans_iters": 20, "vocabulary": None}
+VERIFY_MODELS = ("fundamental", "homography")
+VERIFY_DEFAULTS = {"model": None, "threshold": 3.0, "confidence": 0.999, "max_iters": 10000, "min_inliers": 15, "seed": 0}
 
 
 def match_config(config) -> dict:
@@ -119,6 +135,37 @@ def retrieval_config(config) -> dict:
         if both:
             raise ValueError(f"retrieval.vocabulary: a loaded vocabulary takes no retrieval.{both[0]} (it would be ignored)")
     return r
+
+
+def verify_config(config):
+    """The top-level ``verification`` block with defaults filled in, or None when the config has none.  Unknown,
+    missing or out-of-range keys raise ValueError naming the key."""
+    block = config.get("verification")
+    if block is None:
+        return None
+    if not isinstance(block, dict):
+        raise ValueError(f"verification: expected a mapping, got {block!r}")
+    for k in block:
+        if k not in VERIFY_DEFAULTS:
+            raise ValueError(f"verification.{k}: unknown key (known: {', '.join(VERIFY_DEFAULTS)})")
+    v = dict(VERIFY_DEFAULTS, **block)
+    if v["model"] not in VERIFY_MODELS:
+        raise ValueError(f"verification.model: required, one of {', '.join(VERIFY_MODELS)}, got {v['model']!r}")
+
+    def number(k, ok, what):
+        x = v[k]
+        if isinstance(x, bool) or not isinstance(x, (int, float)) or math.isnan(x) or not ok(x):
+            raise ValueError(f"verification.{k}: must be {what}, got {x!r}")
+        return float(x)
+
+    v["threshold"] = number("threshold", lambda x: 0 < x < math.inf, "a number of pixels > 0")
+    v["confidence"] = number("confidence", lambda x: 0 < x < 1, "a number in (0, 1)")
+    for k, lo, hi in (("max_iters", 1, 1 << 24), ("min_inliers", 0, None), ("seed", 0, 2 ** 64 - 1)):
+        x = v[k]
+        if isinstance(x, bool) or not isinstance(x, int) or x < lo or (hi is not None and x > hi):
+            what = f"in [{lo}, {hi}]" if hi is not None else f">= {lo}"
+            raise ValueError(f"verification.{k}: must be an integer {what}, got {x!r}")
+    return v
 
 
 def load_vocabulary(path):
@@ -235,6 +282,7 @@ def match_folder(config, model, dataset):
     ``retrieval.npz`` with ``pairs: retrieval``)."""
     m = match_config(config)
     r = retrieval_config(config) if m["pairs"] == "retrieval" else None
+    v = verify_config(config)
     vocabulary = load_vocabulary(r["vocabulary"]) if r and r["vocabulary"] else None
     model = model.eval()
     items, kp, counts, desc = extract_features(model, dataset, int(config["data"].get("batch_size", 1)))
@@ -277,6 +325,17 @@ def match_folder(config, model, dataset):
     if r:
         write_npz(out_dir / "retrieval.npz", found)
         summary["n_retrieval_pairs"] = P
+    if v:
+        models, num, hyp, best, inliers = verify.verify_pairs(kp, offsets, matches, pairs, v["model"], v["threshold"],
+                                                              v["confidence"], v["max_iters"], v["seed"])
+        num, inliers = num.cpu().numpy(), inliers.cpu().numpy()
+        geometry = {"pairs": result["pairs"], "models": models.cpu().numpy(), "num_inliers": num,
+                    "hypotheses": hyp.cpu().numpy(), "best": best.cpu().numpy(), "inliers": inliers,
+                    "verified": num >= v["min_inliers"], **{k: np.array(v[k]) for k in VERIFY_DEFAULTS}}
+        geometry["seed"] = np.array(v["seed"], np.uint64)
+        write_npz(out_dir / "geometry.npz", geometry)
+        summary["n_verified_pairs"] = int(geometry["verified"].sum())
+        summary["n_inlier_matches"] = int(inliers[np.repeat(geometry["verified"], np.diff(result["offsets"]))].sum())
     return summary
 
 
@@ -294,6 +353,7 @@ def main(config_path: str, random_init: bool = False) -> None:
         config = yaml.safe_load(f)
     if match_config(config)["pairs"] == "retrieval":
         retrieval_config(config)
+    verify_config(config)
     if not torch.cuda.is_available():
         raise SystemExit("CUDA is not available: this implementation has no CPU fallback")
     from .data.ImageFolder import ImageFolder
