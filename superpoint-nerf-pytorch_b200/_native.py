@@ -1,4 +1,4 @@
-"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h, include/spn_posed.h, include/spn_match.h, include/spn_retrieval.h and include/spn_verify.h.  PyTorch is used only for device memory and streams."""
+"""ctypes binding of include/spn_b200.h, include/spn_jpeg.h, include/spn_nerf.h, include/spn_posed.h, include/spn_match.h, include/spn_retrieval.h, include/spn_verify.h and include/spn_tracks.h.  PyTorch is used only for device memory and streams."""
 from __future__ import annotations
 
 import ctypes as C
@@ -97,6 +97,11 @@ VERIFY_PROTOTYPES = {
     "spn_verify_pairs": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _vp, C.c_int64, _i, C.c_double, C.c_double, _i, C.c_uint64, _vp, _vp,
                               _vp, _vp, _vp, _vp]),
 }
+# name -> (restype, argtypes); must list every symbol include/spn_tracks.h declares
+TRACKS_PROTOTYPES = {
+    "spn_track_labels": (_i, [_vp, _vp, C.c_int64, C.c_int32, _i, _vp, _vp, _vp]),
+    "spn_track_table": (_i, [_vp, _vp, C.c_int32, _vp, C.c_int32, C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+}
 JPEG_OK, JPEG_UNSUPPORTED, JPEG_MALFORMED = 0, 1, 2
 JPEG_INFO_FIELDS = 5
 
@@ -126,7 +131,7 @@ def load_library():
                                       "`python superpoint-nerf-pytorch_b200/build.py` (there is no CPU/PyTorch fallback)")
             lib = C.CDLL(str(_LIB_PATH))
             for name, (res, args) in (PROTOTYPES | JPEG_PROTOTYPES | NERF_PROTOTYPES | POSED_PROTOTYPES | MATCH_PROTOTYPES |
-                                       RETRIEVAL_PROTOTYPES | VERIFY_PROTOTYPES).items():
+                                       RETRIEVAL_PROTOTYPES | VERIFY_PROTOTYPES | TRACKS_PROTOTYPES).items():
                 fn = getattr(lib, name)
                 fn.restype, fn.argtypes = res, args
             _lib = lib
@@ -646,6 +651,57 @@ class Context:
                    int(max_iters), C.c_uint64(seed), *[_ptr(x) if P else None for x in (models, num, hyp, best)],
                    _ptr(inliers) if M else None, self._s())
         return models, num, hyp, best, inliers
+
+    TRACKS_MAX_ROWS = 2 ** 31 - 1
+
+    def track_labels(self, edges, K, labels=None):
+        """Connected components of a match graph (spn_track_labels, include/spn_tracks.h): edges (E,2) int32 CUDA, rows
+        in [0, K).  -> (labels (K,) int32, the smallest row of every row's component; bad (1,) int64, the edges with an
+        endpoint outside [0, K), which are not applied).  ``labels``: the labels of an earlier call with the same K; the
+        edges are joined into its components in place, so an edge list split over several calls gives the labels of one
+        call."""
+        edges = _dense(edges)
+        _chk_dev(edges, torch.int32, "edges", self.device)
+        if edges.dim() != 2 or edges.shape[1] != 2:
+            raise NativeError(f"track_labels: edges must be (E, 2), got shape {tuple(edges.shape)}")
+        if isinstance(K, bool) or not 1 <= int(K) <= self.TRACKS_MAX_ROWS:
+            raise NativeError(f"track_labels: K = {K!r} rows outside [1, {self.TRACKS_MAX_ROWS}]")
+        K, E = int(K), int(edges.shape[0])
+        resume = labels is not None
+        if not resume:
+            labels = torch.empty((K,), dtype=torch.int32, device=edges.device)
+        else:
+            _chk_dev(labels, torch.int32, "labels", self.device)
+            if tuple(labels.shape) != (K,):
+                raise NativeError(f"track_labels: labels must be ({K},), got shape {tuple(labels.shape)}")
+        bad = torch.empty((1,), dtype=torch.int64, device=edges.device)
+        self._call("spn_track_labels", self.handle, _ptr(edges) if E else None, C.c_int64(E), K, int(resume), _ptr(labels),
+                   _ptr(bad), self._s())
+        return labels, bad
+
+    def track_table(self, labels, img_offsets, min_length=2):
+        """The track table of component labels (spn_track_table, include/spn_tracks.h): labels (K,) int32 (track_labels),
+        img_offsets (N+1,) int64 (image n's rows are img_offsets[n]:img_offsets[n+1]), both CUDA.  -> (track_offsets
+        (K//2+1,) int64, obs (K,2) int32 (image, keypoint), consistent (K//2,) uint8, track_of (K,) int32, totals (2,) int64
+        (T, O), bad (1,) int64), at their upper bounds: only the first T (+1) / O entries are written."""
+        labels, img_offsets = _dense(labels), _dense(img_offsets)
+        _chk_dev(labels, torch.int32, "labels", self.device)
+        _chk_dev(img_offsets, torch.int64, "img_offsets", self.device)
+        if labels.dim() != 1 or img_offsets.dim() != 1 or img_offsets.shape[0] < 2:
+            raise NativeError(f"track_table: labels {tuple(labels.shape)} must be (K,) and img_offsets "
+                              f"{tuple(img_offsets.shape)} (N+1,) with N >= 1")
+        K, N = int(labels.shape[0]), int(img_offsets.shape[0]) - 1
+        if not 1 <= K <= self.TRACKS_MAX_ROWS or N >= 2 ** 31 - 1:
+            raise NativeError(f"track_table: K = {K} rows outside [1, {self.TRACKS_MAX_ROWS}] or N = {N} images too many")
+        if isinstance(min_length, bool) or not isinstance(min_length, int) or min_length < 2:
+            raise NativeError(f"track_table: min_length must be an integer >= 2, got {min_length!r}")
+        dev = labels.device
+        out = (torch.empty((K // 2 + 1,), dtype=torch.int64, device=dev), torch.empty((K, 2), dtype=torch.int32, device=dev),
+               torch.empty((K // 2,), dtype=torch.uint8, device=dev), torch.empty((K,), dtype=torch.int32, device=dev),
+               torch.empty((2,), dtype=torch.int64, device=dev), torch.empty((1,), dtype=torch.int64, device=dev))
+        self._call("spn_track_table", self.handle, _ptr(labels), K, _ptr(img_offsets), N, min(min_length, 2 ** 31 - 1),
+                   *[_ptr(x) if x.numel() else None for x in out], self._s())
+        return out
 
     def knn(self, query, train, k, exclude_self=False):
         """The k nearest train rows of every query row (spn_knn, include/spn_retrieval.h): query (nq,C) and train (nt,C)

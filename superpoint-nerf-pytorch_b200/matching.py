@@ -11,7 +11,8 @@ The images are the ``data/ImageFolder.py`` listing of ``<DATA_PATH>/<data.name>/
      nearest neighbour of every keypoint of a among the keypoints of b, filtered by the ``matching`` block's mutual
      check, ratio test and distance threshold;
   4. the kept matches compacted in (pair, keypoint of a) order on the device and one copy to the host;
-  5. with a ``verification`` block only: RANSAC per pair over those matches (``verify.verify_pairs``).
+  5. with a ``verification`` block only: RANSAC per pair over those matches (``verify.verify_pairs``);
+  6. with a ``tracks`` block only: the tracks of the inlier matches of the verified pairs (``tracks.build_tracks``).
 
 ``matching`` keys: ``pairs`` (``exhaustive``: every i < j; ``sequential``: 0 < j - i <= ``window``; ``file``: the
 ``pairs_file``, one ``name_a name_b`` per line, blank lines and lines starting with ``#`` skipped; ``retrieval``: each
@@ -31,6 +32,11 @@ least this many inliers) and ``seed`` (integer >= 0, default 0).  With the block
 (include/spn_verify.h) on the matches of step 4; features.npz, matches.npz and retrieval.npz are the same bytes as
 without it.
 
+``tracks`` keys (an optional top-level block that needs a ``verification`` block; without it tracks.npz is not
+written): ``min_length`` (integer >= 2, default 2: a track has at least this many keypoints).  With the block, step 6
+runs ``tracks.build_tracks`` (include/spn_tracks.h) on the inliers of the verified pairs: a track is a connected
+component of the graph of those matches over all keypoints.  The other outputs are the same bytes as without it.
+
 Outputs, under ``<EXPER_PATH>/matches/<data.experiment_name>/``; the same inputs give byte-identical files:
   features.npz   names (N,), shapes (N,2) decoded (H, W), resize_geometry (N,4) (new_h, new_w, crop_top, crop_left;
                  with ``data.preprocessing.resize`` only), offsets (N+1,) int64 and keypoints (K,2) int32 (row, col) at
@@ -44,6 +50,11 @@ Outputs, under ``<EXPER_PATH>/matches/<data.experiment_name>/``; the same inputs
                  hypotheses and best (P,) int32, inliers (M,) bool row-aligned with matches.npz, verified (P,) bool
                  (num_inliers >= min_inliers) and the settings model, threshold, confidence, max_iters, min_inliers,
                  seed
+  tracks.npz     (with a ``tracks`` block only) offsets (T+1,) int64: track t's observations are
+                 observations[offsets[t]:offsets[t+1]], (image, keypoint) int32 pairs in image order, tracks ordered by
+                 their smallest row of features.npz's keypoints; consistent (T,) bool (no two observations in one
+                 image; inconsistent tracks are kept and flagged); track_of (K,) int32 row-aligned with features.npz's
+                 keypoints (-1: in no track); and the setting min_length
 """
 from __future__ import annotations
 
@@ -55,7 +66,7 @@ from pathlib import Path
 import numpy as np
 import torch
 
-from . import retrieval, settings, verify
+from . import retrieval, settings, tracks, verify
 from ._native import Context
 from .utils.npz import write_npz
 
@@ -64,6 +75,7 @@ MATCH_DEFAULTS = {"pairs": "exhaustive", "window": None, "pairs_file": None, "mu
 RETRIEVAL_DEFAULTS = {"num_neighbors": 20, "vocab_size": 64, "kmeans_iters": 20, "vocabulary": None}
 VERIFY_MODELS = ("fundamental", "homography")
 VERIFY_DEFAULTS = {"model": None, "threshold": 3.0, "confidence": 0.999, "max_iters": 10000, "min_inliers": 15, "seed": 0}
+TRACKS_DEFAULTS = {"min_length": 2}
 
 
 def match_config(config) -> dict:
@@ -166,6 +178,26 @@ def verify_config(config):
             what = f"in [{lo}, {hi}]" if hi is not None else f">= {lo}"
             raise ValueError(f"verification.{k}: must be an integer {what}, got {x!r}")
     return v
+
+
+def tracks_config(config):
+    """The top-level ``tracks`` block with defaults filled in, or None when the config has none.  Unknown or
+    out-of-range keys, and a block without a ``verification`` block, raise ValueError naming the key."""
+    block = config.get("tracks")
+    if block is None:
+        return None
+    if not isinstance(block, dict):
+        raise ValueError(f"tracks: expected a mapping, got {block!r}")
+    for k in block:
+        if k not in TRACKS_DEFAULTS:
+            raise ValueError(f"tracks.{k}: unknown key (known: {', '.join(TRACKS_DEFAULTS)})")
+    t = dict(TRACKS_DEFAULTS, **block)
+    x = t["min_length"]
+    if isinstance(x, bool) or not isinstance(x, int) or x < 2:
+        raise ValueError(f"tracks.min_length: must be an integer >= 2, got {x!r}")
+    if config.get("verification") is None:
+        raise ValueError("tracks: needs a verification block (tracks are built from the inliers of verified pairs)")
+    return t
 
 
 def load_vocabulary(path):
@@ -283,6 +315,7 @@ def match_folder(config, model, dataset):
     m = match_config(config)
     r = retrieval_config(config) if m["pairs"] == "retrieval" else None
     v = verify_config(config)
+    tr = tracks_config(config)
     vocabulary = load_vocabulary(r["vocabulary"]) if r and r["vocabulary"] else None
     model = model.eval()
     items, kp, counts, desc = extract_features(model, dataset, int(config["data"].get("batch_size", 1)))
@@ -328,6 +361,7 @@ def match_folder(config, model, dataset):
     if v:
         models, num, hyp, best, inliers = verify.verify_pairs(kp, offsets, matches, pairs, v["model"], v["threshold"],
                                                               v["confidence"], v["max_iters"], v["seed"])
+        inliers_d = inliers
         num, inliers = num.cpu().numpy(), inliers.cpu().numpy()
         geometry = {"pairs": result["pairs"], "models": models.cpu().numpy(), "num_inliers": num,
                     "hypotheses": hyp.cpu().numpy(), "best": best.cpu().numpy(), "inliers": inliers,
@@ -336,6 +370,18 @@ def match_folder(config, model, dataset):
         write_npz(out_dir / "geometry.npz", geometry)
         summary["n_verified_pairs"] = int(geometry["verified"].sum())
         summary["n_inlier_matches"] = int(inliers[np.repeat(geometry["verified"], np.diff(result["offsets"]))].sum())
+    if tr:
+        verified = torch.from_numpy(geometry["verified"]).to(inliers_d.device)
+        keep = inliers_d & torch.repeat_interleave(verified, offsets.diff(), output_size=M)
+        t_off, obs, consistent, track_of = (x.cpu().numpy() for x in tracks.build_tracks(
+            counts, pairs, offsets, matches, keep, tr["min_length"]))
+        write_npz(out_dir / "tracks.npz", {"offsets": t_off, "observations": obs, "consistent": consistent,
+                                            "track_of": track_of, "min_length": np.array(tr["min_length"])})
+        lengths = np.diff(t_off)
+        summary["n_tracks"] = len(consistent)
+        summary["n_consistent_tracks"] = int(consistent.sum())
+        summary["n_track_observations"] = len(obs)
+        summary["mean_track_length"] = float(lengths[consistent].mean()) if consistent.any() else 0.0
     return summary
 
 
@@ -354,6 +400,7 @@ def main(config_path: str, random_init: bool = False) -> None:
     if match_config(config)["pairs"] == "retrieval":
         retrieval_config(config)
     verify_config(config)
+    tracks_config(config)
     if not torch.cuda.is_available():
         raise SystemExit("CUDA is not available: this implementation has no CPU fallback")
     from .data.ImageFolder import ImageFolder
