@@ -54,7 +54,7 @@ __global__ void __launch_bounds__(128, 1) match_pairs_kernel(const PairParams p)
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(128));
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(tmem_cols(p.C)));
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
   }
   tc_fence_before();
@@ -109,7 +109,7 @@ __global__ void __launch_bounds__(128, 1) match_pairs_kernel(const PairParams p)
   __syncthreads();
   if (warp == 0) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(128));
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols(p.C)));
   }
 }
 

@@ -11,6 +11,7 @@ import torch
 
 from conftest import SP_MODEL, smooth_image
 from oracle import match_oracle as O
+from retrieval_scenes import unit as _unit
 
 pytestmark = pytest.mark.gpu
 
@@ -18,11 +19,6 @@ MARGIN = 1e-5      # decisions are compared where the oracle is at least this fa
 DIST_TOL = 1e-5    # the matcher tolerance of DESIGN.md section 4: on d^2 everywhere, and on d where d >= 0.5 (the
                    # square root divides the few-1e-6 error of d^2 by 2d: ~1e-3 near 0, 3e-5 at d = 0.06)
 FILTERS = list(itertools.product((False, True), (0.0, 0.8, 1.0), (math.inf, 1.1)))   # mutual x ratio x max_dist
-
-
-def _unit(shape, rng):
-    x = rng.randn(*shape).astype(np.float32)
-    return x / np.linalg.norm(x, axis=-1, keepdims=True)
 
 
 def _pool_random(N, cap, counts, seed, C=256):

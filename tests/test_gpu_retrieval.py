@@ -1,6 +1,8 @@
 """spn_knn, spn_residual_sums (include/spn_retrieval.h) and retrieval.py on the GPU: neighbours against the fp64 oracle
-(oracle/retrieval_oracle.py) at ragged sizes, the same d^2 bits as spn_match_pairs, bit-equal residual sums, k-means
-steps, retrieval quality on planted scenes, duplicate images, argument errors, guard bands and the CLI end to end."""
+(oracle/retrieval_oracle.py) at ragged sizes, at the VLAD widths of retrieval (D up to 65 536) on random rows, on
+near-duplicate ladders and on VLAD vectors of planted scenes, the same d^2 bits as spn_match_pairs and
+spn_mutual_nn_match at every width, bit-equal residual sums, k-means steps, retrieval quality on planted scenes,
+duplicate images, argument errors, guard bands and the CLI end to end."""
 import copy
 import math
 
@@ -10,6 +12,8 @@ import torch
 
 from conftest import SP_MODEL, smooth_image
 from oracle import retrieval_oracle as R
+from retrieval_scenes import planted_scenes as _planted_scenes
+from retrieval_scenes import unit as _unit
 
 pytestmark = pytest.mark.gpu
 
@@ -17,18 +21,22 @@ MARGIN = 1e-5      # orders are compared where the oracle is at least this far (
 DIST_TOL = 1e-5    # section 4, the matcher's rule); d^2 within this everywhere
 
 
-def _unit(shape, rng):
-    x = rng.randn(*shape).astype(np.float32)
-    return x / np.linalg.norm(x, axis=-1, keepdims=True)
-
-
 def _ctx():
     from superpoint_nerf_pytorch_b200 import _native
     return _native.get_context(0)
 
 
-def _check_knn(q, t, k, exclude_self, label):
-    idx, d2 = _ctx().knn(torch.from_numpy(q).cuda(), torch.from_numpy(t).cuda(), k, exclude_self)
+def _pair_d2(q, t, idx):
+    """fp64 d^2 of query row i and train row idx[i, s] (idx >= 0)."""
+    q, t = q.astype(np.float64), t.astype(np.float64)
+    d = (q * q).sum(1)[:, None] + (t * t).sum(1)[None, :] - 2.0 * (q @ t.T)
+    return np.maximum(d, 0.0)[np.arange(len(q))[:, None], np.maximum(idx, 0)]
+
+
+def _check_knn(q, t, k, exclude_self, label, got=None):
+    """spn_knn(q, t, k) (or `got` = its (index, dist2) from elsewhere) against the oracle.  -> (queries within the
+    margin, largest |d^2 - fp64 d^2 of the returned pair|)."""
+    idx, d2 = got if got is not None else _ctx().knn(torch.from_numpy(q).cuda(), torch.from_numpy(t).cuda(), k, exclude_self)
     idx, d2 = idx.cpu().numpy(), d2.cpu().numpy()
     w_idx, w_d2, margin = R.knn(q, t, k, exclude_self)
     pad = w_idx < 0
@@ -36,8 +44,10 @@ def _check_knn(q, t, k, exclude_self, label):
     sure = margin > MARGIN
     assert np.array_equal(idx[sure], w_idx[sure]), label
     assert np.abs(d2[~pad].astype(np.float64) - w_d2[~pad]).max(initial=0) <= DIST_TOL, label
+    err = np.abs(d2[~pad].astype(np.float64) - _pair_d2(q, t, idx)[~pad]).max(initial=0)
+    assert err <= DIST_TOL, label                                          # also right for the row it names
     assert (d2[:, 1:] >= d2[:, :-1]).all(), label                         # ascending; +inf >= +inf in the padding
-    return int((~sure).sum())
+    return int((~sure).sum()), float(err)
 
 
 def test_knn_against_the_oracle_at_ragged_sizes():
@@ -48,12 +58,12 @@ def test_knn_against_the_oracle_at_ragged_sizes():
         for nt in sizes:
             q, t = _unit((nq, 64), rng), _unit((nt, 64), rng)
             for k in (1, 2, 5, 128):
-                excluded += _check_knn(q, t, k, False, (nq, nt, k))
+                excluded += _check_knn(q, t, k, False, (nq, nt, k))[0]
         q = _unit((nq, 128), rng)
         for k in (1, 2, 5, 128):
-            excluded += _check_knn(q, q, k, True, (nq, "self", k))
+            excluded += _check_knn(q, q, k, True, (nq, "self", k))[0]
     q, t = _unit((300, 1024), rng), _unit((77, 1024), rng)             # k > nt, and a longer K loop
-    excluded += _check_knn(q, t, 100, False, "k > nt")
+    excluded += _check_knn(q, t, 100, False, "k > nt")[0]
     print(f"knn: {excluded} query rows within the {MARGIN:g} margin (not compared)")
 
 
@@ -68,6 +78,96 @@ def test_knn_planted_duplicates_and_empty_train():
     assert (idx == -1).all() and torch.isinf(d2).all()
     idx, d2 = _ctx().knn(torch.zeros((0, 256), device="cuda"), torch.from_numpy(t).cuda(), 4)
     assert idx.shape == (0, 4)
+
+
+def test_knn_against_the_oracle_at_vlad_widths():
+    """Random unit rows at the widths retrieval runs spn_knn on (D = vocab_size x 256), ragged nq / nt, k up to 128.
+    Random rows at large D have d^2 = 2 +- 2 / sqrt(D), so among a few hundred rows adjacent ranks are often closer
+    than the margin: for k > 1 most queries fall within it by construction of the input.  The d^2 bound holds on every
+    entry, and with k = 1 fewer than 1 % of the queries may fall within the margin."""
+    rng = np.random.RandomState(7)
+    first = first_total = 0
+    for D in (4096, 16384, 65536):
+        pool = _unit((512, D), rng)
+        excluded, total, worst = {}, {}, 0.0
+        for k in (1, 20, 128):
+            cases = [(pool[:nq], pool[-nt:], False, (D, nq, nt, k)) for nq, nt in ((1, 300), (127, 129), (129, 1), (300, 127))]
+            cases += [(pool[:n], pool[:n], True, (D, n, "self", k)) for n in (1, 129, 300)]
+            for q, t, self_, label in cases:
+                ex, err = _check_knn(q, t, k, self_, label)
+                excluded[k] = excluded.get(k, 0) + ex
+                total[k] = total.get(k, 0) + len(q)
+                worst = max(worst, err)
+        first, first_total = first + excluded[1], first_total + total[1]
+        print(f"knn D={D}: largest d^2 error {worst:.2e}; queries within the {MARGIN:g} margin (not compared) "
+              + ", ".join(f"k={k}: {excluded[k]} of {total[k]}" for k in excluded))
+    assert first < 0.01 * first_total, (first, first_total)
+
+
+def _ladder(D, nq, rng, rungs=40, copies=2, others=50):
+    """nq unit queries and a train set holding, per query, `copies` exact copies of it, rungs normalise(q + eps n) with
+    eps from 1e-4 to 1 (true d^2 ~1e-8 to ~0.6, n a random unit row) and `others` random unit rows.  -> q, t, the
+    train indices of the copies (nq, copies)."""
+    q = _unit((nq, D), rng)
+    eps = np.logspace(-4, 0, rungs)
+    blocks, copy_idx = [], []
+    for i in range(nq):
+        near = q[i] + eps[:, None].astype(np.float32) * _unit((rungs, D), rng)
+        near /= np.linalg.norm(near, axis=1, keepdims=True)
+        start = sum(len(b) for b in blocks)
+        copy_idx.append(start + np.arange(copies))
+        blocks.append(np.concatenate([np.repeat(q[i:i + 1], copies, 0), near, _unit((others, D), rng)]))
+    return q, np.concatenate(blocks).astype(np.float32), np.array(copy_idx)
+
+
+@pytest.mark.parametrize("D", [256, 1024, 4096, 16384, 65536])
+def test_knn_near_duplicate_ladder(D):
+    """True d^2 from 0 to ~2 at one width: d^2 within 1e-5 of fp64 at every rank, and the d^2 of an exact copy of the
+    query, which is the accumulation error of the dot product alone (|q|^2 = |t|^2 bit for bit)."""
+    rng = np.random.RandomState(D)
+    q, t, copy_idx = _ladder(D, 4, rng)
+    k = 128
+    idx, d2 = _ctx().knn(torch.from_numpy(q).cuda(), torch.from_numpy(t).cuda(), k)
+    ex, err = _check_knn(q, t, k, False, ("ladder", D), got=(idx, d2))
+    idx, d2 = idx.cpu().numpy(), d2.cpu().numpy()
+    copy_d2 = []
+    for i in range(len(q)):
+        at = np.isin(idx[i], copy_idx[i])
+        assert at.sum() == copy_idx.shape[1], (D, i)                       # every copy is among the k nearest ...
+        assert len(set(d2[i, at].view(np.int32).tolist())) == 1, (D, i)   # ... with one d^2: identical rows, identical bits
+        copy_d2.append(float(d2[i, at][0]))
+    assert max(copy_d2) <= DIST_TOL
+    print(f"ladder D={D}: largest d^2 error {err:.2e}, exact-copy d^2 {max(copy_d2):.2e} (of {len(q)} queries), "
+          f"{ex} of {len(q)} queries within the {MARGIN:g} margin (the rungs below 1e-5 are, by design)")
+
+
+def test_knn_on_vlad_vectors_of_planted_scenes():
+    """spn_knn on intra-normalised VLAD vectors as retrieval makes them (k-means and VLAD on the GPU, 128 scenes x 4
+    views, D = 16 384 and 65 536) against the fp64 oracle on the same fp32 vectors, through retrieval.neighbors, with
+    two images without keypoints.  k = 3 is the other views of the scene: fewer than 1 % of the queries may fall within
+    the margin.  k = 20 adds views of other scenes, whose d^2 to the query crowd near 2."""
+    from superpoint_nerf_pytorch_b200 import retrieval
+    S, V = 128, 4
+    desc = torch.from_numpy(_planted_scenes(7, S, V)).cuda()
+    counts = torch.full((S * V,), desc.shape[1], dtype=torch.int32, device="cuda")
+    counts[[5, 300]] = 0
+    has = torch.nonzero(counts > 0).view(-1)
+    has_np = has.cpu().numpy()
+    for K in (64, 256):
+        words = retrieval.kmeans(desc, counts, K, 5)
+        vec = retrieval.vlad(desc, counts, words)
+        assert vec.shape == (S * V, K * 256) and (vec[[5, 300]] == 0).all()
+        v = vec[has].cpu().numpy()
+        for k in (V - 1, 20):
+            index, dist2 = retrieval.neighbors(vec, counts, k)
+            assert (index[[5, 300]] == -1).all() and torch.isinf(dist2[[5, 300]]).all()
+            local = torch.from_numpy(np.searchsorted(has_np, np.maximum(index[has].cpu().numpy(), 0))).to(torch.int32)
+            local = torch.where(index[has].cpu() >= 0, local, -1)                        # image ids -> rows of v
+            ex, err = _check_knn(v, v, k, True, ("vlad", K, k), got=(local, dist2[has].cpu()))
+            print(f"vlad D={K * 256} k={k}: largest d^2 error {err:.2e}, {ex} of {len(v)} queries within the "
+                  f"{MARGIN:g} margin (not compared)")
+            if k == V - 1:
+                assert ex < 0.01 * len(v), ex
 
 
 def _pool_superpoint(top_k=300, n_img=6):
@@ -87,18 +187,38 @@ def _pool_superpoint(top_k=300, n_img=6):
     return out["descriptor_output"]["desc_sparse"].contiguous(), out["detector_output"]["keypoint_count"].contiguous()
 
 
+def _near_copy_pool(C, rng):
+    """Two random unit sets of 500 rows at width C, the second holding near-copies (noise 0.01) of 63 rows of the
+    first, so that dot products near 1 go through every chunk of the tile; counts 500 and 470."""
+    xa = _unit((500, C), rng)
+    xb = np.concatenate([_unit((437, C), rng), xa[:63] + 0.01 * _unit((63, C), rng)])
+    pool = torch.from_numpy(np.stack([xa, xb / np.linalg.norm(xb, axis=1, keepdims=True)])).cuda()
+    return pool, torch.tensor([500, 470], dtype=torch.int32, device="cuda")
+
+
 def test_knn_has_the_same_bits_as_match_pairs():
+    """The three consumers of nn_tc.cuh's distance tile give the same d^2 bits at every width, from one chunk (C <= 256)
+    to 64 chunks: knn's first neighbour and sqrtf of its d^2 equal match_pairs' match and distance, and match_pairs
+    with the mutual check only equals spn_mutual_nn_match."""
     rng = np.random.RandomState(2)
     random_pool = torch.from_numpy(np.stack([_unit((500, 256), rng), _unit((500, 256), rng)])).cuda()
-    pools = [(random_pool, torch.tensor([500, 437], dtype=torch.int32, device="cuda")), _pool_superpoint()]
-    for desc, counts in pools:
+    pools = [(256, random_pool, torch.tensor([500, 437], dtype=torch.int32, device="cuda")), (256, *_pool_superpoint())]
+    pools += [(C, *_near_copy_pool(C, rng)) for C in (64, 128, 256, 1024, 16384)]
+    for C, desc, counts in pools:
         cnt = counts.cpu().tolist()
         pairs = [(a, b) for a in range(len(cnt)) for b in range(len(cnt)) if a != b]
         match, dist = _ctx().match_pairs(desc, counts, pairs, False, 0.0, math.inf)
         for p, (a, b) in enumerate(pairs):
             idx, d2 = _ctx().knn(desc[a, :cnt[a]], desc[b, :cnt[b]], 2)
-            assert torch.equal(idx[:, 0], match[p, :cnt[a]]), (a, b)
+            assert torch.equal(idx[:, 0], match[p, :cnt[a]]), (C, a, b)
             assert np.array_equal(np.sqrt(d2[:, 0].cpu().numpy()).view(np.int32), dist[p, :cnt[a]].cpu().numpy().view(np.int32))
+        pairs = [(a, b) for a in range(len(cnt)) for b in range(len(cnt))]
+        m, dist = _ctx().match_pairs(desc, counts, pairs, True, 0.0, math.inf)
+        ia = torch.tensor([a for a, _ in pairs], device="cuda")
+        ib = torch.tensor([b for _, b in pairs], device="cuda")
+        m_ref, d_ref = _ctx().mutual_nn_match(desc.index_select(0, ia), counts.index_select(0, ia),
+                                              desc.index_select(0, ib), counts.index_select(0, ib))
+        assert torch.equal(m, m_ref) and torch.equal(dist, d_ref), C
 
 
 def test_residual_sums_are_bit_equal_to_the_oracle():
@@ -156,21 +276,6 @@ def test_kmeans_steps_against_the_oracle():
     print(f"kmeans: objective {objective[0]:.2f} -> {objective[-1]:.2f}, {excluded} assignments within the margin")
     with pytest.raises(ValueError, match="retrieval.vocab_size"):
         retrieval.kmeans(d, torch.full_like(c, 1), 13, 1)
-
-
-def _planted_scenes(seed, S=8, V=4, L=400, keep=300, distractors=50, C=256, sigma=0.1):
-    """S scenes of L random unit landmarks; each of V views holds `keep` of its scene's landmarks with noise and
-    `distractors` random unit rows.  sigma is the noise's scale relative to the unit-norm descriptor (per-component
-    standard deviation sigma / sqrt(C), so the noise vector has norm ~sigma) before re-normalisation."""
-    rng = np.random.RandomState(seed)
-    desc = np.zeros((S * V, keep + distractors, C), np.float32)
-    for s in range(S):
-        landmarks = _unit((L, C), rng)
-        for v in range(V):
-            x = landmarks[rng.choice(L, keep, replace=False)] + sigma / math.sqrt(C) * rng.randn(keep, C).astype(np.float32)
-            rows = np.concatenate([x / np.linalg.norm(x, axis=1, keepdims=True), _unit((distractors, C), rng)])
-            desc[s * V + v] = rows[rng.permutation(len(rows))]
-    return desc
 
 
 def test_retrieval_finds_the_views_of_a_scene():
